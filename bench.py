@@ -2,6 +2,7 @@
 """Benchmark of the à trous hot path on B200 (see DESIGN.md section "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-wow] [--no-extras]
+                    [--dump-outputs DIR]
 
 Workload at N=1 (BASELINE.json configs[1]): B3spline 2-D à trous transform of one 4096x4096 fp32 frame over 10
 scales.  One "step" = one full transform (10 per-scale launches) of a device-resident frame; `value` is
@@ -148,6 +149,26 @@ def cpu_reference_rate(side, levels, repeats=1):
     return side * side * levels / best / 1e6, best, backend, threads
 
 
+DUMP_SAMPLES = 1 << 20  # pixel positions kept per plane: 11 planes x 2^20 x 4 B = 44 MiB
+
+
+def dump_outputs(out_dir, planes):
+    """Writes out_dir/planes_sample.npy: the (LEVELS + 1) planes of one transform at a fixed, seeded sample of
+    DUMP_SAMPLES pixel positions (the same positions in every plane, in row-major order), as a float32 or float64
+    (LEVELS + 1, DUMP_SAMPLES) array.  The positions depend only on the frame size, so two builds run with the same
+    arguments can be compared value for value."""
+    n = planes.shape[-2] * planes.shape[-1]
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_SAMPLES, n), replace=False))
+    flat = planes.reshape(planes.shape[0], n)
+    if isinstance(flat, np.ndarray):
+        sample = flat[:, idx]
+    else:  # torch tensor on the device: gather there, copy only the sample
+        import torch
+        sample = flat[:, torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "planes_sample.npy"), sample)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU path (oracle port) on the host cores; rank 0 only."""
     rank = int(os.environ.get("RANK", "0"))
@@ -175,8 +196,10 @@ def run_reference(args):
     timed = max(1, min(args.steps, int(240.0 / max(t_frame, 1e-3))))
     t0 = time.perf_counter()
     for _ in range(timed):
-        orc.atrous_transform(img, LEVELS, SF_NAME, backend=backend)
+        planes = orc.atrous_transform(img, LEVELS, SF_NAME, backend=backend)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, planes)
     value = side * side * LEVELS * timed / dt / 1e6
     threads = 1
     if backend == "cv2":
@@ -452,6 +475,8 @@ def run_ours(args):
     e1.record(stream)
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, planes)
     if args.steps * 0.4 < 300:  # short run: extend the sampling window with untimed identical steps
         t_end = time.perf_counter() + 0.5
         while time.perf_counter() < t_end:
@@ -637,7 +662,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="N > 1: skip the cfg4 / cfg5 (banded) keys")
     ap.add_argument("--extras-timeout", type=float, default=300.0,
                     help="seconds after which the line is printed without the extra keys that have not finished")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's planes to DIR/planes_sample.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
