@@ -17,7 +17,7 @@
 //      w_s of the centre row (same ring) -> streaming 128-bit store of w'_s.  The same barrier completion tells thread
 //      0 which input slot is free for the next TMA load.
 // Two kernels implement it: wow_rows_kernel (any dtype / width up to one 16 KiB row; keeps a separate w^2 ring and a
-// third phase C) and wow_rows_lean_kernel (fp32 rows wider than 2048 columns: unrolled ring, immediate addressing,
+// third phase C) and wow_rows_lean_kernel (fp32 rows of 513 .. 4096 columns: unrolled ring, immediate addressing,
 // packed fp32x2, squares on the fly -- see the comment above it).
 // Rows outside the image are symmetric reflections: the loader fetches the reflected rows; because the symmetric
 // extension commutes with the symmetric smooth, c_{s+1} / w_s evaluated at such a virtual row equal their reflected
@@ -234,7 +234,7 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
 // kernel (60 - 90 KB) does not fit the instruction cache levels below L2, and every change of kernel inside a cascade
 // starts cold (see atrous_rows_lean_kernel).
 // NTK: threads per block = half the vectors of the widest row the instantiation takes -- 512 (rows of 2049 .. 4096
-// columns, 16 KiB ring slots, one block per SM) or 256 (1025 .. 2048 columns, 8 KiB slots, two blocks per SM).
+// columns, 16 KiB ring slots, one block per SM) or 256 (513 .. 2048 columns, 8 KiB slots, two blocks per SM).
 template <int TAPS, int DMODE, bool HINTS, int MODE, int PAIR = 0, bool DYN = false, int NTK = 512>
 __global__ void __launch_bounds__(NTK, NTK == 512 ? 1 : 2) wow_rows_lean_kernel(const ScaleParams p) {
     static_assert(PAIR == 0 || (DMODE == 0 && PAIR < TAPS), "paired columns need d % 4 == 0 and overlapping taps");
@@ -578,7 +578,7 @@ static bool plan_wow(ScaleParams &p, int taps, int esize, int batch, WowGeom *ge
     int occ = (int)(kMaxSmem / (smem + 1024));
     const int occ_regs = 65536 / (nt * 128);
     if (occ > occ_regs) occ = occ_regs;
-    // the 256-thread lean kernel (fp32 rows of 1025 .. 2048 columns, see launch_wow_h) runs two blocks per SM
+    // the 256-thread lean kernel (fp32 rows of 513 .. 2048 columns, see launch_wow_h) runs two blocks per SM
     if (esize == 4 && p.n_strips == 1 && p.W > kLean256MinW && p.W <= 2048 && occ > 2) occ = 2;
     if (occ < 1) occ = 1;
     const long long slots_total = (long long)device_sm_count() * occ;
@@ -661,13 +661,19 @@ static auto wow_kernel_for(bool packed, int pair, bool dyn, int sig_mode) -> voi
 // consecutive lanes conflict-free).  M = 2 at d = 16 and M = 4 at d = 8 were built and measured (the kernel template
 // takes them): alone the d = 16 launch gains 7 us (48 -> 41), inside wow() the two additional kernels per cascade cost
 // more than that (0.611 -> 0.619 ms, profiles/r2_pair_levels.json) -- not instantiated.
-static int wow_pair_step(int taps, int d) {
+// Thread t owns vectors (t / run) 2 run + t % run and + run of the row (pair_first_vector, run = d / 4): the block's nt
+// threads must cover every first vector of the W / 4 vectors.  They do not at d = W (Triangle on a power-of-two row:
+// the second vectors all fall beyond the row and half of it would never be written), so that case, like the K1 kernels
+// (k1_pair_step), keeps the half-row column groups.
+static int wow_pair_step(int taps, int d, int W, int nt) {
     (void)taps;
     if (d < 32 || (d & (d - 1)) != 0 || wow_pair_level() <= 0) return 0;
-    return 1;
+    const int run = d / 4, nvec = W / 4;
+    const int need = ((nvec + 2 * run - 1) / (2 * run)) * run;
+    return need <= nt ? 1 : 0;
 }
 
-// Rows of 1025 .. 2048 columns: 256-thread blocks on 8 KiB slots, two per SM, with the default choice of not-unrolled /
+// Rows of 513 .. 2048 columns: 256-thread blocks on 8 KiB slots, two per SM, with the default choice of not-unrolled /
 // unrolled kernels only (hints on).
 template <int TAPS, int DMODE>
 static auto wow_lean256_kernel(int pair, int sig_mode) -> void (*)(const ScaleParams) {
@@ -689,11 +695,11 @@ static auto wow_lean256_kernel(int pair, int sig_mode) -> void (*)(const ScalePa
 template <typename T, int TAPS, int DMODE, bool HINTS>
 static int launch_wow_h(const ScaleParams &p, int batch, const WowGeom &geo, cudaStream_t st) {
     // the lean kernel runs 512 threads x 2 vectors on 16 KiB ring slots (rows of 2049 .. 4096 columns) or 256 threads on
-    // 8 KiB slots (1025 .. 2048 columns; hints on); narrower rows and float64 keep the generic kernel
+    // 8 KiB slots (513 .. 2048 columns; hints on); narrower rows and float64 keep the generic kernel
     const bool lean_ok = sizeof(T) == 4 && p.n_strips == 1 && wow_packed_enabled();
     const bool packed = lean_ok && p.W > 2048;
     const bool packed256 = lean_ok && HINTS && p.W > kLean256MinW && p.W <= 2048 && geo.ng == 2;
-    const int pair = ((packed || packed256) && DMODE == 0 && HINTS) ? wow_pair_step(TAPS, p.d) : 0;
+    const int pair = ((packed || packed256) && DMODE == 0 && HINTS) ? wow_pair_step(TAPS, p.d, p.W, packed ? 512 : 256) : 0;
     const bool dyn = packed && HINTS && wow_dyn_for(DMODE, p.sig_mode);
     void (*kern)(const ScaleParams) = nullptr;
     if constexpr (sizeof(T) == 4 && HINTS) {
