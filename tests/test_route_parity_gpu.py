@@ -440,22 +440,25 @@ def test_batched_frames_per_frame_noise_vs_oracle(sf, dt):
 EXPECTED_FAMILIES = sorted(
     ["atrous_generic_kernel", "atrous_rows_kernel ng=1", "atrous_rows_kernel ng=2",
      "atrous_rows_lean_kernel 16 KiB slots", "atrous_rows_lean_kernel 8 KiB slots", "atrous_rows_lean_kernel strip",
-     "atrous_rows_lean_kernel paired", "atrous_rows_lean_kernel OP_WHITEN", "wow_rows_kernel"]
+     "atrous_rows_lean_kernel paired", "atrous_rows_lean_kernel OP_WHITEN", "wow_rows_kernel",
+     "bilateral_lean_kernel", "bilateral_window_kernel", "bilateral_rows_kernel", "bilateral_generic_kernel"]
     + [f"wow_rows_lean_kernel {nt} threads {pr} mode {m}" for nt in (512, 256) for pr in ("paired", "unpaired")
        for m in (0, 1, 2)])
 _KERNEL_RE = re.compile(r"\b(atrous_generic_kernel|atrous_rows_lean_kernel|atrous_rows_kernel|wow_rows_lean_kernel|"
-                        r"wow_rows_kernel)<([^>]*)>")
+                        r"wow_rows_kernel|bilateral_lean_kernel|bilateral_window_kernel|bilateral_rows_kernel|"
+                        r"bilateral_generic_kernel)<([^>]*)>")
 
 
 def kernel_families(name):
-    """Families of one demangled kernel name (template arguments as in atrous_scale.cu / wow_scale.cu)."""
+    """Families of one demangled kernel name (template arguments as in atrous_scale.cu / wow_scale.cu; the K2 kernels of
+    bilateral.cu are one family each)."""
     m = _KERNEL_RE.search(name)
     if not m:
         return set()
     kern = m.group(1)
     args = [re.sub(r"\((?:int|bool)\)", "", a).strip() for a in m.group(2).split(",")]
     args = [{"true": "1", "false": "0"}.get(a, a) for a in args]
-    if kern == "atrous_generic_kernel" or kern == "wow_rows_kernel":
+    if kern in ("atrous_generic_kernel", "wow_rows_kernel") or kern.startswith("bilateral_"):
         return {kern}
     if kern == "atrous_rows_kernel":  # <T, TAPS, DMODE, NG, OP>
         return {f"atrous_rows_kernel ng={args[3]}"}
@@ -482,13 +485,21 @@ def test_kernel_family_parser():
     assert kernel_families("void wb::atrous_rows_kernel<double, 5, 1, 1, 1>(wb::ScaleParams)") == {"atrous_rows_kernel ng=1"}
     assert kernel_families("void wb::atrous_rows_lean_kernel<double, 5, 0, true, 1, 2, 0, 4, 24>(wb::ScaleParams)") == {
         "atrous_rows_lean_kernel strip", "atrous_rows_lean_kernel OP_WHITEN"}
+    assert kernel_families("void wb::bilateral_lean_kernel<5, 0, 3>(wb::BilateralParams)") == {"bilateral_lean_kernel"}
+    assert kernel_families("void wb::bilateral_lean_kernel<(int)3, (int)1, (int)-1>(wb::BilateralParams)") == {
+        "bilateral_lean_kernel"}
+    assert kernel_families("void wb::bilateral_window_kernel<3, 1>(wb::BilateralParams)") == {"bilateral_window_kernel"}
+    assert kernel_families("void wb::bilateral_rows_kernel<double, 5, 0>(wb::BilateralParams)") == {"bilateral_rows_kernel"}
+    assert kernel_families("void wb::bilateral_generic_kernel<float, 3>(wb::BilateralParams)") == {
+        "bilateral_generic_kernel"}
     assert kernel_families("void at::native::vectorized_elementwise_kernel<4, float>()") == set()
 
 
 @pytest.mark.gpu
 def test_route_coverage():
-    """Runs the route cases once more (smallest height of each) under torch.profiler and checks that every kernel family
-    the dispatchers can pick was launched, so that a planner change cannot move the cases off a kernel unnoticed."""
+    """Runs the route cases once more (smallest height of each, K2 at the smallest and deepest scale) under
+    torch.profiler and checks that every kernel family the dispatchers can pick was launched, so that a planner change
+    cannot move the cases off a kernel unnoticed."""
     from torch.profiler import ProfilerActivity, profile
     lib = _gpu_lib()
     par = Parity()
@@ -497,8 +508,9 @@ def test_route_coverage():
         for dt, w, heights in CASES:
             for sf in SCALING:
                 img = _frames(1, heights[0], w, dt, 23 + w)
-                for s in scales_of(sf, w):
-                    check_scale(lib, par, img, s, sf)
+                scales = scales_of(sf, w)
+                for s in scales:
+                    check_scale(lib, par, img, s, sf, bilateral=s in (scales[0], scales[-1]))
         img = _frames(1, 9, 1024, np.float32, 3)
         try:
             assert lib.wb_tune_k1(4, 256, 1, 8, 0) == 0
@@ -520,7 +532,7 @@ def test_route_coverage():
 SWITCH_CASES = [(np.float32, 1020), (np.float32, 1500), (np.float32, 2048), (np.float32, 3000), (np.float32, 4096),
                 (np.float32, 6000), (np.float64, 1024), (np.float64, 2048), (np.float64, 3000)]
 SWITCH_VARS = ("WB_PDL", "WB_L2_HINTS", "WB_L2_HINTS_WOW", "WB_K1_UNROLL", "WB_WOW_DYN", "WB_K1_LEAN", "WB_WOW_LEAN",
-               "WB_K1_PAIR", "WB_WOW_PAIR", "WB_K1_LEAN_STRIPS", "WB_WOW_STRIPS", "WB_K2_WINDOW")
+               "WB_K1_PAIR", "WB_WOW_PAIR", "WB_K1_LEAN_STRIPS", "WB_WOW_STRIPS")
 # Every switch must give planes bit-identical to the default (measured on a B200 for all of them).  The first eight
 # change scheduling, cache hints or loop shape only; the last five run another kernel (generic instead of lean, unpaired
 # instead of paired columns, the row kernel instead of lean strips) that performs the same operations in the same order.

@@ -31,18 +31,13 @@ def main():
         out[tag + "_bil_ms"] = timed(lambda: wb.wow(solar, bilateral=1), args.reps)
         print(tag, {k: round(v, 4) for k, v in out.items() if k.startswith(tag)}, flush=True)
 
-    for k2 in ("", "1"):
-        if k2:
-            os.environ["WB_K2_WINDOW"] = k2
-        else:
-            os.environ.pop("WB_K2_WINDOW", None)
+    for s in range(10):
+        lib.wb_tune_k1(s, 0, 0, 0, 0)
+    run("k3lean")
+    for nt, ng, slots in ((128, 1, 6), (96, 1, 6), (64, 1, 6), (128, 1, 8), (256, 1, 6)):
         for s in range(10):
-            lib.wb_tune_k1(s, 0, 0, 0, 0)
-        run(f"k2mode{k2 or 'auto'}_k3lean")
-        for nt, ng, slots in ((128, 1, 6), (96, 1, 6), (64, 1, 6), (128, 1, 8), (256, 1, 6)):
-            for s in range(10):
-                lib.wb_tune_k1(s, nt, ng, slots, 0)
-            run(f"k2mode{k2 or 'auto'}_k3nt{nt}ng{ng}s{slots}")
+            lib.wb_tune_k1(s, nt, ng, slots, 0)
+        run(f"k3nt{nt}ng{ng}s{slots}")
     for s in range(10):
         lib.wb_tune_k1(s, 0, 0, 0, 0)
     os.makedirs("gpurun_out", exist_ok=True)

@@ -22,7 +22,6 @@ struct BilateralParams {
     ScaleParams sp;
     double var_factor;    // sigma_b[s]^2 * (s + 1 if bilateral_scaling else 1)
     float var_factor_f;   // the same, rounded once on the host (no F2F in the fp32 step loop)
-    unsigned poll_ns;     // window kernel: sleep between the producer's polls of a ring slot (0: the default)
 };
 
 __device__ __forceinline__ float exp2_fast(float x) {
@@ -374,12 +373,10 @@ __device__ __forceinline__ void pair_taps(uint32_t rowb, const uint32_t (&colb)[
 // Row statistics for the variance (law of total variance over the window rows).  For one staged row and this thread's
 // pixel pair, relative to the row's own centre-column pixel x_c:   a = sum_k h_k (x_k - x_c),  b = sum_k h_k (x_k - x_c)^2.
 // They depend on (row, column) only, so they are computed ONCE per input row (when it becomes the newest window row)
-// and kept in a per-thread shared-memory ring for the 2C later windows that contain the row.  With e_i = x_ic - x_cc
+// and kept in registers for the 2C later windows that contain the row.  With e_i = x_ic - x_cc
 // (row centre minus window centre) the window moments are
 //     s1 = sum_i h_i (a_i + e_i),      s2 = sum_i h_i (b_i + e_i (2 a_i + e_i)),      var = s2 - s1^2
 // -- still differences only (no cancellation), 60 packed operations per pixel pair instead of 96.
-static constexpr long long kPairStats = 256 * 16;  // bytes of row statistics per ring slot (256 consumer threads)
-
 template <int TAPS>
 __device__ __forceinline__ P4 row_stats(const u64 (&tv)[TAPS]) {
     constexpr int C = TAPS / 2;
@@ -396,269 +393,26 @@ __device__ __forceinline__ P4 row_stats(const u64 (&tv)[TAPS]) {
     return P4{a, b};
 }
 
-// One step of the software pipeline (see the kernel): range weights + output of the OLD row from the differences in
-// D, differences + variance sums of the NEW row into D.  OLD / NEW are compile-time so the prologue (NEW only) and
-// the drain (OLD only) cost no selects in the steady state.
-template <int TAPS, int DMODE, bool OLD, bool NEW, bool MIRROR>
-__device__ __forceinline__ void pair_step(u64 (&D)[TAPS][TAPS], u64 &xc_old, u64 &nhi, const uint32_t (&rowb)[TAPS],
-                                          const uint32_t (&statb)[TAPS], uint32_t cb,
-                                          const uint32_t (&colb)[PairPlan<TAPS, DMODE>::NL], unsigned rev,
-                                          float var_factor, float *c_dst, float *w_dst, bool act, uint64_t pol_keep) {
-    constexpr int C = TAPS / 2;
-    const float kc = Taps<float, TAPS>::h(C) * Taps<float, TAPS>::h(C);
-    u64 xc = 0ull;
-    if (NEW) xc = lds64(rowb[C] + cb);
-    u64 s1 = 0ull, s2 = 0ull;  // packed +0.0f
-    u64 num = 0ull, den = pk2(kc, kc);
-#pragma unroll
-    for (int i = 0; i < TAPS; ++i) {
-        u64 tv[TAPS];
-        if (NEW) pair_taps<TAPS, DMODE, MIRROR>(rowb[i], colb, rev, tv);
-#pragma unroll
-        for (int k = 0; k < TAPS; ++k) {
-            if (OLD && !(i == C && k == C)) {
-                const float lk = TapLog2<TAPS>::l(i) + TapLog2<TAPS>::l(k);
-                const u64 dd = D[i][k];
-                float a0, a1;
-                up2(fma2(mul2(dd, dd), nhi, pk2(lk, lk)), a0, a1);
-                const u64 gw = pk2(exp2_fast(a0), exp2_fast(a1));
-                den = add2(den, gw);
-                num = fma2(gw, dd, num);
-            }
-            if (NEW) D[i][k] = sub2(xc, tv[k]);
-        }
-        if (NEW) {
-            // window moments from the row statistics: the newest row's are computed here (and stored for the next
-            // 2C windows), the others come from the ring
-            const float hi = Taps<float, TAPS>::h(i);
-            P4 st;
-            if (i == TAPS - 1) {
-                st = row_stats<TAPS>(tv);
-                sts_p4(statb[i], st);
-            } else {
-                st = lds_p4(statb[i]);
-            }
-            if (i == C) {
-                s1 = fma2(pk2(-hi, -hi), st.lo, s1);
-                s2 = fma2(pk2(hi, hi), st.hi, s2);
-            } else {
-                // e = x_ic - x_cc = -D[i][C];  2 a + e = 2 a - D;  b + e (2 a + e) = b - D (2 a - D)
-                // with dc = D[i][C] = -e:  s1 accumulates -(a + e) = dc - a (only s1^2 is used);
-                // b + e (2 a + e) = b + dc (dc - 2 a)
-                const u64 dc = D[i][C];
-                const u64 t = fma2(pk2(-2.0f, -2.0f), st.lo, dc);
-                const u64 u = fma2(dc, t, st.hi);
-                s1 = fma2(pk2(hi, hi), sub2(dc, st.lo), s1);
-                s2 = fma2(pk2(hi, hi), u, s2);
-            }
-        }
-    }
-    if (OLD) {
-        float n0, n1, d0, d1, x0v, x1v;
-        up2(num, n0, n1);
-        up2(den, d0, d1);
-        up2(xc_old, x0v, x1v);
-        const float c0 = fmaf(-n0, rcp_fast(d0), x0v), c1 = fmaf(-n1, rcp_fast(d1), x1v);  // one FFMA each, spelled out: left to
-            // the compiler's contraction, one kernel fused both halves of the pair and another only one (1-ulp differences)
-        if (act) {
-            if (c_dst) {
-                if (pol_keep)
-                    asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1, %2}, %3;" ::"l"(c_dst), "f"(c0), "f"(c1), "l"(pol_keep) : "memory");
-                else
-                    *reinterpret_cast<float2 *>(c_dst) = make_float2(c0, c1);
-            }
-            if (w_dst) __stcs(reinterpret_cast<float2 *>(w_dst), make_float2(x0v - c0, x1v - c1));
-        }
-    }
-    if (NEW) {
-        // var = S[x^2] - S[x]^2 in centred form; V = max(var, 1e-20) * var_factor; exponent scale -log2(e) / (2 V)
-        float v0, v1;
-        up2(sub2(s2, mul2(s1, s1)), v0, v1);
-        v0 = (v0 <= 0.0f) ? 1e-20f : v0;
-        v1 = (v1 <= 0.0f) ? 1e-20f : v1;
-        nhi = pk2(-0.72134752044448170f * rcp_fast(v0 * var_factor), -0.72134752044448170f * rcp_fast(v1 * var_factor));
-        xc_old = xc;
-    }
-}
-
-template <int TAPS, int DMODE>
-__global__ void __launch_bounds__(288, 2) bilateral_pairs_kernel(const BilateralParams bp) {
-    const ScaleParams &p = bp.sp;
-    pdl_launch_dependents();
-    constexpr int C = TAPS / 2;
-    constexpr int NL = PairPlan<TAPS, DMODE>::NL;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    float *rows = reinterpret_cast<float *>(smem_raw);
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + (size_t)p.slots * p.row_stride * sizeof(float));
-    uint64_t *empty = full + p.slots;
-    // per-thread row statistics (a, b) of every staged row: slots x 256 threads x 16 bytes, same slot index as the row
-    const uint32_t stats_base = smem_u32(empty + p.slots);
-
-    const int nt = blockDim.x - 32;  // 8 consumer warps; the last warp is the TMA producer
-    const int nwc = nt >> 5;
-    const int tid = threadIdx.x;
-    const int warp = tid >> 5;
-    const int lane = tid & 31;
-
-    int bx = blockIdx.x;
-    const int strip = bx % p.n_strips;
-    bx /= p.n_strips;
-    const int r = bx % p.d;
-    const int g = bx / p.d;
-    const int frame = blockIdx.y;
-
-    const int n_chain = (r < p.H) ? (p.H - r + p.d - 1) / p.d : 0;
-    const int i0 = g * p.seg;
-    const int n_out = min(p.seg, n_chain - i0);
-    if (n_out <= 0) return;
-    const int n_load = n_out + 2 * C;
-
-    const int x0 = strip * p.wt;
-    const int lo = max(0, x0 - p.halo_al);
-    const int hi = min(p.W, x0 + p.wt + p.halo_al);
-    const uint32_t row_bytes = (uint32_t)(hi - lo) * (uint32_t)sizeof(float);
-    const uint32_t RB = (uint32_t)p.row_stride * (uint32_t)sizeof(float);
-
-    if (tid == 0) {
-        for (int s = 0; s < p.slots; ++s) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], nwc);
-        }
-        fence_mbar_init();
-    }
-    __syncthreads();
-    pdl_wait();  // everything below touches global memory written or read by the previous launch
-
-    if (warp == nwc) {
-        if (lane == 0) {
-            const float *src = reinterpret_cast<const float *>(p.in) + (long long)frame * p.in_bstride + lo;
-            const uint64_t pol_in = policy_evict_first();  // c_s is dead once this launch has read it
-            int slot = 0;
-            uint32_t round = 0;
-            for (int j = 0; j < n_load; ++j) {
-                if (round > 0) {
-                    // the producer runs rows ahead of the consumers: poll rarely, its spinning would take issue slots
-                    // from the warps doing the arithmetic (the kernel is issue / pipe bound)
-                    while (!mbar_test(&empty[slot], (round - 1) & 1)) __nanosleep(2000);
-                }
-                const long long y = reflect_any(p.gwy0 + r + (long long)(i0 - C + j) * p.d, p.Hg) - p.gwy0 + p.row_off_in;
-                mbar_arrive_expect_tx(&full[slot], row_bytes);
-                if (p.l2_hints) tma_load_1d_hint(rows + (size_t)slot * p.row_stride, src + y * p.in_pitch, row_bytes, &full[slot], pol_in);
-                else tma_load_1d(rows + (size_t)slot * p.row_stride, src + y * p.in_pitch, row_bytes, &full[slot]);
-                if (++slot == p.slots) { slot = 0; ++round; }
-            }
-        }
-        return;
-    }
-
-    float *out_c = reinterpret_cast<float *>(p.out_c);
-    float *out_w = reinterpret_cast<float *>(p.out_w);
-    if (out_c) out_c += (long long)frame * p.c_bstride;
-    if (out_w) out_w += (long long)frame * p.w_bstride;
-
-    int xg = x0 + tid * 2;
-    const bool act = xg < p.W && xg < x0 + p.wt;
-    if (!act) xg = x0;  // idle threads shadow the first pair of the strip; their stores are masked
-    uint32_t colb[NL];
-    unsigned rev = 0;
-#pragma unroll
-    for (int k = 0; k < NL; ++k) {
-        const int pcol = xg + (k - NL / 2) * (DMODE == 0 ? p.d : 2);  // even; one reflection at most
-        const bool left = pcol < 0, right = pcol >= p.W;
-        const int q = left ? (-2 - pcol) : (right ? (2 * p.W - 2 - pcol) : pcol);
-        // per-thread tap addresses in slot 0; a window row adds a block-uniform slot offset ([R + UR] addressing)
-        colb[k] = smem_u32(rows) + (uint32_t)(q - lo) * 4u;  // absolute address of the tap in ring slot 0
-        if (left || right) rev |= 1u << k;
-    }
-    const uint32_t cb = smem_u32(rows) + (uint32_t)(xg - lo) * 4u;
-    const uint32_t stat_t = stats_base + (uint32_t)tid * 16u;  // this thread's entry in stats slot 0
-    const float var_factor = (float)bp.var_factor;
-    const uint64_t pol_keep = p.l2_hints ? policy_evict_last() : 0ull;  // c_{s+1}: the next scale reads it back
-
-    // Per output row: pass 1 (differences + variance sums from the window rows in shared memory, FMA pipe only), then
-    // pass 2 (range weights from the differences kept in registers: 2 MUFU per packed tap).  Warps drift freely (no
-    // block barrier), so the passes of different warps overlap on the FMA and MUFU pipes.  [A variant that interleaves
-    // pass 2 of row n-1 with pass 1 of row n inside each thread (pair_step<.., true, true>) measured 20 % slower.]
-    // Warps that own no reflected column (all but the first / last strip's edge warps) run the variant without the
-    // mirror selects; the choice is warp-uniform, so no thread diverges inside the step.
-    auto run = [&](auto mirror) {
-        constexpr bool MIRROR = decltype(mirror)::value != 0;
-        long long orow = (long long)r + (long long)i0 * p.d;
-        int slot = 0, fslot = 0;  // slot of chain row j, slot of row j - 2C (first row of the window, next to be released)
-        uint32_t parity = 0;
-        u64 D[TAPS][TAPS];
-        u64 xc_old = 0ull, nhi = 0ull;
-        for (int j = 0; j < n_load; ++j) {
-            mbar_wait(&full[slot], parity);
-            if (j < 2 * C) {
-                // rows that are never the newest row of a window of this segment: their statistics are computed here
-                u64 tv[TAPS];
-                pair_taps<TAPS, DMODE, MIRROR>((uint32_t)slot * RB, colb, rev, tv);
-                sts_p4(stat_t + (uint32_t)slot * (256u * 16u), row_stats<TAPS>(tv));
-            } else {
-                uint32_t rowb[TAPS], statb[TAPS];
-                int ws = fslot;
-#pragma unroll
-                for (int i = 0; i < TAPS; ++i) {
-                    rowb[i] = (uint32_t)ws * RB;  // block-uniform byte offset of the window row's slot
-                    statb[i] = stat_t + (uint32_t)ws * (256u * 16u);
-                    if (++ws == p.slots) ws = 0;
-                }
-                float *c_dst = out_c ? out_c + (orow + p.row_off_c) * p.c_pitch + xg : nullptr;
-                float *w_dst = out_w ? out_w + (orow + p.row_off_w) * p.w_pitch + xg : nullptr;
-                pair_step<TAPS, DMODE, false, true, MIRROR>(D, xc_old, nhi, rowb, statb, cb, colb, rev, var_factor, c_dst, w_dst, act, pol_keep);
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&empty[fslot]);  // the window rows are only read in pass 1
-                if (++fslot == p.slots) fslot = 0;
-                pair_step<TAPS, DMODE, true, false, MIRROR>(D, xc_old, nhi, rowb, statb, cb, colb, rev, var_factor, c_dst, w_dst, act, pol_keep);
-                orow += p.d;
-            }
-            if (++slot == p.slots) { slot = 0; parity ^= 1; }
-        }
-    };
-    if (__any_sync(0xffffffffu, rev != 0)) run(IC<1>{});
-    else run(IC<0>{});
-}
-
 // ---------------------------------------------------------------------------------------------------------------
-// fp32 fast path, round 2: the same arithmetic with the 5x5 tap VALUES of the pixel pair held in a REGISTER sliding
-// window (bilateral_window_kernel).  ncu on bilateral_pairs_kernel: 457 warp instructions per warp-row of which 255 are
-// FP / MUFU -- the rest is re-loading all 25 tap pairs for every output row (30 LDS.64 with one address add each), the
+// fp32 fast path, round 2: the 5x5 tap VALUES of the pixel pair held in a REGISTER sliding window
+// (bilateral_window_kernel).  The round-1 kernel re-loaded all 25 tap pairs for every output row: ncu counted 457 warp
+// instructions per warp-row of which 255 were FP / MUFU, the rest being 30 LDS.64 with one address add each, a
 // row-statistics ring in shared memory and its indexing.  Here a staged row is read ONCE per thread, when it arrives
 // (TAPS LDS.64), into the window X[row slot][tap]; its row statistics (a, b) stay in registers too.  The step loop is
 // unrolled by TAPS so that the rotating row slot is a compile-time index: no register moves, no shared-memory ring
 // beyond the TMA staging slots (released right after the loads), ~250 warp instructions per warp-row of which 48 are
 // the MUFU ex2 that bound the kernel (2 per packed tap: 24 * 4096^2 exponentials per plane = 87 us of MUFU pipe).
-// Operation order and roundings are those of bilateral_pairs_kernel: the planes are bit-identical (WB_K2_WINDOW=0
-// selects the old kernel; tests/test_wide_parity_gpu.py compares the two).
+// The lean kernel below runs the same operations in the same order, faster; this one serves what it declines (one
+// output, L2 hints off, staged rows over 16 KiB, d * pitch over 2^31 bytes) with bit-identical planes.
 // ---------------------------------------------------------------------------------------------------------------
 // 8 consumer warps + a ninth warp whose lane 0 streams the rows.  Two blocks per SM at the 96 registers ptxas budgets
 // for this block size (a few spilled values; __maxnreg__(104) or (112) removes them but the register file then
-// holds ONE block per SM: 204 - 222 instead of 150 us).  Measured and not kept: 256-thread blocks whose thread 0 tops the ring
-// up with non-blocking probes (213 us: instruction-cache misses and a lagging warp 0).
-// Block geometries (WG).  ptxas orders the tap loop by its register budget: at 96 registers (two 288-thread blocks per
-// SM, the round-2 default) it emits sub -> mul -> fma -> 2 MUFU -> accumulate serially per tap, every MUFU consumed the
-// instruction after it is issued (mean distance 3 instructions); from 128 registers on it keeps several taps in flight
-// (mean distance 8), whatever the source order.  The register file holds 16 warps at 128 registers, so:
-//   WG 0: 8 consumer warps + 1 producer warp, 2 blocks per SM, 96 registers (16 consumer warps per SM);
-//   WG 3: 4 consumer warps + 1 producer warp (160 threads, 256-column strips), 3 blocks per SM, 128 registers
-//         (12 consumer warps per SM, interleaved taps);
-//   WG 1 / 2 / 4: warp-group register reallocation (setmaxnreg): the block carries a producer WARP GROUP of four warps
-//         that gives its registers back (24 left; three of its warps exit at once) and the consumers grow to CREGS.
-//   WG 5 / 6: WG 2 / 4 with the staged row fetched ONE STEP AHEAD into a sixth row of registers (the try_wait -> LDS.64 ->
-//         statistics -> variance -> rcp chain at the head of a step otherwise leaves the warp without exponentials
-//         to issue for ~150 cycles: tools/k2mimic.cu).
-template <int WG> struct WindowGeom {
-    static constexpr bool PF = (WG == 5 || WG == 6);                                       // prefetch the next row
-    static constexpr int G = (WG == 5) ? 2 : (WG == 6 ? 4 : WG);                           // block geometry
-    static constexpr int CW = (G == 2) ? 16 : ((G == 3 || G == 4) ? 4 : 8);                // consumer warps
-    static constexpr bool REALLOC = (G == 1 || G == 2 || G == 4);                          // setmaxnreg
-    static constexpr int THREADS = CW * 32 + (REALLOC ? 128 : 32);                         // block size
-    static constexpr int BLOCKS = (G == 2) ? 1 : ((G == 3 || G == 4) ? 3 : 2);             // resident blocks per SM
-    static constexpr int CREGS = (G == 2) ? 112 : (G == 4 ? 136 : 104);                    // consumer registers after the inc
-};
-template <int TAPS, int DMODE, int WG>
-__device__ __forceinline__ void bilateral_window_body(const BilateralParams &bp) {
+// holds ONE block per SM: 204 - 222 instead of 150 us).  At 96 registers ptxas emits sub -> mul -> fma -> 2 MUFU ->
+// accumulate serially per tap; larger register budgets (setmaxnreg producer warp groups, 160-thread blocks at 128
+// registers, a row prefetched one step ahead) interleave the taps but measured within 3 % of this geometry
+// (DESIGN §4 K2; those variants were deleted).
+template <int TAPS, int DMODE>
+__global__ void __launch_bounds__(288, 2) bilateral_window_kernel(const BilateralParams bp) {
     const ScaleParams &p = bp.sp;
     pdl_launch_dependents();
     constexpr int C = TAPS / 2;
@@ -668,8 +422,7 @@ __device__ __forceinline__ void bilateral_window_body(const BilateralParams &bp)
     uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + (size_t)p.slots * p.row_stride * sizeof(float));
     uint64_t *empty = full + p.slots;
 
-    const int nt = WindowGeom<WG>::CW * 32;  // consumer threads; the warp after them is the TMA producer
-    const int nwc = nt >> 5;
+    constexpr int nt = 256, nwc = 8;  // consumer threads / warps; warp 8 is the TMA producer
     const int tid = threadIdx.x;
     const int warp = tid >> 5;
     const int lane = tid & 31;
@@ -727,27 +480,18 @@ __device__ __forceinline__ void bilateral_window_body(const BilateralParams &bp)
         if (m_pos >= period) m_pos -= period;
     };
     if (warp >= nwc) {
-        if constexpr (WindowGeom<WG>::REALLOC) asm volatile("setmaxnreg.dec.sync.aligned.u32 24;");
         if (warp == nwc && lane == 0) {
+            // one row per iteration: unrolled, this loop would only add instruction-cache footprint
+#pragma unroll 1
             while (next_load < n_load) {
-                // the producer runs rows ahead of the consumers: poll rarely, its spinning would take issue slots
-                // from the warps doing the arithmetic
-                // blocking try_wait; WB_K2_POLL=ns selects a test + nanosleep(ns) poll instead.  Measured identical (154 us,
-                // 91.8 M warp instructions per plane for the blocking wait and for 1000 / 5000 ns polls): neither the
-                // suspend-time hint nor the sleep length changes how often the waiting lane comes back
-                if (lround > 0) {
-                    if (bp.poll_ns) {
-                        while (!mbar_test(&empty[lslot], (lround - 1) & 1)) __nanosleep(bp.poll_ns);
-                    } else {
-                        mbar_wait(&empty[lslot], (lround - 1) & 1);
-                    }
-                }
+                // blocking try_wait: a test + nanosleep poll measured identical (154 us, 91.8 M warp instructions per
+                // plane for 1000 / 5000 ns sleeps), so the waiting lane takes no issue slots from the arithmetic either way
+                if (lround > 0) mbar_wait(&empty[lslot], (lround - 1) & 1);
                 issue_load();
             }
         }
         return;
     }
-    if constexpr (WindowGeom<WG>::REALLOC) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(WindowGeom<WG>::CREGS));
 
     float *out_c = reinterpret_cast<float *>(p.out_c);
     float *out_w = reinterpret_cast<float *>(p.out_w);
@@ -783,25 +527,14 @@ __device__ __forceinline__ void bilateral_window_body(const BilateralParams &bp)
         uint32_t parity = 0;
         // Step j = TAPS u + I: chain row j lands -> its tap pairs and statistics enter slot I; from j = 2C on, the
         // output row j - C (centre slot (I - C) mod TAPS) is produced from the window.
-        auto fetch = [&](u64 (&dst)[TAPS]) {
-            mbar_wait(&full[slot], parity);
-            pair_taps<TAPS, DMODE, MIRROR>((uint32_t)slot * RB, colb, rev, dst);
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty[slot]);  // the staged row is read exactly once per thread
-            if (++slot == p.slots) { slot = 0; parity ^= 1; }
-        };
-        u64 N[TAPS];  // prefetch geometries: the tap pairs of the next chain row
-        if constexpr (WindowGeom<WG>::PF) fetch(N);
         auto step = [&](auto ic, const int j) {
             constexpr int I = decltype(ic)::value;
             if (j >= n_load) return;
-            if constexpr (WindowGeom<WG>::PF) {
-#pragma unroll
-                for (int k = 0; k < TAPS; ++k) X[I][k] = N[k];
-                if (j + 1 < n_load) fetch(N);
-            } else {
-                fetch(X[I]);
-            }
+            mbar_wait(&full[slot], parity);
+            pair_taps<TAPS, DMODE, MIRROR>((uint32_t)slot * RB, colb, rev, X[I]);
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&empty[slot]);  // the staged row is read exactly once per thread
+            if (++slot == p.slots) { slot = 0; parity ^= 1; }
             {
                 const P4 st = row_stats<TAPS>(X[I]);
                 SA[I] = st.lo;
@@ -885,16 +618,6 @@ __device__ __forceinline__ void bilateral_window_body(const BilateralParams &bp)
     // mirror selects; the choice is warp-uniform, so no thread diverges inside the step
     if (__any_sync(0xffffffffu, rev != 0)) run(IC<1>{});
     else run(IC<0>{});
-}
-
-template <int TAPS, int DMODE, int WG = 0>
-__global__ void __launch_bounds__(WindowGeom<WG>::THREADS, WindowGeom<WG>::BLOCKS) bilateral_window_kernel(const BilateralParams bp) {
-    bilateral_window_body<TAPS, DMODE, WG>(bp);
-}
-// WG 3 with the register budget spelled out (launch bounds alone make ptxas stop at 119 and serialise the taps again)
-template <int TAPS, int DMODE>
-__global__ void __maxnreg__(128) bilateral_window128_kernel(const BilateralParams bp) {
-    bilateral_window_body<TAPS, DMODE, 3>(bp);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1020,7 +743,6 @@ __global__ void __launch_bounds__(288, 2) bilateral_lean_kernel(const BilateralP
     const uint32_t sbase = opaque_u32(rows0);
     const uint32_t own = opaque_u32(colb[NL / 2]);
     const uint32_t tstep = opaque_u32((uint32_t)(DMODE == 0 ? p.d : 2) * 4u);
-    const int tstep_u = p.d * 4;  // the same stride as a launch constant (LD == -2)
     const bool mirror_warp = __any_sync(0xffffffffu, rev != 0);
     if (mirror_warp) {
 #pragma unroll
@@ -1059,11 +781,6 @@ __global__ void __launch_bounds__(288, 2) bilateral_lean_kernel(const BilateralP
             mbar_wait_imm<FULL_OFF + 8 * I>(sbase, parity);
             if constexpr (DMODE == 0 && !MIRROR && LD >= 0) {
                 lean_load_taps<TAPS, I * RB, (LD >= 0 ? LD : 0)>(own, X[WS], std::make_integer_sequence<int, TAPS>{});
-            } else if constexpr (DMODE == 0 && !MIRROR && LD == -2) {
-                // the tap offsets (k - C) * stride are the same in every thread: left to ptxas as warp-uniform values they
-                // become the uniform-register term of LDS [R + UR + imm] -- one kernel for every dilation
-#pragma unroll
-                for (int k = 0; k < TAPS; ++k) X[WS][k] = lds64_imm<I * RB>(own + (uint32_t)((k - C) * tstep_u));
             } else if constexpr (DMODE == 0) {
 #pragma unroll
                 for (int k = 0; k < TAPS; ++k) {
@@ -1165,198 +882,6 @@ __global__ void __launch_bounds__(288, 2) bilateral_lean_kernel(const BilateralP
     // warps that own no reflected column (all but the first / last strip's edge warps) run the variant without the
     // mirror selects; the choice is warp-uniform, so no thread diverges inside the step
     if (mirror_warp) run(IC<1>{});
-    else run(IC<0>{});
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// fp32, thread-level parallelism instead of registers (bilateral_stream_kernel).  ncu on the register-window kernel:
-// only 16 consumer warps fit per SM (112 registers), ptxas places every MUFU pair right in front of its consumer, and
-// the MUFU pipe that bounds the kernel idles 35 % of the time (stalls: wait, short scoreboard, MIO queue).  Here nothing
-// lives in registers across output rows: the taps are re-read from the staged rows (LDS.64), the differences are
-// formed where they are used, the row statistics sit in the per-thread shared-memory ring of the round-1 kernel -- 56
-// registers, FOUR blocks per SM (32 consumer warps), so that some warp always has exponentials to issue.
-// Same operations in the same order as bilateral_pairs_kernel: bit-identical planes.
-// ---------------------------------------------------------------------------------------------------------------
-template <int TAPS, int DMODE>
-__global__ void __maxnreg__(56) bilateral_stream_kernel(const BilateralParams bp) {
-    const ScaleParams &p = bp.sp;
-    pdl_launch_dependents();
-    constexpr int C = TAPS / 2;
-    constexpr int NL = PairPlan<TAPS, DMODE>::NL;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    float *rows = reinterpret_cast<float *>(smem_raw);
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + (size_t)p.slots * p.row_stride * sizeof(float));
-    uint64_t *empty = full + p.slots;
-    const uint32_t stats_base = smem_u32(empty + p.slots);  // slots x 256 threads x 16 bytes of row statistics
-
-    const int nt = blockDim.x - 32;  // 8 consumer warps; the last warp is the TMA producer
-    const int nwc = nt >> 5;
-    const int tid = threadIdx.x;
-    const int warp = tid >> 5;
-    const int lane = tid & 31;
-
-    int bx = blockIdx.x;
-    const int strip = bx % p.n_strips;
-    bx /= p.n_strips;
-    const int r = bx % p.d;
-    const int g = bx / p.d;
-    const int frame = blockIdx.y;
-
-    const int n_chain = (r < p.H) ? (p.H - r + p.d - 1) / p.d : 0;
-    const int i0 = g * p.seg;
-    const int n_out = min(p.seg, n_chain - i0);
-    if (n_out <= 0) return;
-    const int n_load = n_out + 2 * C;
-
-    const int x0 = strip * p.wt;
-    const int lo = max(0, x0 - p.halo_al);
-    const int hi = min(p.W, x0 + p.wt + p.halo_al);
-    const uint32_t row_bytes = (uint32_t)(hi - lo) * (uint32_t)sizeof(float);
-    const uint32_t RB = (uint32_t)p.row_stride * (uint32_t)sizeof(float);
-
-    if (tid == 0) {
-        for (int s = 0; s < p.slots; ++s) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], nwc);
-        }
-        fence_mbar_init();
-    }
-    __syncthreads();
-    pdl_wait();  // everything below touches global memory written or read by the previous launch
-
-    if (warp == nwc) {
-        if (lane == 0) {
-            const float *src = reinterpret_cast<const float *>(p.in) + (long long)frame * p.in_bstride + lo;
-            const uint64_t pol_in = policy_evict_first();  // c_s is dead once this launch has read it
-            int slot = 0;
-            uint32_t round = 0;
-            for (int j = 0; j < n_load; ++j) {
-                if (round > 0) {
-                    while (!mbar_test(&empty[slot], (round - 1) & 1)) __nanosleep(500);
-                }
-                const long long y = reflect_any(p.gwy0 + r + (long long)(i0 - C + j) * p.d, p.Hg) - p.gwy0 + p.row_off_in;
-                mbar_arrive_expect_tx(&full[slot], row_bytes);
-                if (p.l2_hints) tma_load_1d_hint(rows + (size_t)slot * p.row_stride, src + y * p.in_pitch, row_bytes, &full[slot], pol_in);
-                else tma_load_1d(rows + (size_t)slot * p.row_stride, src + y * p.in_pitch, row_bytes, &full[slot]);
-                if (++slot == p.slots) { slot = 0; ++round; }
-            }
-        }
-        return;
-    }
-
-    float *out_c = reinterpret_cast<float *>(p.out_c);
-    float *out_w = reinterpret_cast<float *>(p.out_w);
-
-    int xg = x0 + tid * 2;
-    const bool act = xg < p.W && xg < x0 + p.wt;
-    if (!act) xg = x0;  // idle threads shadow the first pair of the strip; their stores are masked
-    uint32_t colb[NL];
-    unsigned rev = 0;
-#pragma unroll
-    for (int k = 0; k < NL; ++k) {
-        const int pcol = xg + (k - NL / 2) * (DMODE == 0 ? p.d : 2);  // even; one reflection at most
-        const bool left = pcol < 0, right = pcol >= p.W;
-        const int q = left ? (-2 - pcol) : (right ? (2 * p.W - 2 - pcol) : pcol);
-        colb[k] = smem_u32(rows) + (uint32_t)(q - lo) * 4u;  // absolute address of the tap in ring slot 0
-        if (left || right) rev |= 1u << k;
-    }
-    const uint32_t cb = smem_u32(rows) + (uint32_t)(xg - lo) * 4u;
-    const uint32_t stat_t = stats_base + (uint32_t)tid * 16u;  // this thread's entry in stats slot 0
-    const float var_factor = bp.var_factor_f;
-    const uint64_t pol_keep = p.l2_hints ? policy_evict_last() : 0ull;  // c_{s+1}: the next scale reads it back
-    const float kc = Taps<float, TAPS>::h(C) * Taps<float, TAPS>::h(C);
-
-    const long long orow0 = (long long)r + (long long)i0 * p.d;
-    float *c_dst = out_c ? out_c + (long long)frame * p.c_bstride + (orow0 + p.row_off_c) * p.c_pitch + xg : nullptr;
-    float *w_dst = out_w ? out_w + (long long)frame * p.w_bstride + (orow0 + p.row_off_w) * p.w_pitch + xg : nullptr;
-    const long long c_step = (long long)p.d * p.c_pitch, w_step = (long long)p.d * p.w_pitch;
-
-    auto run = [&](auto mirror) {
-        constexpr bool MIRROR = decltype(mirror)::value != 0;
-        int slot = 0, fslot = 0;  // slot of chain row j, slot of row j - 2C (first row of the window, next to be released)
-        uint32_t parity = 0;
-#pragma unroll 1
-        for (int j = 0; j < n_load; ++j) {
-            mbar_wait(&full[slot], parity);
-            {
-                // row statistics of the newest row, kept in the per-thread ring for the 2C later windows
-                u64 tv[TAPS];
-                pair_taps<TAPS, DMODE, MIRROR>((uint32_t)slot * RB, colb, rev, tv);
-                sts_p4(stat_t + (uint32_t)slot * (256u * 16u), row_stats<TAPS>(tv));
-            }
-            if (j >= 2 * C) {
-                int cs = fslot + C;
-                if (cs >= p.slots) cs -= p.slots;
-                const u64 xc = lds64(cb + (uint32_t)cs * RB);
-                // window moments from the row statistics (differences only), rows top to bottom
-                u64 s1 = 0ull, s2 = 0ull;
-                int ws = fslot;
-#pragma unroll
-                for (int i = 0; i < TAPS; ++i) {
-                    const float hi_ = Taps<float, TAPS>::h(i);
-                    const P4 st = lds_p4(stat_t + (uint32_t)ws * (256u * 16u));
-                    if (i == C) {
-                        s1 = fma2(pk2(-hi_, -hi_), st.lo, s1);
-                        s2 = fma2(pk2(hi_, hi_), st.hi, s2);
-                    } else {
-                        const u64 dc = sub2(xc, lds64(cb + (uint32_t)ws * RB));
-                        const u64 t = fma2(pk2(-2.0f, -2.0f), st.lo, dc);
-                        const u64 u = fma2(dc, t, st.hi);
-                        s1 = fma2(pk2(hi_, hi_), sub2(dc, st.lo), s1);
-                        s2 = fma2(pk2(hi_, hi_), u, s2);
-                    }
-                    if (++ws == p.slots) ws = 0;
-                }
-                float v0, v1;
-                up2(sub2(s2, mul2(s1, s1)), v0, v1);
-                v0 = (v0 <= 0.0f) ? 1e-20f : v0;
-                v1 = (v1 <= 0.0f) ? 1e-20f : v1;
-                const u64 nhi = pk2(-0.72134752044448170f * rcp_fast(fmaxf(v0 * var_factor, 1e-37f)),
-                                    -0.72134752044448170f * rcp_fast(fmaxf(v1 * var_factor, 1e-37f)));
-                u64 num = 0ull, den = pk2(kc, kc);
-                ws = fslot;
-#pragma unroll
-                for (int i = 0; i < TAPS; ++i) {
-                    u64 tv[TAPS];
-                    pair_taps<TAPS, DMODE, MIRROR>((uint32_t)ws * RB, colb, rev, tv);
-#pragma unroll
-                    for (int k = 0; k < TAPS; ++k) {
-                        if (i == C && k == C) continue;
-                        const float lk = TapLog2<TAPS>::l(i) + TapLog2<TAPS>::l(k);
-                        const u64 dd = sub2(xc, tv[k]);
-                        float a0, a1;
-                        up2(fma2(mul2(dd, dd), nhi, pk2(lk, lk)), a0, a1);
-                        const u64 gw = pk2(exp2_fast(a0), exp2_fast(a1));
-                        den = add2(den, gw);
-                        num = fma2(gw, dd, num);
-                    }
-                    if (++ws == p.slots) ws = 0;
-                }
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&empty[fslot]);  // the oldest window row is not needed any more
-                if (++fslot == p.slots) fslot = 0;
-                float n0, n1, d0, d1, x0v, x1v;
-                up2(num, n0, n1);
-                up2(den, d0, d1);
-                up2(xc, x0v, x1v);
-                const float c0 = fmaf(-n0, rcp_fast(d0), x0v), c1 = fmaf(-n1, rcp_fast(d1), x1v);  // one FFMA each, spelled out: left to
-            // the compiler's contraction, one kernel fused both halves of the pair and another only one (1-ulp differences)
-                if (act) {
-                    if (c_dst) {
-                        if (pol_keep)
-                            asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1, %2}, %3;" ::"l"(c_dst), "f"(c0), "f"(c1), "l"(pol_keep) : "memory");
-                        else
-                            *reinterpret_cast<float2 *>(c_dst) = make_float2(c0, c1);
-                    }
-                    if (w_dst) __stcs(reinterpret_cast<float2 *>(w_dst), make_float2(x0v - c0, x1v - c1));
-                }
-                if (c_dst) c_dst += c_step;
-                if (w_dst) w_dst += w_step;
-            }
-            if (++slot == p.slots) { slot = 0; parity ^= 1; }
-        }
-    };
-    if (__any_sync(0xffffffffu, rev != 0)) run(IC<1>{});
     else run(IC<0>{});
 }
 
@@ -1466,46 +991,9 @@ static bool plan_bilateral(ScaleParams &p, int taps, int esize, int batch) {
     return true;
 }
 
-// WB_K2_WINDOW in the environment: 0 selects the round-1 kernel (bilateral_pairs_kernel), 1 (default) the
-// register-window kernel, 3 the low-register streaming kernel (four blocks per SM) -- for A/B measurements and the
-// bit-identity test.
-static int k2_window_mode() {
-    const char *e = getenv("WB_K2_WINDOW");  // read on every call: the bit-identity test flips it inside one process
-    return (e && e[0] >= '0' && e[0] <= '9') ? e[0] - '0' : -1;
-}
-// Kernel actually launched.  Without WB_K2_WINDOW: the lean kernel (2), 8 - 15 % faster than the register-window kernel
-// in any of its block geometries at every scale (profiles/r2_bench_k2_lean.json; the geometries 4 .. 9 and the
-// prefetch variants all measured within 3 % of geometry 1, profiles/r2_bench_k2_scales.json).
-static int k2_mode_for(int taps, int d) {
-    const int wm = k2_window_mode();
-    if (wm >= 0) return wm;
-    (void)taps; (void)d;
-    return 2;  // the lean kernel (falls back to the window kernel, geometry 1, for what it does not take)
-}
-
 template <int TAPS, int DMODE>
-static int launch_bilateral_stream(const BilateralParams &bp, int batch, cudaStream_t st) {
-    auto kern = bilateral_stream_kernel<TAPS, DMODE>;
-    const ScaleParams &p = bp.sp;
-    const size_t smem = (size_t)p.slots * p.row_stride * sizeof(float) + 16 * (size_t)p.slots + kPairStats * (size_t)p.slots;
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
-        if (e != cudaSuccess) return (int)e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    dim3 grid((unsigned)((long long)p.n_strips * p.d * p.n_seg), (unsigned)batch);
-    return launch_pdl<BilateralParams>(kern, grid, dim3(256 + 32), smem, st, bp);
-}
-
-template <int TAPS, int DMODE, int WG = 0>
 static int launch_bilateral_window(const BilateralParams &bp, int batch, cudaStream_t st) {
-    void (*kern)(const BilateralParams) = bilateral_window_kernel<TAPS, DMODE, WG>;
-    if constexpr (WG == 3) kern = bilateral_window128_kernel<TAPS, DMODE>;
-    BilateralParams bq = bp;
-    if (const char *e = getenv("WB_K2_POLL")) bq.poll_ns = (unsigned)atoi(e);
+    auto kern = bilateral_window_kernel<TAPS, DMODE>;
     const ScaleParams &p = bp.sp;
     const size_t smem = (size_t)p.slots * p.row_stride * sizeof(float) + 16 * (size_t)p.slots;
     static bool configured[64] = {};
@@ -1517,7 +1005,7 @@ static int launch_bilateral_window(const BilateralParams &bp, int batch, cudaStr
         if (dev >= 0 && dev < 64) configured[dev] = true;
     }
     dim3 grid((unsigned)((long long)p.n_strips * p.d * p.n_seg), (unsigned)batch);
-    return launch_pdl<BilateralParams>(kern, grid, dim3(WindowGeom<WG>::THREADS), smem, st, bq);
+    return launch_pdl<BilateralParams>(kern, grid, dim3(256 + 32), smem, st, bp);
 }
 
 template <int TAPS, int DMODE, int LD = -1>
@@ -1543,75 +1031,33 @@ static bool k2_lean_ok(const ScaleParams &p) {
            (long long)p.d * p.c_pitch * 4 < (1LL << 31) && (long long)p.d * p.w_pitch * 4 < (1LL << 31);
 }
 
+// The fp32 pair path: the lean kernel, 8 - 15 % faster than the register-window kernel at every scale
+// (profiles/r2_bench_k2_lean.json), and the window kernel for the calls it declines.
 template <int TAPS, int DMODE>
-static int launch_bilateral_pairs(const BilateralParams &bp, int batch, cudaStream_t st) {
-    int wm = k2_mode_for(TAPS, bp.sp.d);
-    if (wm == 2) {
-        if (k2_lean_ok(bp.sp)) {
-            if constexpr (DMODE == 0) {
-                static int uni = -1;  // WB_K2_UNIFORM=1: one kernel for every dilation (uniform-register tap offsets)
-                if (uni < 0) {
-                    const char *e = getenv("WB_K2_UNIFORM");
-                    uni = (e && e[0] == '1') ? 1 : 0;
-                }
-                if (uni) return launch_bilateral_lean<TAPS, DMODE, -2>(bp, batch, st);
-            }
-            if constexpr (TAPS == 5 && DMODE == 0) {
-                // the B3spline scales of a dyadic cascade: dilation as a template parameter (immediate tap offsets)
-                switch (bp.sp.d) {
-                    case 2: return launch_bilateral_lean<TAPS, DMODE, 1>(bp, batch, st);
-                    case 4: return launch_bilateral_lean<TAPS, DMODE, 2>(bp, batch, st);
-                    case 8: return launch_bilateral_lean<TAPS, DMODE, 3>(bp, batch, st);
-                    case 16: return launch_bilateral_lean<TAPS, DMODE, 4>(bp, batch, st);
-                    case 32: return launch_bilateral_lean<TAPS, DMODE, 5>(bp, batch, st);
-                    case 64: return launch_bilateral_lean<TAPS, DMODE, 6>(bp, batch, st);
-                    case 128: return launch_bilateral_lean<TAPS, DMODE, 7>(bp, batch, st);
-                    case 256: return launch_bilateral_lean<TAPS, DMODE, 8>(bp, batch, st);
-                    case 512: return launch_bilateral_lean<TAPS, DMODE, 9>(bp, batch, st);
-                    default: break;
-                }
-            }
-            return launch_bilateral_lean<TAPS, DMODE>(bp, batch, st);
+static int launch_bilateral_pair_path(const BilateralParams &bp, int batch, cudaStream_t st) {
+    if (!k2_lean_ok(bp.sp)) return launch_bilateral_window<TAPS, DMODE>(bp, batch, st);
+    if constexpr (TAPS == 5 && DMODE == 0) {
+        // the B3spline scales of a dyadic cascade: dilation as a template parameter (immediate tap offsets)
+        switch (bp.sp.d) {
+            case 2: return launch_bilateral_lean<TAPS, DMODE, 1>(bp, batch, st);
+            case 4: return launch_bilateral_lean<TAPS, DMODE, 2>(bp, batch, st);
+            case 8: return launch_bilateral_lean<TAPS, DMODE, 3>(bp, batch, st);
+            case 16: return launch_bilateral_lean<TAPS, DMODE, 4>(bp, batch, st);
+            case 32: return launch_bilateral_lean<TAPS, DMODE, 5>(bp, batch, st);
+            case 64: return launch_bilateral_lean<TAPS, DMODE, 6>(bp, batch, st);
+            case 128: return launch_bilateral_lean<TAPS, DMODE, 7>(bp, batch, st);
+            case 256: return launch_bilateral_lean<TAPS, DMODE, 8>(bp, batch, st);
+            case 512: return launch_bilateral_lean<TAPS, DMODE, 9>(bp, batch, st);
+            default: break;
         }
-        wm = 1;
     }
-    if (wm == 1) return launch_bilateral_window<TAPS, DMODE>(bp, batch, st);
-    if (wm == 4) return launch_bilateral_window<TAPS, DMODE, 1>(bp, batch, st);
-    if (wm == 5) return launch_bilateral_window<TAPS, DMODE, 2>(bp, batch, st);
-    if (wm == 6) return launch_bilateral_window<TAPS, DMODE, 3>(bp, batch, st);
-    if (wm == 7) return launch_bilateral_window<TAPS, DMODE, 4>(bp, batch, st);
-    if (wm == 8) return launch_bilateral_window<TAPS, DMODE, 5>(bp, batch, st);
-    if (wm == 9) return launch_bilateral_window<TAPS, DMODE, 6>(bp, batch, st);
-    if (wm == 3) return launch_bilateral_stream<TAPS, DMODE>(bp, batch, st);
-    auto kern = bilateral_pairs_kernel<TAPS, DMODE>;
-    const ScaleParams &p = bp.sp;
-    const size_t smem = (size_t)p.slots * p.row_stride * sizeof(float) + 16 * (size_t)p.slots + kPairStats * (size_t)p.slots;
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
-        if (e != cudaSuccess) return (int)e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    dim3 grid((unsigned)((long long)p.n_strips * p.d * p.n_seg), (unsigned)batch);
-    return launch_pdl<BilateralParams>(kern, grid, dim3(256 + 32), smem, st, bp);
+    return launch_bilateral_lean<TAPS, DMODE>(bp, batch, st);
 }
 
-static int k2_window_mode();
-static int k2_mode_for(int taps, int d);
-static int k2_blocks_per_sm(int wm) { return wm == 3 ? 4 : ((wm == 5 || wm == 8) ? 1 : ((wm == 6 || wm == 7 || wm == 9) ? 3 : 2)); }
-static int k2_consumer_threads(int wm) { return (wm == 5 || wm == 8) ? 512 : ((wm == 6 || wm == 7 || wm == 9) ? 128 : 256); }
-static int k2_waves() {
-    const char *e = getenv("WB_K2_WAVES");
-    const int v = e ? atoi(e) : 0;
-    return v > 0 ? v : 4;
-}
-
-// Geometry for the fp32 pair kernel: 256 consumer threads x 2 pixels = 512-column strips.
-static bool plan_bilateral_pairs(ScaleParams &p, int taps, int batch, int occ, int cthreads = 256, long long stats = kPairStats) {
+// Geometry for the fp32 pair kernels: 256 consumer threads x 2 pixels = 512-column strips, two resident blocks per SM.
+static bool plan_bilateral_pair_path(ScaleParams &p, int taps, int batch) {
     const int c = taps / 2;
-    p.wt = 2 * cthreads;
+    p.wt = 512;
     p.n_strips = (p.W + p.wt - 1) / p.wt;
     p.halo_al = round_up(c * p.d, 4);
     long long rs = (long long)p.wt + 2LL * p.halo_al;
@@ -1619,15 +1065,14 @@ static bool plan_bilateral_pairs(ScaleParams &p, int taps, int batch, int occ, i
     p.row_stride = (int)rs;
     int slots = taps + 3;
     const int min_slots = taps + 1;
-    // `occ` resident blocks per SM (register-limited: 2, or 4 for the streaming kernel): keep a block under that share
-    // of the shared memory if possible
-    while (slots > min_slots && (long long)slots * (p.row_stride * 4 + 16LL + stats) > kMaxSmem / occ - 1024) --slots;
-    if ((long long)slots * (p.row_stride * 4 + 16LL + stats) > kMaxSmem) return false;
+    // keep a block under half of the shared memory if possible
+    while (slots > min_slots && (long long)slots * (p.row_stride * 4 + 16LL) > kMaxSmem / 2 - 1024) --slots;
+    if ((long long)slots * (p.row_stride * 4 + 16LL) > kMaxSmem) return false;
     p.slots = slots;
     const int n_max = (p.H + p.d - 1) / p.d;
     // Compute-bound kernel: about 4 waves of 2 resident blocks per SM; halo rows only cost L2 reads.
     const long long chains = (long long)p.n_strips * (p.d < p.H ? p.d : p.H) * batch;
-    const long long target = (long long)k2_waves() * occ * device_sm_count();
+    const long long target = 4LL * 2 * device_sm_count();
     long long per_chain = (target + chains - 1) / chains;
     if (per_chain < 1) per_chain = 1;
     int seg = (int)((n_max + per_chain - 1) / per_chain);
@@ -1644,10 +1089,8 @@ static int dispatch_bilateral(BilateralParams &bp, int batch, cudaStream_t st) {
     ScaleParams &p = bp.sp;
     if constexpr (sizeof(T) == 4) {
         // packed fp32x2 pair kernel: dilation 1 or even (every scale of a dyadic cascade)
-        if (fast_path_ok(p, TAPS, 4) && (p.d == 1 || p.d % 2 == 0) &&
-            plan_bilateral_pairs(p, TAPS, batch, k2_blocks_per_sm(k2_mode_for(TAPS, p.d)), k2_consumer_threads(k2_mode_for(TAPS, p.d)),
-                                 (k2_mode_for(TAPS, p.d) == 0 || k2_mode_for(TAPS, p.d) == 3) ? kPairStats : 0))
-            return p.d == 1 ? launch_bilateral_pairs<TAPS, 1>(bp, batch, st) : launch_bilateral_pairs<TAPS, 0>(bp, batch, st);
+        if (fast_path_ok(p, TAPS, 4) && (p.d == 1 || p.d % 2 == 0) && plan_bilateral_pair_path(p, TAPS, batch))
+            return p.d == 1 ? launch_bilateral_pair_path<TAPS, 1>(bp, batch, st) : launch_bilateral_pair_path<TAPS, 0>(bp, batch, st);
     }
     if (fast_path_ok(p, TAPS, (int)sizeof(T)) && plan_bilateral(p, TAPS, (int)sizeof(T), batch)) {
         const int dmode = (p.d % V == 0) ? 0 : p.d;
@@ -1749,7 +1192,6 @@ int wb_atrous_scale_bilateral(const void *in, void *out_c, void *out_w, int batc
     p.c_pitch = out_c_pitch; p.c_bstride = out_c_bstride;
     p.w_pitch = out_w_pitch; p.w_bstride = out_w_bstride;
     bp.var_factor = var_factor;
-    bp.var_factor_f = (float)var_factor;
     bp.var_factor_f = (float)var_factor;
     p.l2_hints = wb::l2_hints_enabled();
     cudaStream_t st = (cudaStream_t)stream;
