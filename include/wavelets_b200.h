@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define WB_ABI_VERSION 1
+#define WB_ABI_VERSION 2
 #define WB_MAX_PEERS 16 /* ranks of one NVLink domain whose band buffers wb_atrous_scale_band_p2p can address */
 
 enum { WB_F32 = 0, WB_F64 = 1 };
@@ -204,6 +204,22 @@ int wb_wow_whiten_scale(const void *w_raw, void *out, int batch, int H, int W,
                         double noise_host, const double *noise_dev, double weight, void *stream);
 
 /*
+ * wb_wow_whiten_scale with a PER-PIXEL noise map (watroo/wavelets.py:133-141 with an array `noise`), per pixel:
+ *     tmp = the sig_mode 0 whitening of w_raw                      (rounded to the plane dtype)
+ *     thr = (double)((T)sigma * map) * sigma_e
+ *     s   = soft ? erf(|(double)w_raw / thr|) : (|(double)w_raw| > thr ? 1 : 0)      (float64)
+ *     out = (T)((double)tmp * s)
+ * Bit-identical to wb_wow_whiten_scale (sig_mode 0) -> wb_significance (same map) -> the float64 product.  `noise_map`
+ * has the plane dtype; its element (frame, y, x) is at frame * map_bstride + y * map_pitch + x (map_bstride 0: one map
+ * for every frame).  sigma == 0 is rejected (WB_EINVAL_ARG): such scales take wb_wow_whiten_scale with sig_mode 0.
+ * `out` must alias neither `w_raw` nor `noise_map`.
+ */
+int wb_wow_whiten_scale_map(const void *w_raw, void *out, const void *noise_map, int batch, int H, int W,
+                            long long in_pitch, long long in_bstride, long long out_pitch, long long out_bstride,
+                            long long map_pitch, long long map_bstride, int scale, int taps, int dtype, int soft,
+                            double sigma, double sigma_e, double weight, void *stream);
+
+/*
  * One WOW scale fused in a single pass: the smooth + subtraction of wb_atrous_scale (watroo/wavelets.py:35-45, :442)
  * AND the whitening of wb_wow_whiten_scale (watroo/utils.py:177,193-203) without ever writing the raw detail plane:
  *     out_c = S_scale[in]                                 (c_{s+1}, needed by the next scale)
@@ -337,6 +353,19 @@ int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, voi
                    int batch, int H, int W, int n_scales, int taps, int dtype, const double *weights, const double *sigmas,
                    const double *sigma_e, const double *var_factors, int soft, double noise_host, double *noise_dev,
                    int estimate_noise, void *workspace, size_t workspace_bytes, void *stream);
+
+/*
+ * wb_wow_cascade with the noise taken from a per-pixel map (no MAD estimate).  Every scale takes two passes: K1
+ * (wb_atrous_scale) or K2 (wb_atrous_scale_bilateral) writes the raw detail plane into scratch, then
+ * wb_wow_whiten_scale_map whitens it where sigmas[s] != 0 and wb_wow_whiten_scale (sig_mode 0) elsewhere; moments,
+ * rescale and synthesis as in wb_wow_cascade.  Bit-identical to issuing those calls one by one.  Map layout as in
+ * wb_wow_whiten_scale_map; the other arguments and the workspace as in wb_wow_cascade.
+ */
+int wb_wow_cascade_map(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch, void *recon,
+                       int batch, int H, int W, int n_scales, int taps, int dtype, const double *weights,
+                       const double *sigmas, const double *sigma_e, const double *var_factors, int soft,
+                       const void *noise_map, long long map_pitch, long long map_bstride, void *workspace,
+                       size_t workspace_bytes, void *stream);
 
 /*
  * n standard-normal float32 samples (Philox4x32-10 + Box-Muller), the device stand-in for

@@ -19,7 +19,7 @@ WB_F32, WB_F64 = 0, 1
 WB_TRIANGLE, WB_B3SPLINE = 3, 5
 WB_BORDER_SYMMETRIC, WB_BORDER_MIRROR = 0, 1
 WB_ENOT_FUSABLE = -7
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 _lock = threading.Lock()
 _lib = None
@@ -57,6 +57,8 @@ SIGNATURES = {
                                               _c_dbl, _c_vp]),
     "wb_wow_whiten_scale": (_c_int, [_c_vp, _c_vp, _c_int, _c_int, _c_int, _c_ll, _c_ll, _c_ll, _c_ll, _c_int, _c_int,
                                      _c_int, _c_int, _c_dbl, _c_dbl, _c_dbl, _c_vp, _c_dbl, _c_vp]),
+    "wb_wow_whiten_scale_map": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_ll, _c_ll, _c_ll, _c_ll, _c_ll,
+                                         _c_ll, _c_int, _c_int, _c_int, _c_int, _c_dbl, _c_dbl, _c_dbl, _c_vp]),
     "wb_wow_scale_path": (_c_int, [_c_int, _c_int, _c_int, _c_ll, _c_ll, _c_ll, _c_int, _c_int, _c_int, _c_vp, _c_vp,
                                    _c_vp]),
     "wb_wow_scale": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_ll, _c_ll, _c_ll, _c_ll, _c_ll, _c_ll,
@@ -75,6 +77,9 @@ SIGNATURES = {
     "wb_wow_cascade": (_c_int, [_c_vp, _c_ll, _c_ll, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int,
                                 ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl),
                                 ctypes.POINTER(_c_dbl), _c_int, _c_dbl, _c_vp, _c_int, _c_vp, _c_sz, _c_vp]),
+    "wb_wow_cascade_map": (_c_int, [_c_vp, _c_ll, _c_ll, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int,
+                                    _c_int, ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl),
+                                    ctypes.POINTER(_c_dbl), _c_int, _c_vp, _c_ll, _c_ll, _c_vp, _c_sz, _c_vp]),
     "wb_filter2d": (_c_int, [_c_vp, _c_vp, _c_int, _c_int, _c_ll, _c_ll, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_vp]),
     "wb_atrous_axis": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_ll, _c_ll, _c_ll, _c_int, _c_int, _c_int, _c_int, _c_vp]),
 }

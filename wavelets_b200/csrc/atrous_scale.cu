@@ -24,7 +24,8 @@
 
 namespace wb {
 
-template <typename T, int TAPS, int DMODE, int NG, int OP>
+// MAP (OP_WHITEN only): the noise-map mode of the epilogue (sig_mode == SIG_MAP, see whiten.cuh).
+template <typename T, int TAPS, int DMODE, int NG, int OP, bool MAP = false>
 __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
     constexpr int V = VecOf<T>::V;
     constexpr int C = TAPS / 2;
@@ -105,7 +106,14 @@ __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
     int out_row = (int)orow;  // band row of the next output
 
     WhitenEpilogue<T> epi;
-    if constexpr (OP == OP_WHITEN) epi.init(p, frame);
+    if constexpr (OP == OP_WHITEN) epi.template init<MAP>(p, frame);
+    // map mode: row pointer into the noise map (whole-frame launches: no row offset)
+    const T *m_ptr = nullptr;
+    long long m_step = 0;
+    if constexpr (MAP) {
+        m_ptr = reinterpret_cast<const T *>(p.noise_map) + (long long)frame * p.map_bstride + orow * p.map_pitch;
+        m_step = (long long)p.d * p.map_pitch;
+    }
     const uint64_t pol_keep = policy_evict_last();  // c_{s+1}: the next scale reads it back
     const bool hints = p.l2_hints != 0;
 
@@ -164,14 +172,21 @@ __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
                         if (act[q]) st_vec_cs(w_ptr + xg[q], raw);
                     }
                 } else {
-                    Pack<T, V> raw = lds_vec<T>(crow_addr + xb[q]);
+                    const Pack<T, V> raw = lds_vec<T>(crow_addr + xb[q]);
+                    Pack<T, V> out;
 #pragma unroll
-                    for (int e = 0; e < V; ++e) raw.v[e] = epi.apply(raw.v[e], cv[q].v[e]);
-                    if (act[q]) st_vec_cs(w_ptr + xg[q], raw);
+                    for (int e = 0; e < V; ++e) out.v[e] = epi.apply(raw.v[e], cv[q].v[e]);
+                    if (MAP && act[q]) {
+                        const Pack<T, V> nz = ld_vec_stream(m_ptr + xg[q]);
+#pragma unroll
+                        for (int e = 0; e < V; ++e) out.v[e] = epi.map_sig(raw.v[e], out.v[e], nz.v[e]);
+                    }
+                    if (act[q]) st_vec_cs(w_ptr + xg[q], out);
                 }
             }
             if (c_ptr) c_ptr += c_step;
             if (w_ptr) w_ptr += w_step;
+            if constexpr (MAP) m_ptr += m_step;
             out_row += p.d;
         }
         if (j >= C) {
@@ -281,7 +296,7 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
     const PackedTaps<TAPS, T> H;
     const uint64_t pol_keep = policy_evict_last();  // c_{s+1}: the next scale reads it back
     WhitenEpilogue<T> epi;
-    if constexpr (OP == OP_WHITEN) epi.init(p, frame);
+    if constexpr (OP == OP_WHITEN) epi.template init<MODE == SIG_MAP>(p, frame);
 
     constexpr int NTAP = PAIR ? 1 : NG, NPT = TAPS + PAIR;
     uint32_t own[NG], tap[NTAP][NV], ptap[NPT];
@@ -337,6 +352,13 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
     if (c_ptr) c_ptr += (long long)frame * p.c_bstride + (orow + p.row_off_c) * p.c_pitch + xg0;
     if (w_ptr) w_ptr += (long long)frame * p.w_bstride + (orow + p.row_off_w) * p.w_pitch + xg0;
     const long long c_step = (long long)p.d * p.c_pitch, w_step = (long long)p.d * p.w_pitch;
+    // map mode: the noise-map vectors of the output vectors (whole-frame launches: no row offset)
+    const T *m_ptr = nullptr;
+    long long m_step = 0;
+    if constexpr (MODE == SIG_MAP) {
+        m_ptr = reinterpret_cast<const T *>(p.noise_map) + (long long)frame * p.map_bstride + orow * p.map_pitch + xg0;
+        m_step = (long long)p.d * p.map_pitch;
+    }
     const bool has_c = c_ptr != nullptr, has_w = w_ptr != nullptr;
     const bool pushing = (p.push_up != nullptr) | (p.push_dn != nullptr);
     int out_row = (int)orow;  // band row of the next output
@@ -380,11 +402,20 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
 #pragma unroll
                 for (int q = 0; q < NG; ++q) {
                     P4 raw = lds_p4_imm<SC * RB>(own[q] + hc);
-                    raw.lo = epi.template apply_lane<MODE>(raw.lo, cv[q].lo);
-                    raw.hi = epi.template apply_lane<MODE>(raw.hi, cv[q].hi);
-                    if (act[q]) stg_p4_cs(w_ptr + q * q_off, raw);
+                    P4 out;
+                    out.lo = epi.template apply_lane<MODE>(raw.lo, cv[q].lo);
+                    out.hi = epi.template apply_lane<MODE>(raw.hi, cv[q].hi);
+                    if constexpr (MODE == SIG_MAP) {
+                        if (act[q]) {
+                            const P4 nz = ldg_p4_stream(m_ptr + q * q_off);
+                            out.lo = epi.map_lane(raw.lo, out.lo, nz.lo);
+                            out.hi = epi.map_lane(raw.hi, out.hi, nz.hi);
+                        }
+                    }
+                    if (act[q]) stg_p4_cs(w_ptr + q * q_off, out);
                 }
                 w_ptr += w_step;
+                if constexpr (MODE == SIG_MAP) m_ptr += m_step;
             } else {
 #pragma unroll
             for (int q = 0; q < NG; ++q) {
@@ -434,7 +465,7 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
 }
 
 // Generic path: one thread per output pixel, full modular reflection, any shape / alignment.
-template <typename T, int TAPS, int OP>
+template <typename T, int TAPS, int OP, bool MAP = false>
 __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p) {
     constexpr int C = TAPS / 2;
     const long long n = (long long)p.H * p.W;
@@ -443,7 +474,7 @@ __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p
     T *out_c = reinterpret_cast<T *>(p.out_c);
     T *out_w = reinterpret_cast<T *>(p.out_w);
     WhitenEpilogue<T> epi;
-    if constexpr (OP == OP_WHITEN) epi.init(p, frame);
+    if constexpr (OP == OP_WHITEN) epi.template init<MAP>(p, frame);
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n;
          idx += (long long)gridDim.x * blockDim.x) {
         const int y = (int)(idx / p.W), x = (int)(idx % p.W);
@@ -474,7 +505,11 @@ __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p
             }
             if (out_w) out_w[(long long)frame * p.w_bstride + ((long long)y + p.row_off_w) * p.w_pitch + x] = raw - acc;
         } else {
-            out_w[(long long)frame * p.w_bstride + ((long long)y + p.row_off_w) * p.w_pitch + x] = epi.apply(raw, acc);
+            T v = epi.apply(raw, acc);
+            if constexpr (MAP)
+                v = epi.map_sig(raw, v, reinterpret_cast<const T *>(p.noise_map)[(long long)frame * p.map_bstride +
+                                                                                  (long long)y * p.map_pitch + x]);
+            out_w[(long long)frame * p.w_bstride + ((long long)y + p.row_off_w) * p.w_pitch + x] = v;
         }
     }
 }
@@ -485,9 +520,9 @@ __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p
 K1Config g_override[32];
 bool g_override_set[32];
 
-template <typename T, int TAPS, int DMODE, int NG, int OP>
+template <typename T, int TAPS, int DMODE, int NG, int OP, bool MAP>
 static int launch_rows(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
-    auto kern = atrous_rows_kernel<T, TAPS, DMODE, NG, OP>;
+    auto kern = atrous_rows_kernel<T, TAPS, DMODE, NG, OP, MAP>;
     const size_t smem = (size_t)p.slots * p.row_stride * sizeof(T) + 16 * (size_t)p.slots;
     static bool configured[64] = {};  // per instantiation, per device
     int dev = 0;
@@ -610,6 +645,7 @@ static int launch_rows_lean_strip_m(const ScaleParams &p, int batch, int nt, cud
 template <typename T, int TAPS, int DMODE, int OP, int PAIR>
 static int launch_rows_lean_strip(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
     if constexpr (OP == OP_WHITEN) {
+        if (p.sig_mode == SIG_MAP) return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, SIG_MAP, PAIR>(p, batch, nt, st);
         if constexpr (sizeof(T) == 4) {
             if (p.sig_mode == 1) return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, 1, PAIR>(p, batch, nt, st);
         }
@@ -621,6 +657,7 @@ static int launch_rows_lean_strip(const ScaleParams &p, int batch, int nt, cudaS
 template <typename T, int TAPS, int OP>
 static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
     constexpr int V = VecOf<T>::V;
+    const bool map = OP == OP_WHITEN && p.sig_mode == SIG_MAP;
     K1Config cfg;
     if (fast_path_ok(p, TAPS, (int)sizeof(T)) && plan_fast(p, TAPS, (int)sizeof(T), batch, scale, &cfg, OP == OP_TRANSFORM)) {
         const int dmode = (p.d % V == 0) ? 0 : p.d;
@@ -653,8 +690,9 @@ static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
                 !(scale < 32 && g_override_set[scale])) {
 #define WB_LEANW_P(DM, PR)                                                                                        \
     (p.sig_mode == 0 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 0, PR>(p, batch, cfg.nt, st)                    \
-                     : (p.sig_mode == 1 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 1, PR>(p, batch, cfg.nt, st) \
-                                        : launch_rows_lean<TAPS, DM, true, OP_WHITEN, 2, PR>(p, batch, cfg.nt, st)))
+     : p.sig_mode == 1 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 1, PR>(p, batch, cfg.nt, st)                  \
+     : p.sig_mode == 2 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 2, PR>(p, batch, cfg.nt, st)                  \
+                       : launch_rows_lean<TAPS, DM, true, OP_WHITEN, SIG_MAP, PR>(p, batch, cfg.nt, st))
 #define WB_LEANW(DM) WB_LEANW_P(DM, 0)
                 if (dmode == 0) {
                     const int pair = k1_pair_step(TAPS, p.d, p.W, cfg.nt);
@@ -694,21 +732,24 @@ static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
                 }
             }
         }
-#define WB_LAUNCH(DM)                                                                   \
-    (cfg.ng == 1 ? launch_rows<T, TAPS, DM, 1, OP>(p, batch, cfg.nt, st)                \
-                 : launch_rows<T, TAPS, DM, 2, OP>(p, batch, cfg.nt, st))
+#define WB_LAUNCH_M(DM, M)                                                              \
+    (cfg.ng == 1 ? launch_rows<T, TAPS, DM, 1, OP, M>(p, batch, cfg.nt, st)             \
+                 : launch_rows<T, TAPS, DM, 2, OP, M>(p, batch, cfg.nt, st))
+#define WB_LAUNCH(DM) (map ? WB_LAUNCH_M(DM, OP == OP_WHITEN) : WB_LAUNCH_M(DM, false))
         if (dmode == 0) return WB_LAUNCH(0);
         if (dmode == 1) return WB_LAUNCH(1);
         if constexpr (V == 4) {
             if (dmode == 2) return WB_LAUNCH(2);
         }
 #undef WB_LAUNCH
+#undef WB_LAUNCH_M
     }
     const long long n = (long long)p.H * p.W;
     long long blocks = (n + 255) / 256;
     const long long cap = 32LL * device_sm_count();
     if (blocks > cap) blocks = cap;
-    atrous_generic_kernel<T, TAPS, OP><<<dim3((unsigned)blocks, (unsigned)batch), 256, 0, st>>>(p);
+    if (map) atrous_generic_kernel<T, TAPS, OP, OP == OP_WHITEN><<<dim3((unsigned)blocks, (unsigned)batch), 256, 0, st>>>(p);
+    else atrous_generic_kernel<T, TAPS, OP><<<dim3((unsigned)blocks, (unsigned)batch), 256, 0, st>>>(p);
     return launch_status();
 }
 
@@ -901,6 +942,27 @@ int wb_wow_whiten_scale(const void *w_raw, void *out, int batch, int H, int W, l
     p.w_pitch = out_pitch; p.w_bstride = out_bstride;
     p.sig_mode = sig_mode; p.sigma = sigma; p.sigma_e = sigma_e;
     p.noise_host = noise_host; p.noise_dev = noise_dev; p.weight = weight;
+    p.l2_hints = wb::l2_hints_enabled();
+    return wb::dispatch_typed<wb::OP_WHITEN>(p, batch, scale, taps, dtype, (cudaStream_t)stream);
+}
+
+int wb_wow_whiten_scale_map(const void *w_raw, void *out, const void *noise_map, int batch, int H, int W,
+                            long long in_pitch, long long in_bstride, long long out_pitch, long long out_bstride,
+                            long long map_pitch, long long map_bstride, int scale, int taps, int dtype, int soft,
+                            double sigma, double sigma_e, double weight, void *stream) {
+    int rc = wb::check_common(batch, H, W, taps, dtype);
+    if (rc) return rc;
+    if (scale < 0 || scale > 30) return WB_EINVAL_SCALE;
+    if (!w_raw || !out || !noise_map || w_raw == out || noise_map == out) return WB_EINVAL_POINTER;
+    if (in_pitch < W || out_pitch < W || map_pitch < W || map_bstride < 0 || sigma == 0.0) return WB_EINVAL_ARG;
+    wb::ScaleParams p;
+    memset(&p, 0, sizeof(p));
+    p.in = w_raw; p.out_c = nullptr; p.out_w = out;
+    p.H = H; p.W = W; p.d = 1 << scale; p.Hg = H;
+    p.in_pitch = in_pitch; p.in_bstride = in_bstride;
+    p.w_pitch = out_pitch; p.w_bstride = out_bstride;
+    p.sig_mode = wb::SIG_MAP; p.sigma = sigma; p.sigma_e = sigma_e; p.weight = weight;
+    p.noise_map = noise_map; p.map_pitch = map_pitch; p.map_bstride = map_bstride; p.map_soft = soft ? 1 : 0;
     p.l2_hints = wb::l2_hints_enabled();
     return wb::dispatch_typed<wb::OP_WHITEN>(p, batch, scale, taps, dtype, (cudaStream_t)stream);
 }

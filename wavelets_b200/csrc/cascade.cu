@@ -2,7 +2,8 @@
 // plain or the bilateral cascade, i.e. what wavelets_b200.utils._wow_stack issues scale by scale -- per scale wb_wow_scale
 // (or, for bilateral scales, where the fused kernel declines, or when the MAD noise has to be estimated from the raw w_0
 // first: wb_atrous_scale / wb_atrous_scale_bilateral [+ wb_abs_median] + wb_wow_whiten_scale), then wb_plane_moments +
-// wb_residual_rescale of the residual plane and wb_synthesis.  Host code
+// wb_residual_rescale of the residual plane and wb_synthesis.  wb_wow_cascade_map runs the same loop with a per-pixel
+// noise map: two passes at every scale, the thresholded ones whitened by wb_wow_whiten_scale_map.  Host code
 // only: it exists because a 512^2 .. 2048^2 frame is finished on the device long before a Python loop has issued its
 // fifteen launches (0.27 - 0.30 ms of interpreter and ctypes time per wow() call, measured; profiles/r2_sizes.json).
 #include "common.cuh"
@@ -11,28 +12,32 @@ namespace wb {
 
 static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
 
-}  // namespace wb
+// Where the thresholds of a cascade come from: a host scalar, device scalars per frame (noise_dev, given or estimated
+// here when `estimate`), or a per-pixel noise map (map != nullptr; every scale then takes the two-pass route).
+struct CascadeNoise {
+    double host;
+    double *dev;
+    int estimate;
+    const void *map;
+    long long map_pitch, map_bstride;
+};
 
-extern "C" {
-
-size_t wb_wow_cascade_workspace_bytes(int dtype, int batch, long long n) {
-    if (batch < 1) batch = 1;
-    return wb::align256(wb_abs_median_workspace_bytes(dtype, batch, n)) + wb::align256(wb_plane_moments_workspace_bytes(batch)) +
-           wb::align256((size_t)batch * 3 * sizeof(double));
-}
-
-int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch, void *recon,
-                   int batch, int H, int W, int n_scales, int taps, int dtype, const double *weights, const double *sigmas,
-                   const double *sigma_e, const double *var_factors, int soft, double noise_host, double *noise_dev,
-                   int estimate_noise, void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = wb::check_common(batch, H, W, taps, dtype);
+static int wow_cascade_impl(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch,
+                            void *recon, int batch, int H, int W, int n_scales, int taps, int dtype,
+                            const double *weights, const double *sigmas, const double *sigma_e,
+                            const double *var_factors, int soft, const CascadeNoise &nz, void *workspace,
+                            size_t workspace_bytes, void *stream) {
+    int rc = check_common(batch, H, W, taps, dtype);
     if (rc) return rc;
     if (n_scales < 1 || n_scales > 30) return WB_EINVAL_SCALE;
     if (!in || !planes || !scratch || !recon || !weights || !sigmas || !sigma_e || !workspace) return WB_EINVAL_POINTER;
-    if (estimate_noise && !noise_dev) return WB_EINVAL_POINTER;
+    if (nz.estimate && !nz.dev) return WB_EINVAL_POINTER;
     const long long n = (long long)H * W;
     if (workspace_bytes < wb_wow_cascade_workspace_bytes(dtype, batch, n)) return WB_EINVAL_ARG;
-    const size_t es = (size_t)wb::dtype_size(dtype);
+    const double noise_host = nz.host;
+    double *noise_dev = nz.dev;
+    const int estimate_noise = nz.estimate;
+    const size_t es = (size_t)dtype_size(dtype);
     const int L = n_scales;
     char *pl = reinterpret_cast<char *>(planes);    // (batch, L + 1, H, W)
     char *sc = reinterpret_cast<char *>(scratch);   // (3, batch, H, W): two ping-pong smooth planes, one raw detail plane
@@ -40,10 +45,10 @@ int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, voi
     auto plane = [&](int s) { return pl + (size_t)s * (size_t)n * es; };
     auto scr = [&](int i) { return sc + (size_t)i * (size_t)batch * (size_t)n * es; };
     char *ws = reinterpret_cast<char *>(workspace);
-    const size_t med_bytes = wb::align256(wb_abs_median_workspace_bytes(dtype, batch, n));
+    const size_t med_bytes = align256(wb_abs_median_workspace_bytes(dtype, batch, n));
     void *med_ws = ws;
     void *mom_ws = ws + med_bytes;
-    double *mom = reinterpret_cast<double *>(ws + med_bytes + wb::align256(wb_plane_moments_workspace_bytes(batch)));
+    double *mom = reinterpret_cast<double *>(ws + med_bytes + align256(wb_plane_moments_workspace_bytes(batch)));
 
     bool have_noise = !estimate_noise;  // a given noise: host scalar, or device scalars when noise_dev != NULL
     const double *nz_dev = estimate_noise ? nullptr : noise_dev;
@@ -57,8 +62,9 @@ int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, voi
         const double sg = need_sig ? sigmas[s] : 0.0, se = need_sig ? sigma_e[s] : 1.0;
         // bilateral scale (var_factors[s] = sigma_bilateral[s]^2 (s + 1 if bilateral_scaling else 1)): the range-weighted
         // gather K2 writes the raw detail plane, K3 whitens it
+        // a noise map: two passes at every scale (the fused kernel has no map mode), K3 with the map where sigmas[s] != 0
         const bool bilateral = var_factors != nullptr;
-        bool two_pass = bilateral, median_of_raw = false;
+        bool two_pass = bilateral || nz.map, median_of_raw = false;
         if (need_sig && !have_noise) {
             if (s == 0) {
                 two_pass = median_of_raw = true;  // from the raw w_0: a grid-wide dependency inside the scale
@@ -88,8 +94,13 @@ int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, voi
                 have_noise = true;
                 nz_dev = noise_dev;
             }
-            rc = wb_wow_whiten_scale(raw, plane(s), batch, H, W, W, n, W, plane_bs, s, taps, dtype, mode, sg, se,
-                                     need_sig ? noise_host : 0.0, need_sig ? nz_dev : nullptr, weights[s], stream);
+            if (nz.map && need_sig)
+                rc = wb_wow_whiten_scale_map(raw, plane(s), nz.map, batch, H, W, W, n, W, plane_bs, nz.map_pitch,
+                                             nz.map_bstride, s, taps, dtype, soft, sg, se, weights[s], stream);
+            else
+                rc = wb_wow_whiten_scale(raw, plane(s), batch, H, W, W, n, W, plane_bs, s, taps, dtype, mode, sg,
+                                         se, need_sig ? noise_host : 0.0, need_sig ? nz_dev : nullptr, weights[s],
+                                         stream);
             if (rc) return rc;
         }
         src = dst_c;
@@ -102,6 +113,37 @@ int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, voi
     rc = wb_residual_rescale(plane(L), n, batch, plane_bs, dtype, mom, weights[L], stream);
     if (rc) return rc;
     return wb_synthesis(planes, L + 1, n, n, batch, plane_bs, recon, n, dtype, stream);
+}
+
+}  // namespace wb
+
+extern "C" {
+
+size_t wb_wow_cascade_workspace_bytes(int dtype, int batch, long long n) {
+    if (batch < 1) batch = 1;
+    return wb::align256(wb_abs_median_workspace_bytes(dtype, batch, n)) + wb::align256(wb_plane_moments_workspace_bytes(batch)) +
+           wb::align256((size_t)batch * 3 * sizeof(double));
+}
+
+int wb_wow_cascade(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch, void *recon,
+                   int batch, int H, int W, int n_scales, int taps, int dtype, const double *weights, const double *sigmas,
+                   const double *sigma_e, const double *var_factors, int soft, double noise_host, double *noise_dev,
+                   int estimate_noise, void *workspace, size_t workspace_bytes, void *stream) {
+    const wb::CascadeNoise nz{noise_host, noise_dev, estimate_noise, nullptr, 0, 0};
+    return wb::wow_cascade_impl(in, in_pitch, in_bstride, planes, scratch, recon, batch, H, W, n_scales, taps, dtype,
+                                weights, sigmas, sigma_e, var_factors, soft, nz, workspace, workspace_bytes, stream);
+}
+
+int wb_wow_cascade_map(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch, void *recon,
+                       int batch, int H, int W, int n_scales, int taps, int dtype, const double *weights,
+                       const double *sigmas, const double *sigma_e, const double *var_factors, int soft,
+                       const void *noise_map, long long map_pitch, long long map_bstride, void *workspace,
+                       size_t workspace_bytes, void *stream) {
+    if (!noise_map) return WB_EINVAL_POINTER;
+    if (map_pitch < W || map_bstride < 0) return WB_EINVAL_ARG;
+    const wb::CascadeNoise nz{0.0, nullptr, 0, noise_map, map_pitch, map_bstride};
+    return wb::wow_cascade_impl(in, in_pitch, in_bstride, planes, scratch, recon, batch, H, W, n_scales, taps, dtype,
+                                weights, sigmas, sigma_e, var_factors, soft, nz, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -77,6 +77,21 @@ template <typename T> struct Taps<T, 5> {
     }
 };
 
+// threshold = (sigma * noise) * sigma_e evaluated like NumPy >= 2: with a scalar noise everything is float64; with a
+// per-pixel noise map of the plane dtype, `sigma * noise` stays in that dtype and only the product with the
+// float64 sigma_e is promoted (watroo/wavelets.py:137,141).  The one definition used by wb_significance,
+// wb_denoise_plane and the map mode of the whitening kernels (whiten.cuh).
+template <typename T>
+__device__ __forceinline__ double map_threshold(T noise, double sigma, double sigma_e) {
+    return (double)((T)sigma * noise) * sigma_e;
+}
+template <typename T>
+__device__ __forceinline__ double threshold_at(const T *noise_map, long long i, double sigma, double scalar,
+                                               double sigma_e) {
+    if (noise_map) return map_threshold<T>(noise_map[i], sigma, sigma_e);
+    return (sigma * scalar) * sigma_e;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // mbarrier + TMA bulk-copy PTX (sm_90+; on sm_100a the copy shows up in SASS as UBLKCP)
 // ---------------------------------------------------------------------------------------------------------------

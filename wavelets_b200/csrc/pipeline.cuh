@@ -29,7 +29,7 @@ struct ScaleParams {
     int row_stride;  // elements per ring slot
     int halo_al;     // x halo kept in shared memory on each side of a strip (multiple of V)
     // --- whitening epilogue (OP_WHITEN): out_w = significance(raw) * raw * (weight / sqrt(max(S[raw^2], 1e-15)))
-    int sig_mode;              // 0: no thresholding, 1: soft (erf), 2: hard
+    int sig_mode;              // 0: no thresholding, 1: soft (erf), 2: hard, SIG_MAP: per-pixel noise map
     double sigma, sigma_e;     // threshold = (sigma * noise) * sigma_e   (watroo/wavelets.py:137,141)
     double noise_host;         // used when noise_dev == nullptr
     const double *noise_dev;   // device scalar per frame (from wb_abs_median), or nullptr
@@ -49,6 +49,12 @@ struct ScaleParams {
     // [0, push_up_rows) go up, rows [push_dn_from, H) go down.  nullptr: no neighbour on that side.
     void *push_up, *push_dn;
     int push_up_rows, push_dn_from;
+    // --- whitening with a noise map (sig_mode == SIG_MAP, wb_wow_whiten_scale_map): map of the plane dtype, element
+    // (frame, y, x) at frame * map_bstride + y * map_pitch + x (map_bstride 0: one map for every frame); map_soft
+    // selects erf (1) or the hard mask (0).  Last, so that the parameter offsets of the other kernels stay put.
+    const void *noise_map;
+    long long map_pitch, map_bstride;
+    int map_soft;
 };
 
 // Second store of a c_{s+1} vector into the neighbours' halo zones (see ScaleParams::push_up).  `c_ptr` points at the
@@ -71,6 +77,7 @@ __device__ __forceinline__ const T *input_row(const ScaleParams &p, long long gy
 }
 
 enum { OP_TRANSFORM = 0, OP_WHITEN = 1 };
+enum { SIG_MAP = 3 };  // ScaleParams::sig_mode of the noise-map whitening (wb_wow_whiten_scale_map)
 
 // Per-thread, per-column-group tap plan, computed ONCE per thread block: the shared-memory element offset of the
 // aligned vector that holds each tap (relative to the start of a staged row) and whether that vector has to be read
@@ -524,6 +531,8 @@ inline bool fast_path_ok(const ScaleParams &p, int taps, int esize) {
     if (p.in_pitch % V || p.in_bstride % V || !aligned16(p.in)) return false;
     if (p.out_c && (p.c_pitch % V || p.c_bstride % V || !aligned16(p.out_c))) return false;
     if (p.out_w && (p.w_pitch % V || p.w_bstride % V || !aligned16(p.out_w))) return false;
+    // the map is read in the vectors of the output
+    if (p.noise_map && (p.map_pitch % V || p.map_bstride % V || !aligned16(p.noise_map))) return false;
     // the vector path stores 16-byte vectors into the neighbours' buffers too (halo push)
     if ((p.push_up && !aligned16(p.push_up)) || (p.push_dn && !aligned16(p.push_dn))) return false;
     return true;

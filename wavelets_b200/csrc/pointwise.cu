@@ -8,16 +8,6 @@
 
 namespace wb {
 
-// threshold = (sigma * noise) * sigma_e evaluated like NumPy >= 2: with a scalar noise everything is float64; with a
-// per-pixel noise map of the plane dtype, `sigma * noise` stays in that dtype and only the product with the
-// float64 sigma_e is promoted (watroo/wavelets.py:137,141).
-template <typename T>
-__device__ __forceinline__ double threshold_at(const T *noise_map, long long i, double sigma, double scalar,
-                                               double sigma_e) {
-    if (noise_map) return (double)((T)sigma * noise_map[i]) * sigma_e;
-    return (sigma * scalar) * sigma_e;
-}
-
 // out: soft -> float64 erf(|w / thr|); hard -> uint8 (|w| > thr).  thr = (sigma * noise) * sigma_e, in float64
 // exactly as NumPy >= 2 evaluates it; noise is a host scalar, a device scalar or a per-pixel map.
 template <typename T>

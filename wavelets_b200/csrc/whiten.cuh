@@ -21,14 +21,35 @@ __device__ __forceinline__ float rsqrt_fast(float x) {
 // two roundings is <= 3 ulp, four orders of magnitude inside the 1e-12 budget.  Soft threshold: erf(|w / thr|) with the reciprocal of thr hoisted (fp32);
 // hard threshold: NumPy >= 2 compares |w| (fp32) with the float64 threshold; |w| > thr in float64 is equivalent to
 // |w| > RD(thr) in fp32 (RD = round towards -inf), so the mask stays bit-exact without float64 instructions.
+//
+// Map mode (sig_mode == SIG_MAP, a per-pixel noise map): the composition of the mode-0 whitening with the significance
+// of wb_significance and the float64 product of Coefficients.significance, per pixel, so that the result is bit-identical
+// to running those three steps one after the other:
+//     tmp = T(w * g)                                       (mode 0, the same instructions as apply / apply_lane)
+//     thr = double(T(sigma) * map) * sigma_e               (map_threshold, common.cuh)
+//     s   = soft ? erf(|double(w) / thr|) : (|double(w)| > thr ? 1.0 : 0.0)
+//     out = T(double(tmp) * s)
+// The last step is a multiply, not a select: masked negative coefficients stay -0.0, and a zero or negative map entry
+// gives the inf / NaN / sign of the unfused composition.
 template <typename T> struct WhitenEpilogue {
     int mode;
     T thr_cmp;  // hard threshold in the plane dtype, rounded down
     T thr;      // fp64: the threshold itself (soft); fp32: unused
     T inv_thr;  // soft: 1 / thr
     T weight;
+    double sigma, sigma_e;  // map mode
+    int map_soft;           // map mode: erf (1) or the hard mask (0); uniform over the launch
+    // MAP: the kernel was compiled for the map mode (sig_mode == SIG_MAP; the thresholds are per pixel, see map_sig)
+    template <bool MAP = false>
     __device__ __forceinline__ void init(const ScaleParams &p, int frame) {
         mode = p.sig_mode;
+        if constexpr (MAP) {
+            sigma = p.sigma;
+            sigma_e = p.sigma_e;
+            map_soft = p.map_soft;
+            weight = (T)p.weight;
+            return;
+        }
         double t = 0.0;
         if (mode) {
             const double noise = p.noise_dev ? p.noise_dev[frame] : p.noise_host;
@@ -94,6 +115,46 @@ template <typename T> struct WhitenEpilogue {
             return Lane<double>::u(x * g);
         }
     }
+    // Map mode, one pixel: raw w, its mode-0 whitening tmp (apply / apply_lane) and its noise-map entry.
+    __device__ __forceinline__ T map_sig(T w, T tmp, T noise) const {
+        const double thr = map_threshold<T>(noise, sigma, sigma_e);
+        const double v = (double)w;
+        const double s = map_soft ? erf(fabs(v / thr)) : (fabs(v) > thr ? 1.0 : 0.0);
+        return (T)((double)tmp * s);
+    }
+    // Map mode, one 64-bit lane of a lean kernel: raw w, its whitening tmp (apply_lane) and the map, as stored.
+    __device__ __forceinline__ u64 map_lane(u64 w, u64 tmp, u64 noise) const {
+        if constexpr (sizeof(T) == 4) {
+            float w0, w1, t0, t1, n0, n1;
+            up2(w, w0, w1);
+            up2(tmp, t0, t1);
+            up2(noise, n0, n1);
+            return pk2(map_sig(w0, t0, n0), map_sig(w1, t1, n1));
+        } else {
+            return Lane<double>::u(map_sig(Lane<double>::d(w), Lane<double>::d(tmp), Lane<double>::d(noise)));
+        }
+    }
 };
+
+// Read-only streaming load of one 16-byte noise-map vector (read once per thresholded scale; not kept in L1).
+__device__ __forceinline__ P4 ldg_p4_stream(const void *p) {
+    P4 r;
+    asm("ld.global.nc.L1::no_allocate.v2.b64 {%0, %1}, [%2];" : "=l"(r.lo), "=l"(r.hi) : "l"(p));
+    return r;
+}
+__device__ __forceinline__ Pack<float, 4> ld_vec_stream(const float *p) {
+    const P4 r = ldg_p4_stream(p);
+    Pack<float, 4> v;
+    up2(r.lo, v.v[0], v.v[1]);
+    up2(r.hi, v.v[2], v.v[3]);
+    return v;
+}
+__device__ __forceinline__ Pack<double, 2> ld_vec_stream(const double *p) {
+    const P4 r = ldg_p4_stream(p);
+    Pack<double, 2> v;
+    v.v[0] = Lane<double>::d(r.lo);
+    v.v[1] = Lane<double>::d(r.hi);
+    return v;
+}
 
 }  // namespace wb

@@ -16,7 +16,7 @@ import torch
 from . import _lib
 from .scaling import B3spline
 from .wavelets import (AtrousTransform, Coefficients, _Noise, _frame_layout, abs_median_noise, atrous_scale,
-                       bilateral_list, plane_moments, synthesis, to_device_image)
+                       bilateral_list, broadcast_noise_map, plane_moments, synthesis, to_device_image)
 
 __all__ = ["denoise", "wow", "wow_batch", "wow_stream", "generalized_anscombe", "enhance", "richardson_lucy"]
 
@@ -132,6 +132,20 @@ def _whiten_scale(lib, w_raw, out, s, scaling_function, sig_mode, sigma, sigma_e
                                            _lib.stream_ptr(w_raw.device)))
 
 
+def _whiten_scale_map(lib, w_raw, out, noise_map, s, scaling_function, soft, sigma, sigma_e, weight):
+    """K3 with a per-pixel noise map (wb_wow_whiten_scale_map): ``noise_map`` is (H, W), shared by every frame, or one
+    (H, W) map per frame of ``w_raw``."""
+    b, h, w, pitch, bstride = _frame_layout(w_raw)
+    _, _, _, o_pitch, o_bstride = _frame_layout(out)
+    _, _, _, m_pitch, m_bstride = _frame_layout(noise_map)
+    with torch.cuda.device(w_raw.device):
+        _lib.check(lib.wb_wow_whiten_scale_map(w_raw.data_ptr(), out.data_ptr(), noise_map.data_ptr(), b, h, w, pitch,
+                                               bstride, o_pitch, o_bstride, m_pitch, m_bstride, s,
+                                               scaling_function.taps_code, _lib.dtype_code(w_raw.dtype),
+                                               1 if soft else 0, float(sigma), float(sigma_e), float(weight),
+                                               _lib.stream_ptr(w_raw.device)))
+
+
 def _wow_scale_fused(lib, src, dst_c, out_w, s, scaling_function, sig_mode, sigma, sigma_e, nz, weight):
     """One fused WOW scale (wb_wow_scale).  Returns False without launching anything when the problem is outside the
     fused kernel (the caller then takes the two-pass route)."""
@@ -162,6 +176,24 @@ def _scalar_noise(noise, device):
     if isinstance(noise, np.ndarray) and noise.ndim > 0:
         return "map"
     return _Noise(host=float(noise))
+
+
+_STACK_NOISE_FORMS = "None, a scalar, per-frame scalars (B,), one map (H, W) for every frame or one map per frame (B, H, W)"
+
+
+def _stack_noise(noise, b, h, w, dtype, device):
+    """The ``noise`` of wow_batch / wow_stream for ``b`` frames of (h, w): None, a _Noise with a host or device scalar,
+    with float64 per-frame scalars (``dev``, shape (b,)), or with a map (``map``, (h, w) or (b, h, w), frame dtype)."""
+    nz = _scalar_noise(noise, device)
+    if not isinstance(nz, str):
+        return nz
+    shape = tuple(noise.shape)
+    if shape == (b,):
+        t = noise if isinstance(noise, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(noise))
+        return _Noise(dev=t.to(device=device, dtype=torch.float64).contiguous())
+    if shape in ((h, w), (b, h, w)):
+        return _Noise(map_=broadcast_noise_map(noise, shape, dtype, device))
+    raise ValueError(f"noise of shape {shape} for {b} frames of {h} x {w}: expected {_STACK_NOISE_FORMS}")
 
 
 def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilateral, bilateral_scaling, whitening,
@@ -212,6 +244,7 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
         if ws is None or ws.numel() < ws_bytes or ws.device != dev:
             ws = buffers["cascade_ws"] = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         any_sig = any(d != 0 for d in dns[:L])
+        nz_map = None if noise is None else noise.map
         estimate = noise is None and any_sig
         nz = noise
         if estimate:
@@ -219,19 +252,24 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
         use = nz if nz is not None else _Noise()
         arr = ctypes.c_double * (L + 1)
         _, _, _, pitch, bstride = _frame_layout(stack)
+        args = (stack.data_ptr(), pitch, bstride, planes.data_ptr(), scratch3.data_ptr(), recon.data_ptr(), b, h, w, L,
+                sf.taps_code, code, arr(*[float(x) for x in wts[:L + 1]]),
+                arr(*([float(x) for x in dns[:L]] + [0.0])), arr(*([float(x) for x in sigma_e[:L]] + [0.0])),
+                None if bilateral is None else arr(*([float(x) for x in factors[:L]] + [0.0])),
+                1 if soft_threshold else 0)
         with torch.cuda.device(dev):
-            _lib.check(lib.wb_wow_cascade(stack.data_ptr(), pitch, bstride, planes.data_ptr(), scratch3.data_ptr(),
-                                          recon.data_ptr(), b, h, w, L, sf.taps_code, code,
-                                          arr(*[float(x) for x in wts[:L + 1]]),
-                                          arr(*([float(x) for x in dns[:L]] + [0.0])),
-                                          arr(*([float(x) for x in sigma_e[:L]] + [0.0])),
-                                          None if bilateral is None else arr(*([float(x) for x in factors[:L]] + [0.0])),
-                                          1 if soft_threshold else 0, float(use.host), use.dev_ptr, 1 if estimate else 0,
-                                          ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev)))
+            if nz_map is not None:
+                _, _, _, m_pitch, m_bstride = _frame_layout(nz_map)
+                _lib.check(lib.wb_wow_cascade_map(*args, nz_map.data_ptr(), m_pitch, m_bstride, ws.data_ptr(),
+                                                  ws.numel(), _lib.stream_ptr(dev)))
+            else:
+                _lib.check(lib.wb_wow_cascade(*args, float(use.host), use.dev_ptr, 1 if estimate else 0, ws.data_ptr(),
+                                              ws.numel(), _lib.stream_ptr(dev)))
         return recon, planes, nz
     scratch = buffer("scratch", (2, b, h, w)) if L > 1 else None
     raw_planes = None  # scratch for the raw w_s of the two-pass route, allocated on first use
     nz = noise  # _Noise or None
+    nz_map = None if noise is None else noise.map  # per-pixel noise: two passes at every scale
     src = stack
     # Bilateral cascade with whitening: K2 is bound by the MUFU/FMA pipes and leaves HBM idle, the exact median and the
     # whitening pass K3 are bound by HBM.  They go to a high-priority side stream: K3 of scale s then runs under K2 of
@@ -254,7 +292,7 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
                 nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
             # One pass (K1+K3 fused, raw w_s stays on chip) unless the scale is bilateral, the MAD noise has to be
             # estimated from the raw w_0 first (grid-wide dependency), or the shape is outside the fused kernel.
-            fused = FUSED_WOW and factors[s] is None and not (need_sig and nz is None) and \
+            fused = FUSED_WOW and factors[s] is None and not (need_sig and nz is None) and nz_map is None and \
                 _wow_scale_fused(lib, src, dst_c, planes[:, s], s, sf, mode, d, sigma_e[s] if need_sig else 1.0,
                                  nz if need_sig else _Noise(), wt)
             if not fused:
@@ -269,8 +307,11 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
                 with torch.cuda.stream(side) if overlap else _NullContext():
                     if need_sig and nz is None:
                         nz = _Noise(dev=abs_median_noise(raw_plane, sigma_e[0]))  # s == 0: from the raw w_0
-                    _whiten_scale(lib, raw_plane, planes[:, s], s, sf, mode, d, sigma_e[s] if need_sig else 1.0,
-                                  nz if need_sig else _Noise(), wt)
+                    if need_sig and nz_map is not None:
+                        _whiten_scale_map(lib, raw_plane, planes[:, s], nz_map, s, sf, soft_threshold, d, sigma_e[s], wt)
+                    else:
+                        _whiten_scale(lib, raw_plane, planes[:, s], s, sf, mode, d, sigma_e[s] if need_sig else 1.0,
+                                      nz if need_sig else _Noise(), wt)
                     if overlap:
                         ev_k3[s % 3] = torch.cuda.Event()
                         ev_k3[s % 3].record(side)
@@ -280,11 +321,16 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
                 nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
             if mode or wt != 1:
                 use = nz if need_sig else _Noise()
-                with torch.cuda.device(dev):
-                    _lib.check(lib.wb_denoise_plane(planes[:, s].data_ptr(), h * w, b, (L + 1) * h * w,
-                                                    _lib.dtype_code(dt), mode, float(d),
-                                                    float(sigma_e[s]) if need_sig else 1.0, use.host, use.dev_ptr, 0,
-                                                    float(wt), _lib.stream_ptr(dev)))
+                # wb_denoise_plane reads one map plane for every frame: one launch per frame for per-frame maps
+                per_frame = need_sig and nz_map is not None and nz_map.ndim == 3
+                for f0, nf in ([(f, 1) for f in range(b)] if per_frame else [(0, b)]):
+                    m_ptr = 0 if not need_sig or nz_map is None else nz_map[f0].data_ptr() if per_frame else \
+                        nz_map.data_ptr()
+                    with torch.cuda.device(dev):
+                        _lib.check(lib.wb_denoise_plane(planes[f0, s].data_ptr(), h * w, nf, (L + 1) * h * w,
+                                                        _lib.dtype_code(dt), mode, float(d),
+                                                        float(sigma_e[s]) if need_sig else 1.0, use.host, use.dev_ptr,
+                                                        m_ptr, float(wt), _lib.stream_ptr(dev)))
         src = dst_c
     if overlap:
         main.wait_stream(side)  # every whitened plane is complete before the tail (and before any buffer is freed)
@@ -339,18 +385,15 @@ def wow(data, scaling_function=B3spline, n_scales=None, weights=[], whitening=Tr
                                  preserve_variance, gamma, gamma_min, gamma_max, h, plan=(n_scales, wts, dns))
         return _result(recon, was_numpy), co
     nz = _scalar_noise(noise, img.device)
-    if nz == "map":
-        # per-pixel noise maps take the unfused route: transform, then whiten plane by plane
-        transform = AtrousTransform(scaling_function, bilateral=sigma_bilateral, bilateral_scaling=bilateral_scaling)
-        co = transform(img, n_scales)
-        co.noise = noise
-        recon, co = _wow_coefficients(co, weights, whitening, denoise_coefficients, bilateral, soft_threshold,
-                                      plan=(n_scales, sigma_bilateral, wts, dns))
-        return _result(recon, was_numpy), co
+    if isinstance(nz, str):
+        # a per-pixel noise map, broadcast to the image: two passes at every scale, the map applied inside K3
+        nz = _Noise(map_=broadcast_noise_map(noise, img.shape, img.dtype, img.device))
     recon, planes, nz = _wow_stack(img.unsqueeze(0), scaling_function, n_scales, wts, dns, sigma_bilateral,
                                    bilateral_scaling, whitening, soft_threshold, nz)
     co = Coefficients(planes[0], scaling_function(2), sigma_bilateral)
-    if nz is not None:
+    if nz is not None and nz.map is not None:
+        co.noise = noise
+    elif nz is not None:
         co.noise = nz.dev if nz.dev is not None else nz.host
     else:
         co.noise = None
@@ -409,17 +452,25 @@ def _wow_nd(co, wts, dns, whitening, soft_threshold, preserve_variance, gamma, g
 def wow_batch(frames, scaling_function=B3spline, n_scales=None, weights=[], whitening=True, denoise_coefficients=[],
               noise=None, bilateral=None, bilateral_scaling=False, soft_threshold=True):
     """NEW entry point (no reference equivalent): WOW of a stack ``(B, H, W)`` of independent frames, every kernel
-    launched once for the whole stack.  Returns ``(recon (B,H,W), planes (B,L+1,H,W), noise (B,) or None)`` as device
-    tensors; per-frame results are identical to ``wow(frame, ...)``."""
+    launched once for the whole stack.  Returns ``(recon (B,H,W), planes (B,L+1,H,W), noise)`` as device tensors;
+    per-frame results are identical to ``wow(frame, noise=<that frame's noise>, ...)``.
+
+    ``noise`` (NumPy or torch): None (MAD estimate per frame), a scalar, per-frame scalars ``(B,)``, one per-pixel map
+    ``(H, W)`` for every frame or one map per frame ``(B, H, W)``; anything else raises ValueError.  The returned noise
+    is the one used: the (B,) float64 estimates or scalars, the scalar, or the map in the frame dtype."""
     stack, _ = to_device_image(frames, ndim_ok=(3,))
     n_scales, sigma_bilateral, wts, dns = _wow_plan(stack.shape[1:], scaling_function, n_scales, weights,
                                                     denoise_coefficients, bilateral)
-    nz = _scalar_noise(noise, stack.device)
-    if nz == "map":
-        raise NotImplementedError("wow_batch() takes a scalar noise or None")
+    b, h, w = stack.shape
+    nz = _stack_noise(noise, b, h, w, stack.dtype, stack.device)
     recon, planes, nz = _wow_stack(stack, scaling_function, n_scales, wts, dns, sigma_bilateral, bilateral_scaling,
                                    whitening, soft_threshold, nz)
-    noise_out = None if nz is None else (nz.dev if nz.dev is not None else nz.host)
+    if nz is None:
+        noise_out = None
+    elif nz.map is not None:
+        noise_out = nz.map
+    else:
+        noise_out = nz.dev if nz.dev is not None else nz.host
     return recon, planes, noise_out
 
 
@@ -429,8 +480,10 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
     device->host copy of the reconstruction of frame n-1 on three CUDA streams (``depth`` device buffers in flight).
 
     ``frames`` / ``out``: torch CPU tensors (pinned memory is used as is, pageable memory is staged through a pinned copy)
-    or NumPy arrays; ``kwargs`` are those of ``wow`` (scalar ``noise`` only).  Returns ``out`` (allocated pinned when None;
-    a NumPy view of it for NumPy input).  Per-frame results are identical to ``wow(frame, ...)[0]``."""
+    or NumPy arrays; ``kwargs`` are those of ``wow``.  ``noise`` takes the forms of ``wow_batch`` with N frames: a
+    scalar, per-frame scalars ``(N,)`` and one map ``(H, W)`` are uploaded once; host maps ``(N, H, W)`` are streamed
+    next to their frames (one device map buffer per frame in flight).  Returns ``out`` (allocated pinned when None; a
+    NumPy view of it for NumPy input).  Per-frame results are identical to ``wow(frame, noise=<its noise>, ...)[0]``."""
     was_numpy = not isinstance(frames, torch.Tensor)
     host = torch.from_numpy(np.ascontiguousarray(frames)) if was_numpy else frames
     if host.ndim != 3:
@@ -459,23 +512,37 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
     # The options of the fused pipeline are planned ONCE and every frame in flight owns one set of device buffers
     # (planes, ping-pong scratch, reconstruction): after the first `depth` frames nothing large is allocated -- with
     # wow() called per frame the caching allocator split and re-grew its blocks while the host ran ahead of the device
-    # (a cudaMalloc of 0.7 GB per frame: 25 ms instead of 1.3).  h > 0, preserve_variance and per-pixel noise maps take
-    # wow() itself, frame by frame.
+    # (a cudaMalloc of 0.7 GB per frame: 25 ms instead of 1.3).  h > 0 and preserve_variance take wow() itself, frame by
+    # frame.
     opts = dict(kwargs)
     unknown = set(opts) - {"n_scales", "weights", "whitening", "denoise_coefficients", "noise", "bilateral",
                            "bilateral_scaling", "soft_threshold", "preserve_variance", "gamma", "gamma_min", "gamma_max", "h"}
     if unknown:
         raise TypeError(f"wow_stream() got unexpected keyword arguments {sorted(unknown)}")
     plan = None
+    noise = opts.get("noise")
+    # per-frame noise: a device vector of scalars (sliced per frame), or the (N, H, W) maps streamed with the frames
+    nz_vec = map_host = None
+    nz0 = None
+    if noise is not None and tuple(getattr(noise, "shape", ())) == (n, h, w) and not getattr(noise, "is_cuda", False):
+        map_host = torch.from_numpy(np.ascontiguousarray(noise)) if not isinstance(noise, torch.Tensor) else noise
+        map_host = map_host.to(host.dtype)
+        if not map_host.is_pinned():
+            map_host = map_host.contiguous().pin_memory()
+    else:
+        nz0 = _stack_noise(noise, n, h, w, host.dtype, dev)
+        if nz0 is not None and ((nz0.dev is not None and nz0.dev.numel() > 1) or
+                                (nz0.map is not None and nz0.map.ndim == 3)):
+            nz_vec, nz0 = nz0, None
+        s_cmp.wait_stream(caller)  # the noise was uploaded on the caller's stream
     if opts.get("h", 0) == 0 and not opts.get("preserve_variance", False):
-        nz0 = _scalar_noise(opts.get("noise"), dev)
-        if not (isinstance(nz0, str) and nz0 == "map"):
-            n_scales, sigma_bilateral, wts, dns = _wow_plan((h, w), scaling_function, opts.get("n_scales"),
-                                                            opts.get("weights", []), opts.get("denoise_coefficients", []),
-                                                            opts.get("bilateral"), h=0)
-            plan = (n_scales, wts, dns, sigma_bilateral, opts.get("bilateral_scaling", False),
-                    opts.get("whitening", True), opts.get("soft_threshold", True), nz0)
+        n_scales, sigma_bilateral, wts, dns = _wow_plan((h, w), scaling_function, opts.get("n_scales"),
+                                                        opts.get("weights", []), opts.get("denoise_coefficients", []),
+                                                        opts.get("bilateral"), h=0)
+        plan = (n_scales, wts, dns, sigma_bilateral, opts.get("bilateral_scaling", False),
+                opts.get("whitening", True), opts.get("soft_threshold", True))
     d_in = [torch.empty((h, w), dtype=host.dtype, device=dev) for _ in range(depth)]
+    d_map = [torch.empty((h, w), dtype=host.dtype, device=dev) for _ in range(depth)] if map_host is not None else None
     d_out = [None] * depth
     bufs = [dict() for _ in range(depth)]
     ev_in = [torch.cuda.Event() for _ in range(depth)]
@@ -487,18 +554,28 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
             if i >= depth:
                 s_in.wait_event(ev_cmp[b])       # the WOW that read d_in[b] is done
             d_in[b].copy_(host[i], non_blocking=True)
+            if d_map is not None:
+                d_map[b].copy_(map_host[i], non_blocking=True)
             ev_in[b].record(s_in)
         with torch.cuda.stream(s_cmp):
             s_cmp.wait_event(ev_in[b])
             if i >= depth:
                 s_cmp.wait_event(ev_out[b])      # the download of d_out[b] is done (its memory is reused)
+            if d_map is not None:
+                nz_i = _Noise(map_=d_map[b])
+            elif nz_vec is not None:
+                nz_i = _Noise(dev=nz_vec.dev[i:i + 1]) if nz_vec.dev is not None else _Noise(map_=nz_vec.map[i])
+            else:
+                nz_i = nz0
             if plan is not None:
-                L, wts, dns, sigma_bilateral, bil_scaling, whitening, soft, nz0 = plan
+                L, wts, dns, sigma_bilateral, bil_scaling, whitening, soft = plan
                 recon, _, _ = _wow_stack(d_in[b].unsqueeze(0), scaling_function, L, wts, dns, sigma_bilateral,
-                                         bil_scaling, whitening, soft, nz0, buffers=bufs[b])
+                                         bil_scaling, whitening, soft, nz_i, buffers=bufs[b])
                 d_out[b] = recon[0]
             else:
-                d_out[b], _ = wow(d_in[b], scaling_function=scaling_function, **kwargs)
+                frame_noise = None if nz_i is None else nz_i.map if nz_i.map is not None else \
+                    nz_i.dev if nz_i.dev is not None else nz_i.host
+                d_out[b], _ = wow(d_in[b], scaling_function=scaling_function, **dict(kwargs, noise=frame_noise))
             ev_cmp[b].record(s_cmp)
         with torch.cuda.stream(s_out):
             s_out.wait_event(ev_cmp[b])
@@ -536,13 +613,11 @@ def _wow_coefficients(co, weights, whitening, denoise_coefficients, bilateral, s
             # local power from the raw plane, significance from the raw plane, then both factors (utils.py:194-203)
             nz = co._noise_arg(d) if d != 0 else _Noise()
             if nz.map is not None:
-                sig = co.significance(d, s, soft_threshold=soft_threshold)
-                _whiten_scale(lib, plane, tmp, s, sf, 0, 0.0, 1.0, _Noise(), wt)
-                plane.copy_((tmp.to(torch.float64) * sig.to(torch.float64)).to(plane.dtype))
+                _whiten_scale_map(lib, plane, tmp, nz.map, s, sf, soft_threshold, d, co.sigma_e[s], wt)
             else:
                 mode = (1 if soft_threshold else 2) if d != 0 else 0
                 _whiten_scale(lib, plane, tmp, s, sf, mode, d, co.sigma_e[s] if d != 0 else 1.0, nz, wt)
-                plane.copy_(tmp)
+            plane.copy_(tmp)
         else:
             co._denoise_plane(lib, s, d, wt, soft_threshold)
     last = data[L]
@@ -583,17 +658,13 @@ def _wow_general(co, weights, whitening, denoise_coefficients, bilateral, soft_t
             mom = plane_moments(plane)[0]                       # [mean, var, std] of the raw plane, float64
             power_norm = torch.sqrt(mom[1] + mom[0] * mom[0]).to(dt)  # sqrt(mean(c**2)), utils.py:182
         nz = co._noise_arg(d) if d != 0 else _Noise()           # lazily, from the current plane 0 (wavelets.py:131)
-        if nz.map is not None:
-            sig = co.significance(d, s, soft_threshold=soft_threshold).to(torch.float64)
-            if white:
-                _whiten_scale(lib, plane, tmp, s, sf, 0, 0.0, 1.0, _Noise(), wt)
-                tmp.copy_((tmp.to(torch.float64) * sig).to(dt))
-            plane.copy_((plane.to(torch.float64) * sig).to(dt))
-        else:
-            mode = (1 if soft_threshold else 2) if d != 0 else 0
-            if white:
+        if white:
+            if nz.map is not None:
+                _whiten_scale_map(lib, plane, tmp, nz.map, s, sf, soft_threshold, d, co.sigma_e[s], wt)
+            else:
+                mode = (1 if soft_threshold else 2) if d != 0 else 0
                 _whiten_scale(lib, plane, tmp, s, sf, mode, d, co.sigma_e[s] if d != 0 else 1.0, nz, wt)
-            co._denoise_plane(lib, s, d, 1, soft_threshold)     # plane <- raw * significance
+        co._denoise_plane(lib, s, d, 1, soft_threshold)         # plane <- raw * significance
         if gamma_scaled is not None:
             gamma_scaled += plane                               # utils.py:200-201: after significance, before weighting
         if white:

@@ -234,6 +234,19 @@ def synthesis(planes, out=None):
     return out
 
 
+def broadcast_noise_map(noise, shape, dtype, device):
+    """A per-pixel noise map (ndarray or tensor) as a contiguous device tensor of ``shape`` and the plane dtype,
+    broadcast NumPy-style as the reference's array arithmetic does (``data / (sigma * noise * sigma_e)``).  Raises
+    ValueError when it does not broadcast to ``shape``."""
+    m = noise if isinstance(noise, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(noise))
+    try:
+        m = torch.broadcast_to(m, tuple(shape))
+    except RuntimeError as exc:
+        raise ValueError(f"a noise map of shape {tuple(noise.shape)} does not broadcast to the plane shape "
+                         f"{tuple(shape)}") from exc
+    return m.to(device=device, dtype=dtype).contiguous()
+
+
 class _Noise:
     """How a threshold kernel receives the noise: host scalar, device scalar (float64) or per-pixel map."""
 
@@ -311,12 +324,11 @@ class Coefficients:
                 if n.is_cuda and n.dtype == torch.float64:
                     return _Noise(dev=n)
                 return _Noise(host=float(n.item()))
-            m = n.to(device=self.data.device, dtype=self.data.dtype).contiguous()
-            return _Noise(map_=m)
+            return _Noise(map_=broadcast_noise_map(n, self.data.shape[1:], self.data.dtype, self.data.device))
         if isinstance(n, np.ndarray):
             if n.ndim == 0:
                 return _Noise(host=float(n))
-            m = torch.from_numpy(np.ascontiguousarray(n)).to(device=self.data.device, dtype=self.data.dtype)
+            m = broadcast_noise_map(n, self.data.shape[1:], self.data.dtype, self.data.device)
             self._noise = m  # keep the device copy for the next scale
             return _Noise(map_=m)
         if isinstance(n, numbers.Number):
