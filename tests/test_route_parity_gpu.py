@@ -411,6 +411,76 @@ def test_row_kernel_one_vector_per_thread_vs_oracle(sf, dt):
     report(f"row kernel ng=1 {np.dtype(dt).name} {sf:8s} 45x{w}: {par.summary()}")
 
 
+LEAN_VS_ROW_WIDTHS = {np.float32: (1500, 2048, 3000, 4096, 6000), np.float64: (2048, 3000)}
+# lean families the default calls of those widths launch: 8 / 16 KiB whole-row slots (fp32 only), 24 KiB strip slots
+# (fp32 rows wider than 4096 columns, float64), paired columns, the K3 form
+LEAN_FAMILIES = {np.float32: {"atrous_rows_lean_kernel 8 KiB slots", "atrous_rows_lean_kernel 16 KiB slots",
+                              "atrous_rows_lean_kernel strip", "atrous_rows_lean_kernel paired",
+                              "atrous_rows_lean_kernel OP_WHITEN"},
+                 np.float64: {"atrous_rows_lean_kernel strip", "atrous_rows_lean_kernel paired",
+                              "atrous_rows_lean_kernel OP_WHITEN"}}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dt", [np.float32, np.float64])
+def test_lean_kernel_equals_row_kernel(dt):
+    """The lean K1 / K3 kernels against the row kernel, bit for bit: every scale of K1 (both outputs) and of K3 (all
+    three significance modes), once with the default dispatch and once under a wb_tune_k1 override of the very geometry
+    plan_fast picks by itself -- under an override dispatch skips the lean kernels.  torch.profiler confirms which
+    kernels each pass ran."""
+    from torch.profiler import ProfilerActivity, profile
+    lib = _gpu_lib()
+    v = 16 // np.dtype(dt).itemsize
+    h = 45
+
+    def k1(img, s, sf):
+        c, wd = torch.empty_like(img), torch.empty_like(img)
+        assert lib.wb_atrous_scale(img.data_ptr(), c.data_ptr(), wd.data_ptr(), 1, h, img.shape[2], img.shape[2], 0,
+                                   img.shape[2], 0, img.shape[2], 0, s, TAPS[sf], DCODE[dt], _stream()) == 0
+        return [c, wd]
+
+    def k3(w_raw, s, sf):
+        outs = []
+        for mode in (0, 1, 2):
+            o = torch.empty_like(w_raw)
+            assert lib.wb_wow_whiten_scale(w_raw.data_ptr(), o.data_ptr(), 1, h, w_raw.shape[2], w_raw.shape[2], 0,
+                                           w_raw.shape[2], 0, s, TAPS[sf], DCODE[dt], mode, SIGMA, SIGMA_E, NOISE, None,
+                                           WEIGHT, _stream()) == 0
+            outs.append(o)
+        return outs
+
+    cases = []  # (w, sf, s, image, default outputs: K1 c, K1 w, K3 of that w in modes 0, 1, 2)
+    with profile(activities=[ProfilerActivity.CUDA], acc_events=True) as prof_default:
+        for w in LEAN_VS_ROW_WIDTHS[dt]:
+            img = torch.from_numpy(_frames(1, h, w, dt, 41 + w)).cuda()
+            for sf in SCALING:
+                for s in scales_of(sf, w):
+                    want = k1(img, s, sf)
+                    cases.append((w, sf, s, img, want + k3(want[1], s, sf)))
+        torch.cuda.synchronize()
+    try:
+        with profile(activities=[ProfilerActivity.CUDA], acc_events=True) as prof_override:
+            for w, sf, s, img, want in cases:
+                nt = min(((w // v + 1) // 2 + 31) // 32 * 32, 512)  # what plan_fast picks for two vectors per thread
+                assert lib.wb_tune_k1(s, nt, 2, 8, 0) == 0
+                got = k1(img, s, sf) + k3(want[1], s, sf)
+                for name, g, r in zip(("K1 c", "K1 w", "K3 mode 0", "K3 mode 1", "K3 mode 2"), got, want):
+                    assert torch.equal(g, r), (np.dtype(dt).name, w, sf, s, name)
+            torch.cuda.synchronize()
+    finally:
+        for s in range(32):
+            lib.wb_tune_k1(s, 0, 0, 0, 0)
+
+    def families(prof):
+        return set().union(*(kernel_families(ev.name) for ev in prof.events()))
+    seen_default, seen_override = families(prof_default), families(prof_override)
+    assert LEAN_FAMILIES[dt] <= seen_default, LEAN_FAMILIES[dt] - seen_default
+    assert "atrous_rows_kernel ng=2" in seen_override
+    assert not any(f.startswith("atrous_rows_lean_kernel") for f in seen_override), seen_override
+    report(f"lean vs row kernel {np.dtype(dt).name} W={LEAN_VS_ROW_WIDTHS[dt]}: {len(cases)} scales bit-identical; "
+           f"default ran {sorted(f for f in seen_default if 'lean' in f)}")
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # 2. batches of different frames, per-frame device noise, both NULL output forms of K1
 # ---------------------------------------------------------------------------------------------------------------------
@@ -462,28 +532,30 @@ def kernel_families(name):
         return {kern}
     if kern == "atrous_rows_kernel":  # <T, TAPS, DMODE, NG, OP>
         return {f"atrous_rows_kernel ng={args[3]}"}
-    if kern == "atrous_rows_lean_kernel":  # <T, TAPS, DMODE, HINTS, OP, MODE, PAIR, UNROLL, RBK>
-        rbk = args[8] if len(args) > 8 else "16"
-        fams = {"atrous_rows_lean_kernel " + {"16": "16 KiB slots", "8": "8 KiB slots", "24": "strip"}[rbk]}
-        if len(args) > 6 and args[6] != "0":
+    if kern == "atrous_rows_lean_kernel":  # <T, TAPS, DMODE, HINTS, OP, MODE, PAIR, RBK>
+        fams = {"atrous_rows_lean_kernel " + {"16": "16 KiB slots", "8": "8 KiB slots", "24": "strip"}[args[7]]}
+        if args[6] != "0":
             fams.add("atrous_rows_lean_kernel paired")
-        if len(args) > 4 and args[4] == "1":
+        if args[4] == "1":
             fams.add("atrous_rows_lean_kernel OP_WHITEN")
         return fams
-    # wow_rows_lean_kernel<TAPS, DMODE, HINTS, MODE, PAIR, DYN, NTK>
-    ntk = args[6] if len(args) > 6 else "512"
-    pair = len(args) > 4 and args[4] != "0"
-    return {f"wow_rows_lean_kernel {ntk} threads {'paired' if pair else 'unpaired'} mode {args[3]}"}
+    # wow_rows_lean_kernel<TAPS, DMODE, HINTS, MODE, PAIR, NTK>
+    pair = args[4] != "0"
+    return {f"wow_rows_lean_kernel {args[5]} threads {'paired' if pair else 'unpaired'} mode {args[3]}"}
 
 
 def test_kernel_family_parser():
     assert kernel_families("void wb::atrous_rows_lean_kernel<float, (int)3, (int)0, (bool)1, (int)0, (int)0, (int)1, "
-                           "(int)4, (int)8>(wb::ScaleParams)") == {"atrous_rows_lean_kernel 8 KiB slots",
-                                                                    "atrous_rows_lean_kernel paired"}
-    assert kernel_families("void wb::wow_rows_lean_kernel<5, 0, true, 2, 1, true, 256>(wb::ScaleParams)") == {
+                           "(int)8>(wb::ScaleParams)") == {"atrous_rows_lean_kernel 8 KiB slots",
+                                                           "atrous_rows_lean_kernel paired"}
+    assert kernel_families("void wb::atrous_rows_lean_kernel<float, 5, 2, false, 0, 0, 0, 16>(wb::ScaleParams)") == {
+        "atrous_rows_lean_kernel 16 KiB slots"}
+    assert kernel_families("void wb::wow_rows_lean_kernel<5, 0, true, 2, 1, 256>(wb::ScaleParams)") == {
         "wow_rows_lean_kernel 256 threads paired mode 2"}
+    assert kernel_families("void wb::wow_rows_lean_kernel<(int)3, (int)1, (bool)0, (int)0, (int)0, (int)512>"
+                           "(wb::ScaleParams)") == {"wow_rows_lean_kernel 512 threads unpaired mode 0"}
     assert kernel_families("void wb::atrous_rows_kernel<double, 5, 1, 1, 1>(wb::ScaleParams)") == {"atrous_rows_kernel ng=1"}
-    assert kernel_families("void wb::atrous_rows_lean_kernel<double, 5, 0, true, 1, 2, 0, 4, 24>(wb::ScaleParams)") == {
+    assert kernel_families("void wb::atrous_rows_lean_kernel<double, 5, 0, true, 1, 2, 0, 24>(wb::ScaleParams)") == {
         "atrous_rows_lean_kernel strip", "atrous_rows_lean_kernel OP_WHITEN"}
     assert kernel_families("void wb::bilateral_lean_kernel<5, 0, 3>(wb::BilateralParams)") == {"bilateral_lean_kernel"}
     assert kernel_families("void wb::bilateral_lean_kernel<(int)3, (int)1, (int)-1>(wb::BilateralParams)") == {
@@ -531,14 +603,13 @@ def test_route_coverage():
 # ---------------------------------------------------------------------------------------------------------------------
 SWITCH_CASES = [(np.float32, 1020), (np.float32, 1500), (np.float32, 2048), (np.float32, 3000), (np.float32, 4096),
                 (np.float32, 6000), (np.float64, 1024), (np.float64, 2048), (np.float64, 3000)]
-SWITCH_VARS = ("WB_PDL", "WB_L2_HINTS", "WB_L2_HINTS_WOW", "WB_K1_UNROLL", "WB_WOW_DYN", "WB_K1_LEAN", "WB_WOW_LEAN",
-               "WB_K1_PAIR", "WB_WOW_PAIR", "WB_K1_LEAN_STRIPS", "WB_WOW_STRIPS")
-# Every switch must give planes bit-identical to the default (measured on a B200 for all of them).  The first eight
-# change scheduling, cache hints or loop shape only; the last five run another kernel (generic instead of lean, unpaired
-# instead of paired columns, the row kernel instead of lean strips) that performs the same operations in the same order.
-SWITCHES = ["WB_PDL=0", "WB_L2_HINTS=0", "WB_L2_HINTS_WOW=0", "WB_L2_HINTS_WOW=1", "WB_L2_HINTS_WOW=2", "WB_K1_UNROLL=8",
-            "WB_WOW_DYN=0", "WB_WOW_DYN=1",
-            "WB_K1_LEAN=0", "WB_WOW_LEAN=0", "WB_K1_PAIR=0", "WB_WOW_PAIR=0", "WB_K1_LEAN_STRIPS=0"]
+SWITCH_VARS = ("WB_PDL", "WB_L2_HINTS")
+# The two A/B switches of the CUDA library; each must give planes bit-identical to the default.  WB_PDL=0 changes
+# scheduling only.  WB_L2_HINTS=0 drops the cache hints and with them moves launches to other kernels that perform the
+# same operations in the same order: the generic fused kernel instead of the 256-thread lean one, the unhinted lean
+# kernels on 16 KiB slots, the row kernel instead of the lean strips and float64 rows, and the bilateral window kernel
+# instead of the lean one.
+SWITCHES = ["WB_PDL=0", "WB_L2_HINTS=0"]
 
 _CHILD = """
 import json, sys

@@ -2,8 +2,6 @@
 real reference and against the oracle evaluated in float64 (dual-oracle protocol of SURVEY.md 8(d))."""
 import warnings
 
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -510,45 +508,3 @@ def test_wow_nd_golden(dt):
         for p in range(len(ref_p)):
             tp = dual_tol(ref_p[p], p64[p], dt, fp64_tol=1e-11 if bil else 1e-12, base=2e-5)
             assert orc.emax(got[p], p64[p]) <= tp, (k, p, orc.emax(got[p], p64[p]), tp)
-
-
-@pytest.mark.parametrize("dt", ["float32", "float64"])
-def test_wow_fused_column_strips_equal_two_pass(dt):
-    """Column-strip mode of the fused kernel (the route of float64 rows wider than 2048 columns; forced here with
-    WB_WOW_STRIPS on narrower rows too so that strip edges fall at many positions): c_{s+1} bit-identical to K1, w'_s
-    bit-identical to K1 -> K3 away from the top/bottom border, every strip-edge column included."""
-    from wavelets_b200 import _lib, utils
-    from wavelets_b200.wavelets import atrous_scale
-    lib = _lib.load(require_cuda=True)
-    tdt = getattr(torch, dt)
-    gen = torch.Generator(device="cuda").manual_seed(11)
-    try:
-        for sf in ("b3spline", "triangle"):
-            scf = _sf(sf)(2)
-            c = scf.taps_code // 2
-            for (b, h, w, strips) in ((1, 150, 4096, 2), (2, 40, 1024, 2), (1, 130, 2304, 3), (1, 64, 3000, 5), (1, 90, 6144, 2),
-                                      (1, 150, 4096, 4)):
-                os.environ["WB_WOW_STRIPS"] = str(strips)
-                src = torch.randn((b, h, w), generator=gen, device="cuda", dtype=tdt) * 3 + 1
-                n_fused = 0
-                for s in range(0, 9):
-                    if c * 2 ** s > w:
-                        break
-                    for mode, nz in ((0, utils._Noise()), (1, utils._Noise(host=0.9))):
-                        c_ref, w_raw = atrous_scale(src, s, scf)
-                        w_ref = torch.empty_like(src)
-                        utils._whiten_scale(lib, w_raw, w_ref, s, scf, mode, 2.5, 0.3, nz, 1.25)
-                        c_f, w_f = torch.full_like(src, float("nan")), torch.full_like(src, float("nan"))
-                        if not utils._wow_scale_fused(lib, src, c_f, w_f, s, scf, mode, 2.5, 0.3, nz, 1.25):
-                            continue
-                        n_fused += 1
-                        assert torch.equal(c_f, c_ref), (sf, b, h, w, strips, s, mode)
-                        edge = c * 2 ** s
-                        if h > 2 * edge:
-                            assert torch.equal(w_f[:, edge:h - edge], w_ref[:, edge:h - edge]), (sf, b, h, w, strips, s, mode)
-                        assert torch.isfinite(w_f).all()
-                        rel = (w_f - w_ref).abs().max() / w_ref.abs().max()
-                        assert rel.item() < (1e-5 if dt == "float32" else 1e-13), (sf, b, h, w, strips, s, mode, rel.item())
-                assert n_fused >= 6, (sf, b, h, w, strips, n_fused)
-    finally:
-        os.environ.pop("WB_WOW_STRIPS", None)

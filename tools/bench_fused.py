@@ -1,5 +1,4 @@
-"""Per-scale launch time of the fused WOW scale kernel and of wow() itself (GPU box only; A/B runs set the WB_WOW_*
-environment switches of csrc/wow_scale.cu before the process starts).
+"""Per-scale launch time of the fused WOW scale kernel and of wow() itself (GPU box only).
 
     python tools/bench_fused.py [--side 4096] [--reps 30] [--tag name]
 """

@@ -1,5 +1,5 @@
 """Quick device-resident timings of the three headline calls (GPU box only), for A/B runs under environment switches
-(WB_L2_PERSIST, WB_L2_HINTS, WB_PDL, WB_K1_LEAN ...).
+(WB_L2_HINTS, WB_PDL).
 
     python tools/bench_quick.py [--reps 200] [--tag name]"""
 import argparse

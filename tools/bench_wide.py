@@ -1,6 +1,6 @@
 """K1 on rows wider than one ring slot (column strips): per-scale launch time and whole transforms (GPU box only).
 
-    python tools/bench_wide.py [--tag name]      # A/B: WB_K1_LEAN_STRIPS=0 selects the generic kernel
+    python tools/bench_wide.py [--tag name]
 """
 import argparse
 import json

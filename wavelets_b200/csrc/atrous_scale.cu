@@ -205,7 +205,7 @@ __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
 // ---------------------------------------------------------------------------------------------------------------
 // K1, fp32 whole-row strips: the same pipeline, LEAN (see wow_scale.cu for the measurements behind the recipe).  The
 // kernel above spends ~330 warp instructions per warp-step of which ~100 are floating point (ncu: 22.5 M warp
-// instructions per 4096^2 plane, 67 % issue-active).  Here the consumer loop is unrolled by the 8-slot ring, ring
+// instructions per 4096^2 plane, 67 % issue-active).  Here the consumer loop is unrolled by half the 8-slot ring, ring
 // slots have a fixed 16 KiB stride (every LDS is [register + immediate]), pixel pairs are carried as 64-bit
 // register pairs (FFMA2 / FMUL2 / FADD2, same roundings as the scalar instructions) and the output pointers are
 // per-thread and advance by one add per row.  Same operation order as atrous_rows_kernel: bit-identical planes.
@@ -216,18 +216,16 @@ static constexpr int kLeanSlots = 8;
 // SQUARES of the staged raw w_s rows and the epilogue whitens the raw centre value -- same pipeline, 2*T bytes per pixel.
 // PAIR = M > 0 (DMODE 0, d >= 8): a thread's two column vectors are M dilation steps apart (x, x + M d) and share
 // TAPS - M of their tap vectors (lean_row_pass_pair, see wow_rows_lean_kernel): 8 instead of 12 LDS.128 per step at M = 1.
-// UNROLL: steps per iteration of the step loop, 8 (= the ring: every slot offset an immediate) or 4 (the ring's two
-// halves alternate: one more address term per access, HALF the code -- a 60 KB kernel does not fit the 32 KB
-// instruction cache level, and every change of kernel inside a cascade starts cold).
+// The step loop is unrolled by half the ring and the ring's two halves alternate: one more address term per access than
+// a loop unrolled by the whole ring, but HALF the code -- a 60 KB kernel does not fit the 32 KB instruction cache level,
+// and every change of kernel inside a cascade starts cold.
 // T / RBK (round 2): float64 rows (one double per 64-bit lane: DFMA instead of FFMA2, see Lane<T>) and COLUMN STRIPS -- a
 // block stages columns [x0 - halo, x0 + wt + halo) of its strip in ring slots of RBK KiB (16: whole rows of <= 4096 fp32
 // columns, the geometry the kernel was written for; 24: strips of 4096 fp32 / 2048 fp64 columns with up to 1024 / 512
 // halo columns per side, i.e. rows wider than one slot at every dilation up to 512 / 256).
-template <typename T, int TAPS, int DMODE, bool HINTS, int OP = OP_TRANSFORM, int MODE = 0, int PAIR = 0, int UNROLL = 8,
-          int RBK = 16>
+template <typename T, int TAPS, int DMODE, bool HINTS, int OP, int MODE, int PAIR, int RBK>
 __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams p) {
     static_assert(PAIR == 0 || (DMODE == 0 && PAIR < TAPS), "paired columns need d % V == 0 and overlapping taps");
-    static_assert(UNROLL == 8 || UNROLL == 4, "the step loop is unrolled by the ring or by half of it");
     constexpr int V = VecOf<T>::V, NG = 2;
     constexpr int C = TAPS / 2;
     constexpr int NV = PlanSize<TAPS, DMODE>::NV;
@@ -363,9 +361,9 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
     const bool pushing = (p.push_up != nullptr) | (p.push_dn != nullptr);
     int out_row = (int)orow;  // band row of the next output
 
-    // Step j = UNROLL u + I: input row j lands (ring slot j % 8 = I + (half ? 4 : 0)) -> row pass -> column feed -> c row
+    // Step j = 4 u + I: input row j lands (ring slot j % 8 = I + (half ? 4 : 0)) -> row pass -> column feed -> c row
     // j-C; w = raw centre row - c; release the centre row's slot.  `half` / `half_c`: byte offset (0 or 4 RB) of the ring
-    // half this iteration's rows land in / of the other half (UNROLL == 4; both 0 when the loop is unrolled by the ring).
+    // half this iteration's rows land in / of the other half.
     auto step = [&](auto ic, auto mirror, const int j, const uint32_t par, const uint32_t half, const uint32_t half_c) {
         constexpr int I = decltype(ic)::value;
         constexpr bool MIRROR = decltype(mirror)::value != 0;
@@ -394,9 +392,9 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
                 cv[q].hi = col_feed_p<TAPS>(S[q][1], v.hi, H);
             }
         }
-        // raw centre row j-C: slot (I - C) mod UNROLL of this half, or of the other half when the index wraps
-        constexpr int SC = (I - C + UNROLL) & (UNROLL - 1);
-        const uint32_t hc = (UNROLL == 4 && I < C) ? half_c : half;
+        // raw centre row j-C: slot (I - C) mod 4 of this half, or of the other half when the index wraps
+        constexpr int SC = (I - C + 4) & 3;
+        const uint32_t hc = (I < C) ? half_c : half;
         if (j >= 2 * C) {
             if constexpr (OP == OP_WHITEN) {
 #pragma unroll
@@ -444,20 +442,14 @@ __global__ void __launch_bounds__(544) atrous_rows_lean_kernel(const ScaleParams
     };
     auto run = [&](auto mirror) {
 #pragma unroll 1
-        for (int jb = 0; jb < n_load; jb += UNROLL) {
+        for (int jb = 0; jb < n_load; jb += 4) {
             const uint32_t par = (uint32_t)(jb >> 3) & 1u;
-            const uint32_t half = (UNROLL == 4 && (jb & 4)) ? 4u * RB : 0u;
-            const uint32_t half_c = (UNROLL == 4) ? (half ^ (4u * RB)) : 0u;
+            const uint32_t half = (jb & 4) ? 4u * RB : 0u;
+            const uint32_t half_c = half ^ (4u * RB);
             step(IC<0>{}, mirror, jb + 0, par, half, half_c);
             step(IC<1>{}, mirror, jb + 1, par, half, half_c);
             step(IC<2>{}, mirror, jb + 2, par, half, half_c);
             step(IC<3>{}, mirror, jb + 3, par, half, half_c);
-            if constexpr (UNROLL == 8) {
-                step(IC<4>{}, mirror, jb + 4, par, half, half_c);
-                step(IC<5>{}, mirror, jb + 5, par, half, half_c);
-                step(IC<6>{}, mirror, jb + 6, par, half, half_c);
-                step(IC<7>{}, mirror, jb + 7, par, half, half_c);
-            }
         }
     };
     if (mirror_warp) run(IC<1>{});
@@ -536,70 +528,26 @@ static int launch_rows(const ScaleParams &p, int batch, int nt, cudaStream_t st)
     return launch_pdl<ScaleParams>(kern, grid, dim3((unsigned)(nt + 32)), smem, st, p);
 }
 
-// WB_K1_LEAN=0 in the environment selects the generic row-pipeline kernel for fp32 too (A/B measurements).
-static bool k1_lean_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_K1_LEAN");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v != 0;
-}
-
-// Paired columns (x, x + M d) with M = 1 from d = 32 on; WB_K1_PAIR=0 in the environment keeps the nt-vector column
-// groups at every dilation (A/B measurements).  M = 2 at d = 16 and M = 4 at d = 8 were built and measured (the kernel
-// template takes them): no gain per launch and two more distinct kernels per cascade (0.336 -> 0.358 ms per transform
-// with the step loop unrolled by 8, profiles/r2_pair_levels.json) -- not instantiated.
-static int k1_pair_step(int taps, int d, int cols, int nt, int V = 4) {
-    static int level = -1;
-    if (level < 0) {
-        const char *e = getenv("WB_K1_PAIR");
-        level = e ? atoi(e) : 1;
-    }
-    (void)taps;
+// Paired columns (x, x + M d) with M = 1 from d = 32 on.  M = 2 at d = 16 and M = 4 at d = 8 were built and measured (the
+// kernel template takes them): no gain per launch and two more distinct kernels per cascade (0.336 -> 0.358 ms per
+// transform with the step loop unrolled by 8, profiles/r2_pair_levels.json) -- not instantiated.
+static bool k1_pair_step(int d, int cols, int nt, int V = 4) {
     // runs of d / V >= 8 consecutive vectors: eight consecutive lanes read eight consecutive vectors
-    if (d < 8 * V || (d & (d - 1)) != 0 || level <= 0) return 0;
+    if (d < 8 * V || (d & (d - 1)) != 0) return false;
     // thread t owns vectors (t / run) 2 run + t % run and + run of its strip: the consumer threads must cover every first
     // vector of the `cols` columns a block owns
     const int run = d / V, nvec = cols / V;
     const int need = ((nvec + 2 * run - 1) / (2 * run)) * run;
-    return need <= nt ? 1 : 0;
+    return need <= nt;
 }
 
-// WB_K1_UNROLL=8 in the environment selects the step loop unrolled by the whole ring (A/B measurements).
-static int k1_unroll() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_K1_UNROLL");
-        v = (e && atoi(e) == 8) ? 8 : 4;
-    }
-    return v;
-}
-
-template <int TAPS, int DMODE, bool HINTS, int OP = OP_TRANSFORM, int MODE = 0, int PAIR = 0>
+// The lean kernel on ring slots of RBK KiB: 16 (whole fp32 rows of 2049 .. 4096 columns), 8 (whole fp32 rows of
+// 1025 .. 2048 columns: two blocks per SM, so a 2048^2 frame runs 296 segments of 7 rows instead of 148 of 14 -- the
+// launch is bound by the number of steps per block) or kLeanStripKiB (column strips and float64 rows).
+template <typename T, int TAPS, int DMODE, bool HINTS, int OP, int MODE, int PAIR, int RBK>
 static int launch_rows_lean(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
-    const bool u8 = k1_unroll() == 8;
-    auto kern = u8 ? atrous_rows_lean_kernel<float, TAPS, DMODE, HINTS, OP, MODE, PAIR, 8>
-                   : atrous_rows_lean_kernel<float, TAPS, DMODE, HINTS, OP, MODE, PAIR, 4>;
-    const size_t smem = (size_t)kLeanSlots * kLeanRB + 16 * (size_t)kLeanSlots;
-    static bool configured[2][64] = {};  // per instantiation, per unroll, per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[u8][dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
-        if (e != cudaSuccess) return (int)e;
-        if (dev >= 0 && dev < 64) configured[u8][dev] = true;
-    }
-    dim3 grid((unsigned)((long long)p.n_strips * p.d * p.n_seg), (unsigned)batch);
-    return launch_pdl<ScaleParams>(kern, grid, dim3((unsigned)(nt + 32)), smem, st, p);
-}
-
-// The cascade kernel on whole fp32 rows of 1025 .. 2048 columns: 8 KiB ring slots, two blocks per SM (a 2048^2 frame then
-// runs 296 segments of 7 rows instead of 148 of 14: the launch is bound by the number of steps per block).
-template <int TAPS, int DMODE, int PAIR>
-static int launch_rows_lean_small(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
-    auto kern = atrous_rows_lean_kernel<float, TAPS, DMODE, true, OP_TRANSFORM, 0, PAIR, 4, 8>;
-    const size_t smem = (size_t)kLeanSlots * 8 * 1024 + 16 * (size_t)kLeanSlots;
+    auto kern = atrous_rows_lean_kernel<T, TAPS, DMODE, HINTS, OP, MODE, PAIR, RBK>;
+    const size_t smem = (size_t)kLeanSlots * RBK * 1024 + 16 * (size_t)kLeanSlots;
     static bool configured[64] = {};  // per instantiation, per device
     int dev = 0;
     cudaGetDevice(&dev);
@@ -613,45 +561,21 @@ static int launch_rows_lean_small(const ScaleParams &p, int batch, int nt, cudaS
 }
 
 // The lean kernel on column strips / float64 rows: ring slots of 24 KiB (a strip of 16 KiB plus the halo columns of
-// both sides), L2 hints on, step loop unrolled by half the ring.
+// both sides), L2 hints on.
 static constexpr int kLeanStripKiB = 24;
-
-// WB_K1_LEAN_STRIPS=0 in the environment keeps the generic kernel for float64 and for rows wider than one ring slot.
-static bool k1_lean_strips_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_K1_LEAN_STRIPS");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v != 0;
-}
-
-template <typename T, int TAPS, int DMODE, int OP, int MODE, int PAIR>
-static int launch_rows_lean_strip_m(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
-    auto kern = atrous_rows_lean_kernel<T, TAPS, DMODE, true, OP, MODE, PAIR, 4, kLeanStripKiB>;
-    const size_t smem = (size_t)kLeanSlots * kLeanStripKiB * 1024 + 16 * (size_t)kLeanSlots;
-    static bool configured[64] = {};  // per instantiation, per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem);
-        if (e != cudaSuccess) return (int)e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    dim3 grid((unsigned)((long long)p.n_strips * p.d * p.n_seg), (unsigned)batch);
-    return launch_pdl<ScaleParams>(kern, grid, dim3((unsigned)(nt + 32)), smem, st, p);
-}
 
 template <typename T, int TAPS, int DMODE, int OP, int PAIR>
 static int launch_rows_lean_strip(const ScaleParams &p, int batch, int nt, cudaStream_t st) {
+#define WB_STRIP(MODE) launch_rows_lean<T, TAPS, DMODE, true, OP, MODE, PAIR, kLeanStripKiB>(p, batch, nt, st)
     if constexpr (OP == OP_WHITEN) {
-        if (p.sig_mode == SIG_MAP) return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, SIG_MAP, PAIR>(p, batch, nt, st);
+        if (p.sig_mode == SIG_MAP) return WB_STRIP(SIG_MAP);
         if constexpr (sizeof(T) == 4) {
-            if (p.sig_mode == 1) return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, 1, PAIR>(p, batch, nt, st);
+            if (p.sig_mode == 1) return WB_STRIP(1);
         }
-        if (p.sig_mode == 2) return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, 2, PAIR>(p, batch, nt, st);
+        if (p.sig_mode == 2) return WB_STRIP(2);
     }
-    return launch_rows_lean_strip_m<T, TAPS, DMODE, OP, 0, PAIR>(p, batch, nt, st);
+    return WB_STRIP(0);
+#undef WB_STRIP
 }
 
 template <typename T, int TAPS, int OP>
@@ -661,47 +585,38 @@ static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
     K1Config cfg;
     if (fast_path_ok(p, TAPS, (int)sizeof(T)) && plan_fast(p, TAPS, (int)sizeof(T), batch, scale, &cfg, OP == OP_TRANSFORM)) {
         const int dmode = (p.d % V == 0) ? 0 : p.d;
+        // a geometry override (wb_tune_k1) runs the row kernel
+        const bool lean_ok = cfg.ng == 2 && cfg.slots == kLeanSlots && !(scale < 32 && g_override_set[scale]);
         if constexpr (sizeof(T) == 4 && OP == OP_TRANSFORM) {
             // whole-row strips with two vectors per thread and the default ring: the lean kernel
-            if (p.n_strips == 1 && cfg.ng == 2 && p.W > 1024 && cfg.slots == kLeanSlots && k1_lean_enabled() &&
-                !(scale < 32 && g_override_set[scale])) {
-#define WB_LEAN(DM) (p.l2_hints ? launch_rows_lean<TAPS, DM, true>(p, batch, cfg.nt, st) \
-                                : launch_rows_lean<TAPS, DM, false>(p, batch, cfg.nt, st))
-                if (p.W <= 2048 && p.l2_hints) {  // (the planner counted on two blocks per SM: plan_fast)
-                    if (dmode == 0 && k1_pair_step(TAPS, p.d, p.W, cfg.nt) == 1)
-                        return launch_rows_lean_small<TAPS, 0, 1>(p, batch, cfg.nt, st);
-                    if (dmode == 0) return launch_rows_lean_small<TAPS, 0, 0>(p, batch, cfg.nt, st);
-                    if (dmode == 1) return launch_rows_lean_small<TAPS, 1, 0>(p, batch, cfg.nt, st);
-                    if (dmode == 2) return launch_rows_lean_small<TAPS, 2, 0>(p, batch, cfg.nt, st);
+            if (p.n_strips == 1 && p.W > 1024 && lean_ok) {
+                const bool pair = dmode == 0 && k1_pair_step(p.d, p.W, cfg.nt);
+#define WB_LEAN(DM, H, PR, RBK) launch_rows_lean<T, TAPS, DM, H, OP, 0, PR, RBK>(p, batch, cfg.nt, st)
+                if (p.W <= 2048 && p.l2_hints) {  // 8 KiB slots (the planner counted on two blocks per SM: plan_fast)
+                    if (pair) return WB_LEAN(0, true, 1, 8);
+                    if (dmode == 0) return WB_LEAN(0, true, 0, 8);
+                    if (dmode == 1) return WB_LEAN(1, true, 0, 8);
+                    if (dmode == 2) return WB_LEAN(2, true, 0, 8);
                 }
-                if (dmode == 0 && p.l2_hints) {
-                    const int pair = k1_pair_step(TAPS, p.d, p.W, cfg.nt);
-                    if (pair == 1) return launch_rows_lean<TAPS, 0, true, OP_TRANSFORM, 0, 1>(p, batch, cfg.nt, st);
-                }
-                if (dmode == 0) return WB_LEAN(0);
-                if (dmode == 1) return WB_LEAN(1);
-                if (dmode == 2) return WB_LEAN(2);
+                if (pair && p.l2_hints) return WB_LEAN(0, true, 1, 16);
+                if (dmode == 0) return p.l2_hints ? WB_LEAN(0, true, 0, 16) : WB_LEAN(0, false, 0, 16);
+                if (dmode == 1) return p.l2_hints ? WB_LEAN(1, true, 0, 16) : WB_LEAN(1, false, 0, 16);
+                if (dmode == 2) return p.l2_hints ? WB_LEAN(2, true, 0, 16) : WB_LEAN(2, false, 0, 16);
 #undef WB_LEAN
             }
         }
         if constexpr (sizeof(T) == 4 && OP == OP_WHITEN) {
             // the whitening pass of the two-pass WOW routes on whole-row strips: lean kernel, hints on
-            if (p.n_strips == 1 && cfg.ng == 2 && p.W > 1024 && cfg.slots == kLeanSlots && k1_lean_enabled() &&
-                !(scale < 32 && g_override_set[scale])) {
-#define WB_LEANW_P(DM, PR)                                                                                        \
-    (p.sig_mode == 0 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 0, PR>(p, batch, cfg.nt, st)                    \
-     : p.sig_mode == 1 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 1, PR>(p, batch, cfg.nt, st)                  \
-     : p.sig_mode == 2 ? launch_rows_lean<TAPS, DM, true, OP_WHITEN, 2, PR>(p, batch, cfg.nt, st)                  \
-                       : launch_rows_lean<TAPS, DM, true, OP_WHITEN, SIG_MAP, PR>(p, batch, cfg.nt, st))
-#define WB_LEANW(DM) WB_LEANW_P(DM, 0)
-                if (dmode == 0) {
-                    const int pair = k1_pair_step(TAPS, p.d, p.W, cfg.nt);
-                    if (pair == 1) return WB_LEANW_P(0, 1);
-                }
-                if (dmode == 0) return WB_LEANW(0);
-                if (dmode == 1) return WB_LEANW(1);
-                if (dmode == 2) return WB_LEANW(2);
-#undef WB_LEANW_P
+            if (p.n_strips == 1 && p.W > 1024 && lean_ok) {
+#define WB_LEANW(DM, PR, M) launch_rows_lean<T, TAPS, DM, true, OP, M, PR, 16>(p, batch, cfg.nt, st)
+#define WB_LEANW_M(DM, PR)                                                                                            \
+    (p.sig_mode == 0 ? WB_LEANW(DM, PR, 0) : p.sig_mode == 1 ? WB_LEANW(DM, PR, 1)                                    \
+                     : p.sig_mode == 2 ? WB_LEANW(DM, PR, 2) : WB_LEANW(DM, PR, SIG_MAP))
+                if (dmode == 0 && k1_pair_step(p.d, p.W, cfg.nt)) return WB_LEANW_M(0, 1);
+                if (dmode == 0) return WB_LEANW_M(0, 0);
+                if (dmode == 1) return WB_LEANW_M(1, 0);
+                if (dmode == 2) return WB_LEANW_M(2, 0);
+#undef WB_LEANW_M
 #undef WB_LEANW
             }
         }
@@ -711,14 +626,12 @@ static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
         // fp32 strips 2 - 11 % faster at d >= 4 (kept; d < 4 keeps the generic kernel), float64 K1 equal within 2 % except
         // with paired columns (d >= 16: 1 - 5 us faster, kept), float64 K3 12 - 22 us faster per 4096^2 plane except with
         // the soft threshold (the inlined double-precision erf: 10 us slower, generic kept).
-        if ((sizeof(T) == 8 || p.n_strips > 1) && cfg.ng == 2 && cfg.slots == kLeanSlots && p.l2_hints &&
+        if ((sizeof(T) == 8 || p.n_strips > 1) && lean_ok && p.l2_hints &&
             (long long)p.row_stride * (long long)sizeof(T) <= (long long)kLeanStripKiB * 1024 &&
             // (only where the planner laid the segments out for ONE block per SM, which is what 24 KiB slots give)
-            2 * ((long long)kLeanSlots * p.row_stride * (long long)sizeof(T) + 16 * kLeanSlots + 1024) > (long long)kMaxSmem &&
-            k1_lean_enabled() && k1_lean_strips_enabled() &&
-            !(scale < 32 && g_override_set[scale])) {
+            2 * ((long long)kLeanSlots * p.row_stride * (long long)sizeof(T) + 16 * kLeanSlots + 1024) > (long long)kMaxSmem) {
             const int cols = p.n_strips == 1 ? p.W : p.wt;
-            const bool pair = dmode == 0 && k1_pair_step(TAPS, p.d, cols, cfg.nt, V) == 1;
+            const bool pair = dmode == 0 && k1_pair_step(p.d, cols, cfg.nt, V);
             if constexpr (sizeof(T) == 4) {
                 if (pair) return launch_rows_lean_strip<T, TAPS, 0, OP, 1>(p, batch, cfg.nt, st);
                 if (dmode == 0) return launch_rows_lean_strip<T, TAPS, 0, OP, 0>(p, batch, cfg.nt, st);

@@ -334,8 +334,6 @@ __device__ __forceinline__ u64 col_feed_p(u64 (&S)[TAPS - 1], u64 v, const Packe
 // Pieces of the LEAN fp32 kernels (wow_rows_lean_kernel, atrous_rows_lean_kernel): fixed 16 KiB ring slots so that
 // every shared-memory access is [per-thread register + immediate], step loops unrolled by the ring.
 // ---------------------------------------------------------------------------------------------------------------
-static constexpr uint32_t kLeanRB = 16384;  // bytes per ring slot (4096 fp32 columns)
-
 template <int OFF> __device__ __forceinline__ P4 lds_p4_imm(uint32_t a) {
     P4 r;
     asm volatile("ld.shared.v2.b64 {%0, %1}, [%2+%3];" : "=l"(r.lo), "=l"(r.hi) : "r"(a), "n"(OFF));

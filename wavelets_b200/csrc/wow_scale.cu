@@ -22,8 +22,8 @@
 // Rows outside the image are symmetric reflections: the loader fetches the reflected rows; because the symmetric
 // extension commutes with the symmetric smooth, c_{s+1} / w_s evaluated at such a virtual row equal their reflected
 // values (up to the rounding of a reversed summation order), which is what the power filter needs at the border.
-// The strip is normally the whole row, so the x border is an index reflection inside the staged row for both row
-// passes (same tap plan); wow_rows_kernel can also walk column strips (see plan_wow).  Away from the top/bottom border the arithmetic is exactly K1 followed by K3.
+// A block stages whole rows, so the x border is an index reflection inside the staged row for both row passes (same tap
+// plan).  Away from the top/bottom border the arithmetic is exactly K1 followed by K3.
 #include "pipeline.cuh"
 #include "whiten.cuh"
 
@@ -62,10 +62,11 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
     const int n_out = min(p.seg, n_chain - i0);
     if (n_out <= 0) return;
     const int n_load = n_out + 4 * C;  // input rows i0-2C .. i0+n_out+2C-1 of the chain (virtual rows are reflected)
-    // Column strip [x0, x1) of the outputs (whole row: one strip, halo_al = 0).  The power filter needs w_s on
+    // Column strip [x0, x1) of the outputs.  plan_wow plans whole rows (one strip, halo_al = 0), but the general strip
+    // indexing stays: without it ptxas allocates the registers of the float64 5-tap kernels differently (spills in the
+    // step loop) and a 2048^2 float64 scale takes 44 instead of 38 us.  The power filter needs w_s on
     // [e_lo, e_hi) = strip +- C d, which needs c_s on [lo, hi) = strip +- 2 C d: the block stages [lo, hi), every thread
-    // owns columns of [e_lo, e_hi) for BOTH passes, and only the columns inside the strip are stored (the halo
-    // columns' power sums read ring positions nobody wrote; they are never stored).
+    // owns columns of [e_lo, e_hi) for BOTH passes, and only the columns inside the strip are stored.
     const int x0 = strip * p.wt;
     const int x1 = min(p.W, x0 + p.wt);
     const int e_lo = max(0, x0 - p.halo_al), e_hi = min(p.W, x1 + p.halo_al);
@@ -76,7 +77,6 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
 
     const uint64_t pol_in = policy_evict_first();   // c_s is dead once this launch has read it
     const uint64_t pol_keep = policy_evict_last();  // c_{s+1}: the next scale reads it back
-    constexpr bool hints = HINTS, hints_c = HINTS;
     int next_load = 0;  // thread 0: next chain row to request
     pdl_wait();  // everything below touches global memory written or read by the previous launch
     if (tid == 0) {
@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
         for (; next_load < n0; ++next_load) {
             const long long y = reflect_any(y_first + (long long)next_load * p.d, p.H);
             mbar_arrive_expect_tx(&full[next_load], row_bytes);
-            if (hints) tma_load_1d_hint(smem_raw + (size_t)next_load * RB, src + y * p.in_pitch, row_bytes, &full[next_load], pol_in);
+            if (HINTS) tma_load_1d_hint(smem_raw + (size_t)next_load * RB, src + y * p.in_pitch, row_bytes, &full[next_load], pol_in);
             else tma_load_1d(smem_raw + (size_t)next_load * RB, src + y * p.in_pitch, row_bytes, &full[next_load]);
         }
     }
@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
                     const int sl = next_load & (kInRing - 1);
                     const long long y = reflect_any(y_first + (long long)next_load * p.d, p.H);
                     mbar_arrive_expect_tx(&full[sl], row_bytes);
-                    if (hints) tma_load_1d_hint(smem_raw + (size_t)sl * RB, src + y * p.in_pitch, row_bytes, &full[sl], pol_in);
+                    if (HINTS) tma_load_1d_hint(smem_raw + (size_t)sl * RB, src + y * p.in_pitch, row_bytes, &full[sl], pol_in);
                     else tma_load_1d(smem_raw + (size_t)sl * RB, src + y * p.in_pitch, row_bytes, &full[sl]);
                     ++next_load;
                 }
@@ -187,7 +187,7 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
 #pragma unroll
             for (int q = 0; q < NG; ++q) {
                 if (store_c && outm[q]) {
-                    if (hints_c) st_vec_hint(c_ptr + xg[q], cv[q], pol_keep);
+                    if (HINTS) st_vec_hint(c_ptr + xg[q], cv[q], pol_keep);
                     else st_vec(c_ptr + xg[q], cv[q]);
                 }
                 Pack<T, V> raw = lds_vec<T>(crow + xb[q]);
@@ -229,16 +229,22 @@ __global__ void __launch_bounds__(512, 1) wow_rows_kernel(const ScaleParams p) {
 // half a row apart, so both row passes load TAPS + M tap vectors for the two of them instead of 2 TAPS
 // (lean_row_pass_pair): with M = 1 (d >= 32) 18 instead of 26 LDS/STS.128 per thread and step; M = 2 for d = 16 (20), M = 4
 // for d = 8 (24) keep eight consecutive lanes on eight consecutive vectors (see pair_first_vector).
+// NTK: threads per block = half the vectors of the widest row the instantiation takes -- 512 (rows of 2049 .. 4096
+// columns, 16 KiB ring slots, one block per SM) or 256 (513 .. 2048 columns, 8 KiB slots, two blocks per SM).
 // DYN: the step loop is NOT unrolled -- ring slots and barrier parities are computed from the step index (warp-uniform
 // values: one more address term per shared-memory access) and the kernel is a quarter of the code.  The unrolled
 // kernel (60 - 90 KB) does not fit the instruction cache levels below L2, and every change of kernel inside a cascade
-// starts cold (see atrous_rows_lean_kernel).
-// NTK: threads per block = half the vectors of the widest row the instantiation takes -- 512 (rows of 2049 .. 4096
-// columns, 16 KiB ring slots, one block per SM) or 256 (513 .. 2048 columns, 8 KiB slots, two blocks per SM).
-template <int TAPS, int DMODE, bool HINTS, int MODE, int PAIR = 0, bool DYN = false, int NTK = 512>
+// starts cold (see atrous_rows_lean_kernel).  Measured at 4096^2 (profiles/r2_fused_dyn.json): not unrolled, a kernel
+// is 22 - 33 KB instead of 54 - 92 KB and no longer costs ~5 us of cold instruction cache, but the plain d % 4 == 0
+// kernels lose 2 us per launch in the steady state (47.1 -> 49.7, 41.5 -> 43.4 us: no scheduling across steps); the
+// d = 1 / d = 2 kernels lose nothing (39.8 us) and the kernels with an inlined erff / hard threshold are faster (scales
+// 0 / 1: 55.8 -> 52.3 us, paired: 65.5 -> 62.8 us).  So every hinted kernel but the plain d % 4 == 0 one is not
+// unrolled; the unhinted kernels (WB_L2_HINTS=0) keep the unrolled loop.
+template <int TAPS, int DMODE, bool HINTS, int MODE, int PAIR, int NTK>
 __global__ void __launch_bounds__(NTK, NTK == 512 ? 1 : 2) wow_rows_lean_kernel(const ScaleParams p) {
     static_assert(PAIR == 0 || (DMODE == 0 && PAIR < TAPS), "paired columns need d % 4 == 0 and overlapping taps");
     static_assert(NTK == 512 || NTK == 256, "block sizes the ring geometry was laid out for");
+    constexpr bool DYN = HINTS && (DMODE != 0 || MODE != 0);
     using T = float;
     constexpr int V = 4, NG = 2, NT = NTK;
     constexpr int C = TAPS / 2;
@@ -526,60 +532,32 @@ struct WowGeom { int nt, ng; size_t smem; };
 // blocks to the row)
 static constexpr int kLean256MinW = 512;
 
-// WB_WOW_STRIPS=k in the environment forces k column strips (>= 2) where the whole row would fit (A/B measurements).
-static int wow_forced_strips() {
-    const char *e = getenv("WB_WOW_STRIPS");
-    return e ? atoi(e) : 0;
-}
-
 static bool plan_wow(ScaleParams &p, int taps, int esize, int batch, WowGeom *geo) {
     const int V = 16 / esize;
     const int c = taps / 2;
     if (!fast_path_ok(p, taps, esize)) return false;
     if (!p.out_c || !p.out_w) return false;
     const int ng = 2;
-    const int rows = kInRing + kWRing + kW2Ring;
-    const int forced = wow_forced_strips();
-    int nt = 0;
-    size_t smem = 0;
-    // Whole-row strips when the row fits 512 threads x 2 vectors (W <= 4096 fp32 / 2048 fp64).  The kernel also runs
-    // COLUMN strips (WB_WOW_STRIPS=k: the fewest >= k strips whose staged range, strip + 4 C d columns, fits the 14-row
-    // ring and whose extended range, strip + 2 C d, fits the block), built for float64 rows of 4096 columns -- and
-    // measured SLOWER than the two-pass route there (4096^2 float64: 142 - 229 us per scale against 75 + 60 us for K1 +
-    // K3, profiles/r2_bench_wow_f64_v2.json: this generic kernel is bound by instruction issue, not by the bytes the
-    // fusion saves), so wider rows are declined (WB_ENOT_FUSABLE -> two passes) unless the variable forces strips.
-    const int halo = round_up(c * p.d, V);
-    int k_strips = 0;
-    for (int k = (forced >= 2 ? forced : 1); k <= 64; ++k) {
-        const int wt = (k == 1) ? p.W : round_up((p.W + k - 1) / k, V);
-        const int h = (k == 1) ? 0 : halo;
-        long long stage = (long long)wt + 4LL * h, ext = (long long)wt + 2LL * h;
-        if (stage > p.W) stage = p.W;
-        if (ext > p.W) ext = p.W;
-        const int need = round_up((int)((ext / V + ng - 1) / ng), 32);
-        const size_t sm = (size_t)rows * (size_t)stage * esize + 8 * (size_t)(kInRing + kW2Ring);
-        if (k > 1 && forced < 2) break;  // see the note above: strips are not chosen automatically
-        if (k > 1 && (2 * h > wt || 5 * ext > 8 * (long long)wt)) break;  // halo too wide: more than 1.6 x the columns
-        if (need <= 512 && sm <= (size_t)kMaxSmem) {
-            k_strips = k;
-            p.wt = wt;
-            p.halo_al = h;
-            p.row_stride = (int)stage;
-            nt = need;
-            smem = sm;
-            break;
-        }
-    }
-    if (!k_strips) return false;
-    p.n_strips = (p.W + p.wt - 1) / p.wt;
+    // Whole rows only, when the row fits 512 threads x 2 vectors (W <= 4096 fp32 / 2048 fp64) and the 14-row ring.  Wider
+    // rows are declined (WB_ENOT_FUSABLE -> two passes): a column-strip mode of the generic kernel, built for float64
+    // rows of 4096 columns, measured SLOWER than the two-pass route there (4096^2 float64: 142 - 229 us per scale against
+    // 75 + 60 us for K1 + K3, profiles/r2_bench_wow_f64_v2.json: this generic kernel is bound by instruction issue, not
+    // by the bytes the fusion saves).
+    const int nt = round_up((p.W / V + ng - 1) / ng, 32);
+    const size_t smem = (size_t)(kInRing + kWRing + kW2Ring) * (size_t)p.W * esize + 8 * (size_t)(kInRing + kW2Ring);
+    if (nt > 512 || smem > (size_t)kMaxSmem) return false;
+    p.n_strips = 1;
+    p.wt = p.W;
+    p.halo_al = 0;
+    p.row_stride = p.W;
     p.slots = kInRing;
     const int n_max = (p.H + p.d - 1) / p.d;
-    const long long chains = (long long)p.n_strips * (p.d < p.H ? p.d : p.H) * batch;
+    const long long chains = (long long)(p.d < p.H ? p.d : p.H) * batch;
     int occ = (int)(kMaxSmem / (smem + 1024));
     const int occ_regs = 65536 / (nt * 128);
     if (occ > occ_regs) occ = occ_regs;
     // the 256-thread lean kernel (fp32 rows of 513 .. 2048 columns, see launch_wow_h) runs two blocks per SM
-    if (esize == 4 && p.n_strips == 1 && p.W > kLean256MinW && p.W <= 2048 && occ > 2) occ = 2;
+    if (esize == 4 && p.W > kLean256MinW && p.W <= 2048 && occ > 2) occ = 2;
     if (occ < 1) occ = 1;
     const long long slots_total = (long long)device_sm_count() * occ;
     long long per_chain = slots_total / chains;
@@ -598,65 +576,6 @@ static bool plan_wow(ScaleParams &p, int taps, int esize, int batch, WowGeom *ge
     return true;
 }
 
-// WB_WOW_LEAN=0 in the environment selects the generic kernel for fp32 too (A/B measurements, bit-identity tests).
-static bool wow_packed_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_WOW_LEAN");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v != 0;
-}
-
-// WB_WOW_PAIR=0 in the environment keeps the half-row column groups at every dilation (A/B measurements).
-static int wow_pair_level() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_WOW_PAIR");
-        v = e ? atoi(e) : 1;
-    }
-    return v;
-}
-
-// Which lean kernels run with the step loop NOT unrolled (DYN).  Measured at 4096^2 (profiles/r2_fused_dyn.json): not
-// unrolled, a kernel is 22 - 33 KB instead of 54 - 92 KB and a change of kernel inside a cascade no longer costs ~5 us of
-// cold instruction cache, but the plain d % 4 == 0 kernels lose 2 us per launch in the steady state (47.1 -> 49.7,
-// 41.5 -> 43.4 us: no scheduling across steps); the d = 1 / d = 2 kernels lose nothing (39.8 us) and the kernels with
-// an inlined erff / hard threshold are faster (scales 0 / 1: 55.8 -> 52.3 us, paired: 65.5 -> 62.8 us).  Default: not
-// unrolled unless the kernel is the plain d % 4 == 0 one; WB_WOW_DYN=0 / 1 in the environment: never / always.
-static bool wow_dyn_for(int dmode, int sig_mode) {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("WB_WOW_DYN");
-        v = e ? (e[0] == '0' ? 0 : 1) : 2;
-    }
-    if (v < 2) return v != 0;
-    return dmode != 0 || sig_mode != 0;
-}
-
-template <int TAPS, int DMODE, bool HINTS, int M, bool DYN>
-static auto wow_lean_kernel_mode(int sig_mode) -> void (*)(const ScaleParams) {
-    return sig_mode == 0 ? wow_rows_lean_kernel<TAPS, DMODE, HINTS, 0, M, DYN>
-                         : (sig_mode == 1 ? wow_rows_lean_kernel<TAPS, DMODE, HINTS, 1, M, DYN>
-                                          : wow_rows_lean_kernel<TAPS, DMODE, HINTS, 2, M, DYN>);
-}
-
-template <typename T, int TAPS, int DMODE, bool HINTS>
-static auto wow_kernel_for(bool packed, int pair, bool dyn, int sig_mode) -> void (*)(const ScaleParams) {
-    if constexpr (sizeof(T) == 4) {
-        if constexpr (HINTS) {
-            if constexpr (DMODE == 0) {
-                if (packed && pair == 1)
-                    return dyn ? wow_lean_kernel_mode<TAPS, 0, true, 1, true>(sig_mode)
-                               : wow_lean_kernel_mode<TAPS, 0, true, 1, false>(sig_mode);
-            }
-            if (packed && dyn) return wow_lean_kernel_mode<TAPS, DMODE, true, 0, true>(sig_mode);
-        }
-        if (packed) return wow_lean_kernel_mode<TAPS, DMODE, HINTS, 0, false>(sig_mode);
-    }
-    return wow_rows_kernel<T, TAPS, DMODE, 2, HINTS>;
-}
-
 // Paired columns (x, x + M d): M = 1 from d = 32 on (runs of d / 4 >= 8 consecutive vectors keep the LDS.128 of eight
 // consecutive lanes conflict-free).  M = 2 at d = 16 and M = 4 at d = 8 were built and measured (the kernel template
 // takes them): alone the d = 16 launch gains 7 us (48 -> 41), inside wow() the two additional kernels per cascade cost
@@ -665,52 +584,49 @@ static auto wow_kernel_for(bool packed, int pair, bool dyn, int sig_mode) -> voi
 // threads must cover every first vector of the W / 4 vectors.  They do not at d = W (Triangle on a power-of-two row:
 // the second vectors all fall beyond the row and half of it would never be written), so that case, like the K1 kernels
 // (k1_pair_step), keeps the half-row column groups.
-static int wow_pair_step(int taps, int d, int W, int nt) {
-    (void)taps;
-    if (d < 32 || (d & (d - 1)) != 0 || wow_pair_level() <= 0) return 0;
+static bool wow_pair_step(int d, int W, int nt) {
+    if (d < 32 || (d & (d - 1)) != 0) return false;
     const int run = d / 4, nvec = W / 4;
     const int need = ((nvec + 2 * run - 1) / (2 * run)) * run;
-    return need <= nt ? 1 : 0;
+    return need <= nt;
 }
 
-// Rows of 513 .. 2048 columns: 256-thread blocks on 8 KiB slots, two per SM, with the default choice of not-unrolled /
-// unrolled kernels only (hints on).
-template <int TAPS, int DMODE>
-static auto wow_lean256_kernel(int pair, int sig_mode) -> void (*)(const ScaleParams) {
-    if constexpr (DMODE == 0) {
-        if (pair == 1)
-            return sig_mode == 0 ? wow_rows_lean_kernel<TAPS, 0, true, 0, 1, false, 256>
-                                 : (sig_mode == 1 ? wow_rows_lean_kernel<TAPS, 0, true, 1, 1, true, 256>
-                                                  : wow_rows_lean_kernel<TAPS, 0, true, 2, 1, true, 256>);
-        return sig_mode == 0 ? wow_rows_lean_kernel<TAPS, 0, true, 0, 0, false, 256>
-                             : (sig_mode == 1 ? wow_rows_lean_kernel<TAPS, 0, true, 1, 0, true, 256>
-                                              : wow_rows_lean_kernel<TAPS, 0, true, 2, 0, true, 256>);
-    } else {
-        return sig_mode == 0 ? wow_rows_lean_kernel<TAPS, DMODE, true, 0, 0, true, 256>
-                             : (sig_mode == 1 ? wow_rows_lean_kernel<TAPS, DMODE, true, 1, 0, true, 256>
-                                              : wow_rows_lean_kernel<TAPS, DMODE, true, 2, 0, true, 256>);
+// The lean kernel of one block size, significance mode and column layout.  Paired columns need d % 4 == 0 and L2 hints.
+template <int TAPS, int DMODE, bool HINTS, int NTK>
+static auto wow_lean_kernel(bool pair, int sig_mode) -> void (*)(const ScaleParams) {
+#define WB_MODES(PR)                                                                                                  \
+    (sig_mode == 0 ? wow_rows_lean_kernel<TAPS, DMODE, HINTS, 0, PR, NTK>                                             \
+                   : sig_mode == 1 ? wow_rows_lean_kernel<TAPS, DMODE, HINTS, 1, PR, NTK>                             \
+                                   : wow_rows_lean_kernel<TAPS, DMODE, HINTS, 2, PR, NTK>)
+    if constexpr (DMODE == 0 && HINTS) {
+        if (pair) return WB_MODES(1);
     }
+    return WB_MODES(0);
+#undef WB_MODES
 }
 
 template <typename T, int TAPS, int DMODE, bool HINTS>
 static int launch_wow_h(const ScaleParams &p, int batch, const WowGeom &geo, cudaStream_t st) {
     // the lean kernel runs 512 threads x 2 vectors on 16 KiB ring slots (rows of 2049 .. 4096 columns) or 256 threads on
     // 8 KiB slots (513 .. 2048 columns; hints on); narrower rows and float64 keep the generic kernel
-    const bool lean_ok = sizeof(T) == 4 && p.n_strips == 1 && wow_packed_enabled();
-    const bool packed = lean_ok && p.W > 2048;
-    const bool packed256 = lean_ok && HINTS && p.W > kLean256MinW && p.W <= 2048 && geo.ng == 2;
-    const int pair = ((packed || packed256) && DMODE == 0 && HINTS) ? wow_pair_step(TAPS, p.d, p.W, packed ? 512 : 256) : 0;
-    const bool dyn = packed && HINTS && wow_dyn_for(DMODE, p.sig_mode);
-    void (*kern)(const ScaleParams) = nullptr;
-    if constexpr (sizeof(T) == 4 && HINTS) {
-        if (packed256) kern = wow_lean256_kernel<TAPS, DMODE>(pair, p.sig_mode);
+    void (*kern)(const ScaleParams) = wow_rows_kernel<T, TAPS, DMODE, 2, HINTS>;
+    int nt = geo.nt, kidx = 0;  // kidx: generic, lean-512 x 3 significance modes x {plain, paired}, lean-256 x 3 x 2
+    size_t smem = geo.smem;
+    if constexpr (sizeof(T) == 4) {
+        const bool lean512 = p.W > 2048;
+        const bool lean256 = HINTS && p.W > kLean256MinW && p.W <= 2048 && geo.ng == 2;
+        if (lean512 || lean256) {
+            nt = lean512 ? 512 : 256;
+            const bool pair = DMODE == 0 && HINTS && wow_pair_step(p.d, p.W, nt);
+            if (lean512) kern = wow_lean_kernel<TAPS, DMODE, HINTS, 512>(pair, p.sig_mode);
+            if constexpr (HINTS) {
+                if (lean256) kern = wow_lean_kernel<TAPS, DMODE, true, 256>(pair, p.sig_mode);
+            }
+            smem = (size_t)(kInRing + kWRing) * (size_t)nt * 32 + 8 * (size_t)(kInRing + kWRing);
+            kidx = (lean512 ? 1 : 7) + p.sig_mode + 3 * (pair ? 1 : 0);
+        }
     }
-    if (!kern) kern = wow_kernel_for<T, TAPS, DMODE, HINTS>(packed, pair, dyn, p.sig_mode);
-    const int nt = packed ? 512 : (packed256 ? 256 : geo.nt);
-    const size_t smem = (packed || packed256) ? (size_t)(kInRing + kWRing) * (size_t)nt * 32 + 8 * (size_t)(kInRing + kWRing) : geo.smem;
-    // generic, lean x 3 significance modes x {plain, paired} x {unrolled, not}, lean-256 x 3 x {plain, paired}; per device
-    static bool configured[19][64] = {};
-    const int kidx = packed ? 1 + p.sig_mode + 3 * pair + 6 * (dyn ? 1 : 0) : (packed256 ? 13 + p.sig_mode + 3 * pair : 0);
+    static bool configured[13][64] = {};  // per kernel (kidx), per device
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !configured[kidx][dev]) {
@@ -754,15 +670,7 @@ static int fill_wow_params(ScaleParams &p, const void *in, void *out_c, void *ou
     p.in_pitch = in_pitch; p.in_bstride = in_bstride;
     p.c_pitch = c_pitch; p.c_bstride = c_bstride;
     p.w_pitch = w_pitch; p.w_bstride = w_bstride;
-    {
-        static int v = -1;  // WB_L2_HINTS_WOW=0/1/2/3 (bit 0: input evict-first, bit 1: c_{s+1} evict-last); A/B measurements
-        if (v < 0) {
-            const char *e = getenv("WB_L2_HINTS_WOW");
-            v = e ? atoi(e) : 3;
-        }
-        p.l2_hints = l2_hints_enabled() ? v : 0;
-    }
-
+    p.l2_hints = l2_hints_enabled();
     return WB_OK;
 }
 
