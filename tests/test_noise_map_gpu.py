@@ -180,22 +180,16 @@ def _frame(shape, dt, seed=3, flux=0.05):
 @pytest.mark.parametrize("case", range(len(WOW_MAP_CASES)))
 def test_wow_map_equals_parent_route(case):
     import wavelets_b200 as wb
-    from wavelets_b200 import utils
     shape, dt, kw = WOW_MAP_CASES[case]
     kw = dict(kw)
     sf = _sf(kw.pop("scaling_function", "b3spline"))
     img = torch.from_numpy(_frame(shape, dt)).cuda()
     nmap = torch.from_numpy(_photon_map(_frame(shape, dt))).cuda()
     r_ref, p_ref = _parent_map_route(img, nmap, sf, **kw)
-    try:
-        for c_cascade in (True, False):
-            utils.C_CASCADE = c_cascade
-            r, co = wb.wow(img, scaling_function=sf, noise=nmap, **kw)
-            _assert_bitwise(r, r_ref, (case, c_cascade, "recon"))
-            _assert_bitwise(co.data, p_ref, (case, c_cascade, "planes"))
-            assert co.noise is nmap
-    finally:
-        utils.C_CASCADE = True
+    r, co = wb.wow(img, scaling_function=sf, noise=nmap, **kw)
+    _assert_bitwise(r, r_ref, (case, "recon"))
+    _assert_bitwise(co.data, p_ref, (case, "planes"))
+    assert co.noise is nmap
     # wow() on existing coefficients with a map (the per-scale entry point)
     n_scales = len(p_ref) - 1
     co = wb.AtrousTransform(sf, bilateral=kw.get("bilateral"), bilateral_scaling=kw.get("bilateral_scaling", False))(
@@ -232,7 +226,6 @@ def _stack(n, shape=(192, 256), dt=np.float32):
 @pytest.mark.parametrize("kw", range(len(BATCH_KW)))
 def test_wow_batch_noise_forms_equal_single_calls(kw):
     import wavelets_b200 as wb
-    from wavelets_b200 import utils
     kw = BATCH_KW[kw]
     frames = _stack(3)
     maps = np.stack([_photon_map(f) for f in frames])
@@ -241,22 +234,17 @@ def test_wow_batch_noise_forms_equal_single_calls(kw):
              ("vec_t", torch.from_numpy(vec).cuda(), lambda i: float(vec[i])),
              ("shared", maps[0], lambda i: maps[0]),
              ("per_frame", torch.from_numpy(maps), lambda i: maps[i])]
-    try:
-        for c_cascade in (True, False):
-            utils.C_CASCADE = c_cascade
-            for name, noise, single in forms:
-                recon, planes, used = wb.wow_batch(frames, noise=noise, **kw)
-                for i in range(len(frames)):
-                    r, co = wb.wow(frames[i], noise=single(i), **kw)
-                    r = torch.from_numpy(r).cuda()
-                    _assert_bitwise(recon[i], r, (name, c_cascade, i, "recon"))
-                    _assert_bitwise(planes[i], co.data, (name, c_cascade, i, "planes"))
-                if name.startswith("vec"):
-                    assert used.dtype == torch.float64 and used.shape == (3,)
-                else:
-                    assert used.dtype == torch.float32 and tuple(used.shape) == np.shape(noise)
-    finally:
-        utils.C_CASCADE = True
+    for name, noise, single in forms:
+        recon, planes, used = wb.wow_batch(frames, noise=noise, **kw)
+        for i in range(len(frames)):
+            r, co = wb.wow(frames[i], noise=single(i), **kw)
+            r = torch.from_numpy(r).cuda()
+            _assert_bitwise(recon[i], r, (name, i, "recon"))
+            _assert_bitwise(planes[i], co.data, (name, i, "planes"))
+        if name.startswith("vec"):
+            assert used.dtype == torch.float64 and used.shape == (3,)
+        else:
+            assert used.dtype == torch.float32 and tuple(used.shape) == np.shape(noise)
 
 
 def test_wow_batch_rejects_bad_noise_shapes():

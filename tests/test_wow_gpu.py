@@ -238,13 +238,62 @@ def test_wow_batch_matches_single_frames():
     assert np.array_equal(rb[0].cpu().numpy(), r0)
 
 
-def test_wow_c_cascade_equals_python_loop():
-    """wb_wow_cascade (the whole WOW pipeline, plain or bilateral, in one library call) against the Python loop over the same entry
-    points, bit for bit: default, MAD noise from the raw w_0 (scale 0) and from the whitened plane 0 (first threshold at
-    scale 1), given noise (host scalar and device scalar), hard thresholds, weights, Triangle, float64, shapes the fused
-    kernel declines (two-pass inside the call), batches."""
+def _wow_per_scale(stack, scaling_function=None, n_scales=None, weights=(), denoise_coefficients=(), noise=None,
+                   bilateral=None, bilateral_scaling=False, soft_threshold=True):
+    """Reference for wb_wow_cascade: the same launches, issued one per-scale entry point at a time.  Per scale the fused
+    wb_wow_scale, or where the scale is bilateral, the noise is a map, the MAD noise must first be estimated from the raw
+    w_0 or the fused kernel declines: wb_atrous_scale[_bilateral] (+ wb_abs_median of the raw w_0) and the whitening K3.
+    The noise is estimated lazily from the whitened plane 0 when the first threshold comes later.  Then the residual
+    rescale and the synthesis.  ``stack`` is (B, H, W) on the device; returns (recon, planes, noise as a _Noise)."""
     import wavelets_b200 as wb
-    from wavelets_b200 import utils
+    from wavelets_b200 import _lib, utils
+    from wavelets_b200.wavelets import _Noise, abs_median_noise, atrous_scale, plane_moments, synthesis
+    lib = _lib.load(require_cuda=True)
+    sfc = scaling_function or wb.B3spline
+    b, h, w = stack.shape
+    L, sigma_bilateral, wts, dns = utils._wow_plan((h, w), sfc, n_scales, weights, denoise_coefficients, bilateral)
+    sf = sfc(2)
+    sigma_e = sf.sigma_e(bilateral=sigma_bilateral)
+    factors = [None] * L if sigma_bilateral is None else \
+        wb.AtrousTransform(sfc, bilateral=sigma_bilateral, bilateral_scaling=bilateral_scaling).var_factors(L)
+    nz = utils._stack_noise(noise, b, h, w, stack.dtype, stack.device)
+    nz_map = None if nz is None else nz.map
+    planes = torch.empty((b, L + 1, h, w), dtype=stack.dtype, device=stack.device)
+    scratch = torch.empty((2, b, h, w), dtype=stack.dtype, device=stack.device)
+    raw = torch.empty_like(stack)
+    src = stack
+    for s in range(L):
+        dst_c = planes[:, L] if s == L - 1 else scratch[s & 1]
+        d, wt = dns[s], wts[s]
+        need_sig = d != 0
+        mode = (1 if soft_threshold else 2) if need_sig else 0
+        se = sigma_e[s] if need_sig else 1.0
+        if need_sig and nz is None and s > 0:
+            nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
+        fused = factors[s] is None and nz_map is None and not (need_sig and nz is None) and \
+            utils._wow_scale_fused(lib, src, dst_c, planes[:, s], s, sf, mode, d, se, nz if need_sig else _Noise(), wt)
+        if not fused:
+            atrous_scale(src, s, sf, out_c=dst_c, out_w=raw, var_factor=factors[s])
+            if need_sig and nz is None:
+                nz = _Noise(dev=abs_median_noise(raw, sigma_e[0]))
+            if need_sig and nz_map is not None:
+                utils._whiten_scale_map(lib, raw, planes[:, s], nz_map, s, sf, soft_threshold, d, sigma_e[s], wt)
+            else:
+                utils._whiten_scale(lib, raw, planes[:, s], s, sf, mode, d, se, nz if need_sig else _Noise(), wt)
+        src = dst_c
+    last = planes[:, L]
+    mom = plane_moments(last)
+    _lib.check(lib.wb_residual_rescale(last.data_ptr(), h * w, b, (L + 1) * h * w, _lib.dtype_code(stack.dtype),
+                                       mom.data_ptr(), float(wts[L]), _lib.stream_ptr(stack.device)))
+    return synthesis(planes), planes, nz
+
+
+def test_wow_cascade_equals_per_scale_entry_points():
+    """wb_wow_cascade (the whole WOW pipeline, plain or bilateral, in one library call) against the same launches issued
+    per scale, bit for bit: default, MAD noise from the raw w_0 (scale 0) and from the whitened plane 0 (first threshold
+    at scale 1), given noise (host scalar and device scalar), hard thresholds, weights, Triangle, float64, shapes the
+    fused kernel declines (two-pass inside the call), batches."""
+    import wavelets_b200 as wb
     cases = [((256, 256), np.float32, {}), ((256, 256), np.float32, {"denoise_coefficients": [5, 2]}),
              ((192, 320), np.float32, {"denoise_coefficients": [0, 3, 1]}),
              ((130, 1024), np.float32, {"denoise_coefficients": [4, 2], "noise": 0.7}),
@@ -255,31 +304,31 @@ def test_wow_c_cascade_equals_python_loop():
              ((256, 256), np.float32, {"bilateral": 1, "denoise_coefficients": [5, 2]}),
              ((96, 1536), np.float32, {"bilateral": [1, 2], "denoise_coefficients": [0, 3], "bilateral_scaling": True}),
              ((128, 128), np.float64, {"bilateral": 1, "noise": 0.5, "denoise_coefficients": [4, 1]})]
-    try:
-        for shape, dt, kw in cases:
-            img = orc.solar_like(max(shape), seed=3, flux=0.05, dtype=dt)[:shape[0], :shape[1]].copy()
-            dev = torch.from_numpy(img).cuda()
-            utils.C_CASCADE = True
-            r1, c1 = wb.wow(dev, **kw)
-            utils.C_CASCADE = False
-            r0, c0 = wb.wow(dev, **kw)
-            assert torch.equal(r1, r0) and torch.equal(c1.data, c0.data), (shape, dt, kw)
-            assert (c1.noise is None and c0.noise is None) or c1.noise == c0.noise, (shape, kw)
-        dev_noise = torch.tensor([0.7], dtype=torch.float64, device="cuda")
-        img = torch.from_numpy(orc.solar_like(256, seed=5, flux=0.05, dtype=np.float32)).cuda()
-        utils.C_CASCADE = True
-        r1, c1 = wb.wow(img, denoise_coefficients=[4, 2], noise=dev_noise)
-        utils.C_CASCADE = False
-        r0, c0 = wb.wow(img, denoise_coefficients=[4, 2], noise=dev_noise)
-        assert torch.equal(r1, r0) and torch.equal(c1.data, c0.data)
-        frames = np.stack([orc.solar_like(256, seed=s, flux=0.05, dtype=np.float32) for s in (1, 2, 3)])
-        utils.C_CASCADE = True
-        rb1, pb1, nb1 = wb.wow_batch(frames, denoise_coefficients=[5, 2])
-        utils.C_CASCADE = False
-        rb0, pb0, nb0 = wb.wow_batch(frames, denoise_coefficients=[5, 2])
-        assert torch.equal(rb1, rb0) and torch.equal(pb1, pb0) and torch.equal(nb1, nb0)
-    finally:
-        utils.C_CASCADE = True
+    for shape, dt, kw in cases:
+        img = orc.solar_like(max(shape), seed=3, flux=0.05, dtype=dt)[:shape[0], :shape[1]].copy()
+        dev = torch.from_numpy(img).cuda()
+        r1, c1 = wb.wow(dev, **kw)
+        r0, p0, n0 = _wow_per_scale(dev.unsqueeze(0), **kw)
+        assert torch.equal(r1, r0[0]) and torch.equal(c1.data, p0[0]), (shape, dt, kw)
+        if n0 is None:
+            assert c1.noise is None, (shape, kw)
+        else:
+            assert c1.noise == (n0.dev.item() if n0.dev is not None else n0.host), (shape, kw)
+    dev_noise = torch.tensor([0.7], dtype=torch.float64, device="cuda")
+    img = torch.from_numpy(orc.solar_like(256, seed=5, flux=0.05, dtype=np.float32)).cuda()
+    r1, c1 = wb.wow(img, denoise_coefficients=[4, 2], noise=dev_noise)
+    r0, p0, _ = _wow_per_scale(img.unsqueeze(0), denoise_coefficients=[4, 2], noise=dev_noise)
+    assert torch.equal(r1, r0[0]) and torch.equal(c1.data, p0[0])
+    nmap = torch.sqrt(1.5 * img.clamp(min=0) + 9)  # wb_wow_cascade_map
+    for kw in ({"denoise_coefficients": [4, 0, 2]},
+               {"bilateral": 1, "denoise_coefficients": [5, 2], "soft_threshold": False}):
+        r1, c1 = wb.wow(img, noise=nmap, **kw)
+        r0, p0, _ = _wow_per_scale(img.unsqueeze(0), noise=nmap, **kw)
+        assert torch.equal(r1, r0[0]) and torch.equal(c1.data, p0[0]), kw
+    frames = np.stack([orc.solar_like(256, seed=s, flux=0.05, dtype=np.float32) for s in (1, 2, 3)])
+    rb1, pb1, nb1 = wb.wow_batch(frames, denoise_coefficients=[5, 2])
+    rb0, pb0, nb0 = _wow_per_scale(torch.from_numpy(frames).cuda(), denoise_coefficients=[5, 2])
+    assert torch.equal(rb1, rb0) and torch.equal(pb1, pb0) and torch.equal(nb1, nb0.dev)
 
 
 def test_wow_stream_of_host_frames_matches_per_frame_calls():
@@ -415,17 +464,14 @@ def test_wow_fused_scale_equals_two_pass(dt, sf):
     o1, o2 = torch.zeros_like(odd), torch.zeros_like(odd)
     assert not utils._wow_scale_fused(lib, odd, o1, o2, 0, scf, 0, 0.0, 1.0, utils._Noise(), 1.0)
     assert not out1.any() and not o1.any()
-    # whole pipeline: fused and two-pass wow() agree bit for bit
+    # whole pipeline: wow() of the image (fused scales) and wow() of its coefficients (K3 on every raw plane) agree
     img = torch.from_numpy(orc.solar_like(512, seed=3, flux=0.05, dtype=np.dtype(dt).type)).cuda()
     for kw in ({}, dict(denoise_coefficients=[5, 2]), dict(denoise_coefficients=[0, 3], soft_threshold=False, noise=2.0),
                dict(weights=[0.5, 2.0], noise=1.5, denoise_coefficients=[4])):
-        utils.FUSED_WOW = True
         r1, c1 = wb.wow(img, scaling_function=_sf(sf), **kw)
-        utils.FUSED_WOW = False
-        try:
-            r2, c2 = wb.wow(img, scaling_function=_sf(sf), **kw)
-        finally:
-            utils.FUSED_WOW = True
+        c2 = wb.AtrousTransform(_sf(sf))(img, len(c1) - 1)
+        c2.noise = kw.get("noise")
+        r2, _ = wb.wow(c2, **{k: v for k, v in kw.items() if k != "noise"})
         if kw.get("soft_threshold", True):
             assert orc.emax(r1.cpu().numpy(), r2.cpu().numpy()) < (1e-5 if dt == "float32" else 1e-12), kw
             assert orc.emax(c1.data.cpu().numpy(), c2.data.cpu().numpy()) < (1e-5 if dt == "float32" else 1e-12), kw

@@ -70,19 +70,15 @@ def main():
 
     for name, kw in (("default", {}), ("den", dict(denoise_coefficients=[5, 2])),
                      ("bil_den", dict(bilateral=1, denoise_coefficients=[5, 2])), ("bil", dict(bilateral=1))):
-        for fused in (True, False):
-            utils.FUSED_WOW = fused
-            ms = timed(lambda: wb.wow(img, **kw), args.reps)
-            L = len(wb.wow(img, **kw)[1]) - 1
-            algo = (5 * L + 3) * es * n * n
-            res["wow"][f"{name}{'' if fused else '_twopass'}"] = {
-                "ms": ms, "frames_per_s": 1e3 / ms, "scales": L, "algorithmic_gb": algo / 1e9,
-                "achieved_gbs": algo / ms / 1e6, "frac": algo / ms / 1e6 / peak}
-            print(name, "fused" if fused else "two-pass", f"{ms:.3f} ms  {1e3 / ms:.1f} frames/s  "
-                  f"{algo / ms / 1e6:.0f} GB/s algorithmic ({algo / ms / 1e6 / peak:.1%})", flush=True)
-    utils.FUSED_WOW = True
+        ms = timed(lambda: wb.wow(img, **kw), args.reps)
+        L = len(wb.wow(img, **kw)[1]) - 1
+        algo = (5 * L + 3) * es * n * n
+        res["wow"][name] = {"ms": ms, "frames_per_s": 1e3 / ms, "scales": L, "algorithmic_gb": algo / 1e9,
+                            "achieved_gbs": algo / ms / 1e6, "frac": algo / ms / 1e6 / peak}
+        print(name, f"{ms:.3f} ms  {1e3 / ms:.1f} frames/s  "
+              f"{algo / ms / 1e6:.0f} GB/s algorithmic ({algo / ms / 1e6 / peak:.1%})", flush=True)
 
-    # per-kernel, per-scale launch times
+    # per-kernel, per-scale launch times (k1 + k3_whiten against fused: the two-pass and the fused route of a scale)
     src = img.unsqueeze(0)
     c = torch.empty_like(src)
     w = torch.empty_like(src)

@@ -88,22 +88,21 @@ def main():
             torch.cuda.empty_cache()
     # ---- WOW on bands (two halo exchanges per scale + all-gather of the residual moments) vs the unsharded two-pass wow
     if not args.no_check and not args.quick:
-        from wavelets_b200 import utils
         from wavelets_b200.sharded import BandedWow
         for dt in (torch.float32, torch.float64):
             gen = torch.Generator(device=dev).manual_seed(11)
             img = (torch.randn((h, w), generator=gen, device=dev, dtype=torch.float32) * 5 + 40).to(dt)
             # noise given for float32; float64 estimates it (distributed exact MAD of the raw w_0)
-            kw = dict(n_scales=min(args.levels, 6), weights=[1.5, 1.2], denoise_coefficients=[4, 2])
+            kw = dict(weights=[1.5, 1.2], denoise_coefficients=[4, 2])
             if dt == torch.float32:
                 kw["noise"] = 1.5
-            recon_b, planes_b = BandedWow(wb.B3spline, poison=True)(img[y0:y1].contiguous(), h, **kw)
-            utils.FUSED_WOW = False
-            try:
-                recon, co = wb.wow(img, **kw)
-            finally:
-                utils.FUSED_WOW = True
+            recon_b, planes_b = BandedWow(wb.B3spline, poison=True)(img[y0:y1].contiguous(), h,
+                                                                    n_scales=min(args.levels, 6), **kw)
             L = planes_b.shape[0] - 1
+            # two-pass reference: wow() of the unsharded coefficients whitens every raw plane with K3
+            co = wb.AtrousTransform(wb.B3spline)(img, L)
+            co.noise = kw.pop("noise", None)
+            recon, co = wb.wow(co, **kw)
             same = torch.equal(planes_b[:L], co.data[:L, y0:y1])
             tol = 1e-5 if dt == torch.float32 else 1e-12
             close = ((recon_b - recon[y0:y1]).abs().max() <= tol * recon.abs().max()) and \

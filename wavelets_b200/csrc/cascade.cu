@@ -1,11 +1,13 @@
 // The WOW pipeline of a stack of frames in ONE library call: the loop of watroo/utils.py:172-205 (whitening on) on the
-// plain or the bilateral cascade, i.e. what wavelets_b200.utils._wow_stack issues scale by scale -- per scale wb_wow_scale
-// (or, for bilateral scales, where the fused kernel declines, or when the MAD noise has to be estimated from the raw w_0
-// first: wb_atrous_scale / wb_atrous_scale_bilateral [+ wb_abs_median] + wb_wow_whiten_scale), then wb_plane_moments +
+// plain or the bilateral cascade, as a sequence of the per-scale entry points -- per scale wb_wow_scale (or, for
+// bilateral scales, where the fused kernel declines, or when the MAD noise has to be estimated from the raw w_0 first:
+// wb_atrous_scale / wb_atrous_scale_bilateral [+ wb_abs_median] + wb_wow_whiten_scale), then wb_plane_moments +
 // wb_residual_rescale of the residual plane and wb_synthesis.  wb_wow_cascade_map runs the same loop with a per-pixel
-// noise map: two passes at every scale, the thresholded ones whitened by wb_wow_whiten_scale_map.  Host code
-// only: it exists because a 512^2 .. 2048^2 frame is finished on the device long before a Python loop has issued its
-// fifteen launches (0.27 - 0.30 ms of interpreter and ctypes time per wow() call, measured; profiles/r2_sizes.json).
+// noise map: two passes at every scale, the thresholded ones whitened by wb_wow_whiten_scale_map.  This is the only
+// place that decides, per scale, between the fused and the two-pass route and when the noise is estimated; wow(),
+// wow_batch() and wow_stream() with whitening call it.  Host code only: it exists because a 512^2 .. 2048^2 frame is
+// finished on the device long before a Python loop has issued its fifteen launches (0.27 - 0.30 ms of interpreter and
+// ctypes time per wow() call, measured; profiles/r2_sizes.json).
 #include "common.cuh"
 
 namespace wb {

@@ -7,7 +7,6 @@ results; torch tensor in -> torch CUDA tensor out.  ``coefficients.data`` always
 from __future__ import annotations
 
 import copy
-import os
 import warnings
 
 import numpy as np
@@ -19,28 +18,6 @@ from .wavelets import (AtrousTransform, Coefficients, _Noise, _frame_layout, abs
                        bilateral_list, broadcast_noise_map, plane_moments, synthesis, to_device_image)
 
 __all__ = ["denoise", "wow", "wow_batch", "wow_stream", "generalized_anscombe", "enhance", "richardson_lucy"]
-
-# Development switch (tests compare the fused one-pass WOW scales against the two-pass route bit for bit).
-FUSED_WOW = True
-# The cascade with whitening in ONE library call (wb_wow_cascade) instead of a Python loop over the scales: the same
-# launches, without the interpreter / ctypes time per launch (tests switch it off to compare the two bit for bit).
-C_CASCADE = os.environ.get("WB_C_CASCADE", "1") != "0"
-# Bilateral WOW, Python loop only: run the memory-bound half of every scale (exact median, whitening K3) on a
-# high-priority side stream while the compute-bound bilateral kernel K2 of the next scale runs on the caller's stream.
-# Measured: 1 % on 4096^2 fp32 frames (K2 is issue-bound: a co-resident kernel is paid in full) against 0.4 ms of host
-# time per frame on small ones -- off by default (WB_OVERLAP_BILATERAL=1 turns it on and bypasses wb_wow_cascade).
-OVERLAP_BILATERAL = os.environ.get("WB_OVERLAP_BILATERAL", "0") != "0"
-_SIDE_STREAMS: dict = {}
-
-
-def _side_stream(device):
-    """One high-priority stream per device for the whitening passes that overlap with K2 (created once)."""
-    key = (device.type, device.index)
-    st = _SIDE_STREAMS.get(key)
-    if st is None:
-        st = _SIDE_STREAMS[key] = torch.cuda.Stream(device, priority=-1)
-    return st
-
 
 _PIPELINE_STREAMS: dict = {}
 
@@ -62,14 +39,6 @@ def generalized_anscombe(signal, alpha=1, g=0, sigma=0, inverse=False):
         return ((alpha * signal / 2) ** 2 + alpha * g - sigma ** 2 - 3 * alpha / 8) / alpha
     dum = alpha * signal + 3 * alpha ** 2 / 8 + sigma ** 2 - alpha * g
     return 2 * torch.sqrt(torch.clamp(dum, min=0)) / alpha
-
-
-class _NullContext:
-    def __enter__(self):
-        return None
-
-    def __exit__(self, *exc):
-        return False
 
 
 def _result(t, as_numpy):
@@ -200,15 +169,15 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
                soft_threshold, noise, buffers=None):
     """The fused WOW pipeline on a stack (B, H, W) of frames.  Returns (recon (B,H,W), planes (B,L+1,H,W), noise).
 
-    ``buffers``: optional dict of preallocated device tensors ("planes", "scratch", "raw_planes", "recon"), filled in
+    ``buffers``: optional dict of preallocated device tensors (planes, scratch, reconstruction, workspace), filled in
     on first use and reused by later calls with the same geometry (``wow_stream`` keeps one per frame in flight, so
     that its steady state allocates nothing large).
 
-    Per plain scale ONE fused launch (wb_wow_scale: smooth, detail, local power, significance, whitening; the raw
-    detail plane never exists in HBM).  Bilateral scales, and scale 0 when the MAD noise must first be estimated from
-    the raw w_0, take two passes: K1/K2 writes c_{s+1} into a ping-pong scratch and the raw w_s into a one-plane
-    scratch, K3 whitens it into the output.  The noise is estimated on the device (no host synchronisation anywhere),
-    the residual plane is rescaled in place and K5 sums the planes."""
+    With whitening and at least one scale, the whole pipeline is ONE library call (wb_wow_cascade, or
+    wb_wow_cascade_map for a per-pixel noise map; csrc/cascade.cu holds its per-scale policy).  Without whitening,
+    K1/K2 write every plane and wb_denoise_plane thresholds and weights it in place, with the MAD noise estimated from
+    plane 0 where a threshold first needs it.  Then the residual plane is rescaled (whitening) or weighted and K5 sums
+    the planes.  The noise is estimated on the device: no host synchronisation anywhere."""
     lib = _lib.load(require_cuda=True)
     sf = scaling_function_class(2)
     b, h, w = stack.shape
@@ -230,11 +199,7 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
     factors = transform.var_factors(L) if bilateral is not None else [None] * L
     if L == 0:
         planes[:, 0].copy_(stack)
-    # (bilateral cascades: in one call unless the side-stream overlap of K3 with K2 is asked for -- it gains 1 % on 4096^2
-    # frames and costs 0.4 ms of host time on small ones)
-    if C_CASCADE and FUSED_WOW and whitening and (bilateral is None or not OVERLAP_BILATERAL) and L >= 1 and \
-            dev.type == "cuda":
-        # one call: wb_wow_cascade issues exactly the launches of the loop below
+    if whitening and L >= 1:
         import ctypes
         scratch3 = buffer("scratch3", (3, b, h, w))
         recon = buffer("recon", (b, h, w))
@@ -267,74 +232,31 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
                                               ws.numel(), _lib.stream_ptr(dev)))
         return recon, planes, nz
     scratch = buffer("scratch", (2, b, h, w)) if L > 1 else None
-    raw_planes = None  # scratch for the raw w_s of the two-pass route, allocated on first use
     nz = noise  # _Noise or None
-    nz_map = None if noise is None else noise.map  # per-pixel noise: two passes at every scale
+    nz_map = None if noise is None else noise.map
     src = stack
-    # Bilateral cascade with whitening: K2 is bound by the MUFU/FMA pipes and leaves HBM idle, the exact median and the
-    # whitening pass K3 are bound by HBM.  They go to a high-priority side stream: K3 of scale s then runs under K2 of
-    # scale s+1 (its blocks are scheduled as K2 blocks retire).  Three raw planes rotate (with two, K2 of scale 2 had to
-    # wait for the whitening of scale 0, which itself waits for the exact median); events order the hand-over.
-    overlap = OVERLAP_BILATERAL and whitening and bilateral is not None and L > 1 and dev.type == "cuda"
-    main = torch.cuda.current_stream(dev) if overlap else None
-    side = _side_stream(dev) if overlap else None
-    ev_k3 = [None, None, None]  # whitening of the scale that last used raw_planes[i]
     for s in range(L):
         dst_c = planes[:, L] if s == L - 1 else scratch[s & 1]
         d, wt = dns[s], wts[s]
         need_sig = d != 0
         mode = (1 if soft_threshold else 2) if need_sig else 0
-        if whitening:
-            if need_sig and nz is None and s > 0:
-                # lazily, from the current state of plane 0 (already whitened here) -- watroo/wavelets.py:131-132
-                if overlap:
-                    main.wait_stream(side)
-                nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
-            # One pass (K1+K3 fused, raw w_s stays on chip) unless the scale is bilateral, the MAD noise has to be
-            # estimated from the raw w_0 first (grid-wide dependency), or the shape is outside the fused kernel.
-            fused = FUSED_WOW and factors[s] is None and not (need_sig and nz is None) and nz_map is None and \
-                _wow_scale_fused(lib, src, dst_c, planes[:, s], s, sf, mode, d, sigma_e[s] if need_sig else 1.0,
-                                 nz if need_sig else _Noise(), wt)
-            if not fused:
-                if raw_planes is None:
-                    raw_planes = buffer("raw_planes", (3 if overlap else 1, b, h, w))
-                raw_plane = raw_planes[s % 3] if overlap else raw_planes[0]
-                if overlap and ev_k3[s % 3] is not None:
-                    main.wait_event(ev_k3[s % 3])  # the whitening that read this raw plane three scales ago is done
-                atrous_scale(src, s, sf, out_c=dst_c, out_w=raw_plane, var_factor=factors[s])
-                if overlap:
-                    side.wait_stream(main)
-                with torch.cuda.stream(side) if overlap else _NullContext():
-                    if need_sig and nz is None:
-                        nz = _Noise(dev=abs_median_noise(raw_plane, sigma_e[0]))  # s == 0: from the raw w_0
-                    if need_sig and nz_map is not None:
-                        _whiten_scale_map(lib, raw_plane, planes[:, s], nz_map, s, sf, soft_threshold, d, sigma_e[s], wt)
-                    else:
-                        _whiten_scale(lib, raw_plane, planes[:, s], s, sf, mode, d, sigma_e[s] if need_sig else 1.0,
-                                      nz if need_sig else _Noise(), wt)
-                    if overlap:
-                        ev_k3[s % 3] = torch.cuda.Event()
-                        ev_k3[s % 3].record(side)
-        else:
-            atrous_scale(src, s, sf, out_c=dst_c, out_w=planes[:, s], var_factor=factors[s])
-            if need_sig and nz is None:
-                nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
-            if mode or wt != 1:
-                use = nz if need_sig else _Noise()
-                # wb_denoise_plane reads one map plane for every frame: one launch per frame for per-frame maps
-                per_frame = need_sig and nz_map is not None and nz_map.ndim == 3
-                for f0, nf in ([(f, 1) for f in range(b)] if per_frame else [(0, b)]):
-                    m_ptr = 0 if not need_sig or nz_map is None else nz_map[f0].data_ptr() if per_frame else \
-                        nz_map.data_ptr()
-                    with torch.cuda.device(dev):
-                        _lib.check(lib.wb_denoise_plane(planes[f0, s].data_ptr(), h * w, nf, (L + 1) * h * w,
-                                                        _lib.dtype_code(dt), mode, float(d),
-                                                        float(sigma_e[s]) if need_sig else 1.0, use.host, use.dev_ptr,
-                                                        m_ptr, float(wt), _lib.stream_ptr(dev)))
+        atrous_scale(src, s, sf, out_c=dst_c, out_w=planes[:, s], var_factor=factors[s])
+        if need_sig and nz is None:
+            nz = _Noise(dev=abs_median_noise(planes[:, 0], sigma_e[0]))
+        if mode or wt != 1:
+            use = nz if need_sig else _Noise()
+            # wb_denoise_plane reads one map plane for every frame: one launch per frame for per-frame maps
+            per_frame = need_sig and nz_map is not None and nz_map.ndim == 3
+            for f0, nf in ([(f, 1) for f in range(b)] if per_frame else [(0, b)]):
+                m_ptr = 0 if not need_sig or nz_map is None else nz_map[f0].data_ptr() if per_frame else \
+                    nz_map.data_ptr()
+                with torch.cuda.device(dev):
+                    _lib.check(lib.wb_denoise_plane(planes[f0, s].data_ptr(), h * w, nf, (L + 1) * h * w,
+                                                    _lib.dtype_code(dt), mode, float(d),
+                                                    float(sigma_e[s]) if need_sig else 1.0, use.host, use.dev_ptr,
+                                                    m_ptr, float(wt), _lib.stream_ptr(dev)))
         src = dst_c
-    if overlap:
-        main.wait_stream(side)  # every whitened plane is complete before the tail (and before any buffer is freed)
-    # residual plane: c_L *= wt_L / std(c_L)  (watroo/utils.py:185-189, :203)
+    # residual plane: c_L *= wt_L / std(c_L)  (watroo/utils.py:185-189, :203); with whitening only for L == 0 here
     last = planes[:, L]
     if whitening:
         # (a fused rescale + synthesis pass measured slower: the separate rescale finds c_L still in L2)
