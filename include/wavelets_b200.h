@@ -368,6 +368,37 @@ int wb_wow_cascade_map(const void *in, long long in_pitch, long long in_bstride,
                        size_t workspace_bytes, void *stream);
 
 /*
+ * wb_wow_cascade with the gamma blend (h > 0, watroo/utils.py:157-158, :207-217) and / or preserve_variance
+ * (:178-184): the whole image branch of `wow` for those options in one call.  Every scale takes two passes: K1 / K2
+ * write the raw detail plane into scratch, [wb_plane_moments of it when preserve_variance,] K3 whitens it into the
+ * plane when `whitening` (map mode where sigmas[s] != 0 and a map is used), and a K5 epilogue then
+ *   - forms dn = dtype(double(w) * significance) (w itself for unthresholded scales and a zero host-scalar noise),
+ *   - adds dn to the gamma plane (h > 0),
+ *   - scales the whitened plane by pn = dtype(sqrt(mean(w^2))) (whitening and preserve_variance), or writes
+ *     dtype(dn * factor), factor = dtype(pn * dtype(weight)) or dtype(weight) (no whitening).
+ * The residual plane is added to the gamma plane, then c_L <- c_L * dtype(weight_L [* std] [/ max(std, 1e-15)]) in
+ * float64 with std rounded to the dtype; recon = the sum of the planes, or with h > 0
+ *   dtype(dtype(1 - h) * sum + dtype(h) * clamp((gamma - lo) / (hi - lo), 0, 1) ** (1 / gamma))
+ * with lo / hi the per-frame min / max of the gamma plane or the given gamma_min / gamma_max, every operation rounded
+ * to the dtype as the element-wise route of `wow` rounds it.
+ *   whitening: the caller passes `whitening and h < 1` (utils.py:186, :193).
+ *   gamma_plane: (batch, H, W) scratch, required when h > 0 (then gamma != 0); not read otherwise.
+ *   n_scales may be 0 (h >= 1 without denoise coefficients): plane 0 is then the image.  scratch may be NULL then.
+ *   Noise: host scalar / noise_dev / estimate as in wb_wow_cascade; use_map != 0 takes the per-pixel noise_map instead
+ *   (layout of wb_wow_whiten_scale_map; estimate_noise must then be 0).
+ *   workspace: wb_wow_cascade_blend_workspace_bytes(dtype, batch, H*W) bytes of device memory.
+ * The other arguments as in wb_wow_cascade.
+ */
+size_t wb_wow_cascade_blend_workspace_bytes(int dtype, int batch, long long n);
+int wb_wow_cascade_blend(const void *in, long long in_pitch, long long in_bstride, void *planes, void *scratch,
+                         void *recon, void *gamma_plane, int batch, int H, int W, int n_scales, int taps, int dtype,
+                         const double *weights, const double *sigmas, const double *sigma_e, const double *var_factors,
+                         int soft, double noise_host, double *noise_dev, int estimate_noise, int use_map,
+                         const void *noise_map, long long map_pitch, long long map_bstride, int whitening,
+                         int preserve_variance, double h, double gamma, double gamma_min, int gamma_min_given,
+                         double gamma_max, int gamma_max_given, void *workspace, size_t workspace_bytes, void *stream);
+
+/*
  * n standard-normal float32 samples (Philox4x32-10 + Box-Muller), the device stand-in for
  * np.random.normal(...).astype(np.float32) of compute_noise_weights (watroo/wavelets.py:225).
  * `offset` advances the counter so that successive calls with one seed give independent fields.

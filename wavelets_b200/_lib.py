@@ -80,6 +80,12 @@ SIGNATURES = {
     "wb_wow_cascade_map": (_c_int, [_c_vp, _c_ll, _c_ll, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int,
                                     _c_int, ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl),
                                     ctypes.POINTER(_c_dbl), _c_int, _c_vp, _c_ll, _c_ll, _c_vp, _c_sz, _c_vp]),
+    "wb_wow_cascade_blend_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_ll]),
+    "wb_wow_cascade_blend": (_c_int, [_c_vp, _c_ll, _c_ll, _c_vp, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int,
+                                      _c_int, _c_int, ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl),
+                                      ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), _c_int, _c_dbl, _c_vp, _c_int,
+                                      _c_int, _c_vp, _c_ll, _c_ll, _c_int, _c_int, _c_dbl, _c_dbl, _c_dbl, _c_int, _c_dbl,
+                                      _c_int, _c_vp, _c_sz, _c_vp]),
     "wb_filter2d": (_c_int, [_c_vp, _c_vp, _c_int, _c_int, _c_ll, _c_ll, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_vp]),
     "wb_atrous_axis": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_ll, _c_ll, _c_ll, _c_int, _c_int, _c_int, _c_int, _c_vp]),
 }

@@ -335,4 +335,17 @@ inline int launch_pdl_v(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t sm
     return (int)cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
+// Gamma-blend / preserve_variance passes of wb_wow_cascade_blend (kernels in csrc/pointwise.cu).
+int blend_scale(const void *raw, void *plane, long long plane_bs, void *gamma, long long n, int W, int batch, int dtype,
+                int first, int write_mode, int sig_mode, double sigma, double sigma_e, double noise_host,
+                const double *noise_dev, const void *noise_map, long long map_pitch, long long map_bstride,
+                const double *moments, double weight, cudaStream_t st);
+int blend_residual(void *c, long long n, int batch, long long bstride, void *gamma, int first, int dtype,
+                   const double *moments, double weight, int preserve_variance, int whitening, unsigned long long *minmax,
+                   cudaStream_t st);
+int synthesis_blend(const void *planes, int nplanes, long long plane_stride, long long n, int batch,
+                    long long in_bstride, const void *gamma_plane, void *out, int dtype, const unsigned long long *minmax,
+                    double h, double gamma, double gamma_min, int min_given, double gamma_max, int max_given,
+                    cudaStream_t st);
+
 }  // namespace wb

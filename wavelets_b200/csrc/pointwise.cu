@@ -3,6 +3,7 @@
 //   * in-place denoise of a plane Coefficients.denoise           watroo/wavelets.py:145-149
 //   * residual-plane rescale      wow(), last plane              watroo/utils.py:185-189,203
 //   * synthesis sum               np.sum(coefficients, axis=0)   watroo/utils.py:98,205
+//   * gamma blend / preserve_variance epilogues of wow()         watroo/utils.py:157-158,174-217
 //   * N(0,1) fp32 noise fields    np.random.normal               watroo/wavelets.py:225 (device Philox4x32-10)
 #include "common.cuh"
 
@@ -121,6 +122,223 @@ __global__ void __launch_bounds__(256) synthesis_kernel(const T *planes, int npl
             for (int k = 1; k < nplanes; ++k) acc += pf[(long long)k * plane_stride + i];
             of[i] = acc;
         }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Gamma blend (h > 0) and preserve_variance of wow() (watroo/utils.py:157-158, :174-217) as three passes of the
+// cascade call: a per-scale epilogue, the residual plane, and the synthesis with the blend.  Each reproduces the
+// torch element-wise ops of the plane-by-plane route one by one: every op rounds to the plane dtype on its own, so the
+// explicit _rn intrinsics keep nvcc from contracting a multiply and an add into an FMA.
+// ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float sub_rn(float a, float b) { return __fsub_rn(a, b); }
+__device__ __forceinline__ double sub_rn(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ float div_rn(float a, float b) { return __fdiv_rn(a, b); }
+__device__ __forceinline__ double div_rn(double a, double b) { return __ddiv_rn(a, b); }
+__device__ __forceinline__ float sqrt_rn(float a) { return __fsqrt_rn(a); }
+__device__ __forceinline__ double sqrt_rn(double a) { return __dsqrt_rn(a); }
+
+__device__ __forceinline__ float rsqrt_t(float a) { return rsqrtf(a); }
+__device__ __forceinline__ double rsqrt_t(double a) { return rsqrt(a); }
+__device__ __forceinline__ float pow_t(float a, float e) { return powf(a, e); }
+__device__ __forceinline__ double pow_t(double a, double e) { return pow(a, e); }
+
+// Total order of the bit patterns (-0 < +0), as unsigned keys for atomicMin / atomicMax.
+__device__ __forceinline__ unsigned long long order_key(float x) {
+    const uint32_t u = __float_as_uint(x);
+    return (u & 0x80000000u) ? (unsigned long long)(~u) : (unsigned long long)(u | 0x80000000u);
+}
+__device__ __forceinline__ unsigned long long order_key(double x) {
+    const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+    return (u & 0x8000000000000000ull) ? ~u : (u | 0x8000000000000000ull);
+}
+__device__ __forceinline__ unsigned long long bits_of(float x) { return (unsigned long long)__float_as_uint(x); }
+__device__ __forceinline__ unsigned long long bits_of(double x) { return (unsigned long long)__double_as_longlong(x); }
+template <typename T> __device__ __forceinline__ T from_bits(unsigned long long b);
+template <> __device__ __forceinline__ float from_bits<float>(unsigned long long b) { return __uint_as_float((uint32_t)b); }
+template <> __device__ __forceinline__ double from_bits<double>(unsigned long long b) { return __longlong_as_double((long long)b); }
+template <typename T> __device__ __forceinline__ T from_order_key(unsigned long long k);
+template <> __device__ __forceinline__ float from_order_key<float>(unsigned long long k) {
+    const uint32_t u = (uint32_t)k;
+    return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+template <> __device__ __forceinline__ double from_order_key<double>(unsigned long long k) {
+    return __longlong_as_double((long long)((k & 0x8000000000000000ull) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
+// Per-scale epilogue, reading the raw w_s (frame stride n) that K1 / K2 left in scratch:
+//   dn     = T(double(w) * significance)  where the plane-by-plane route launched wb_denoise_plane (sig_mode != 0;
+//            the same expression as denoise_plane_kernel with weight 1), else w itself
+//   gamma <- T(gamma + dn)                 (accumulate; `first`: T(+0 + dn), since zeros_like + (-0.0) is +0.0)
+//   write_mode 1: plane <- T(plane * pn)   (whitening and preserve_variance: K3's output times the power norm)
+//   write_mode 2: plane <- T(dn * factor)  (no whitening: factor = T(pn * T(weight)) or T(weight); dn itself when
+//                                           neither preserve_variance nor a weight != 1 asks for the product)
+// pn = T(sqrt(var + mean * mean)) of the raw plane from wb_plane_moments (`moments`, NULL without preserve_variance).
+template <typename T>
+__global__ void __launch_bounds__(256) blend_scale_kernel(const T *raw, T *plane, long long plane_bs, T *gamma,
+                                                          long long n, int W, int first, int accumulate, int write_mode,
+                                                          int sig_mode, double sigma, double sigma_e, double noise_host,
+                                                          const double *noise_dev, const T *noise_map,
+                                                          long long map_pitch, long long map_bstride,
+                                                          const double *moments, double weight, double unit) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int frame = blockIdx.y;
+    const T *rf = raw + (long long)frame * n;
+    T *pf = plane + (long long)frame * plane_bs;
+    T *gf = accumulate ? gamma + (long long)frame * n : nullptr;
+    const T *mf = noise_map ? noise_map + (long long)frame * map_bstride : nullptr;
+    int mode = sig_mode;
+    const double nz = noise_dev ? noise_dev[frame] : noise_host;
+    if (mode && !noise_map && nz == 0.0) mode = 0;
+    T pn = T(0);
+    if (moments) {
+        const double mean = moments[frame * 3 + 0], var = moments[frame * 3 + 1];
+        pn = (T)__dsqrt_rn(__dadd_rn(var, __dmul_rn(mean, mean)));
+    }
+    const bool scale_dn = moments != nullptr || weight != 1.0;
+    const T factor = moments ? mul_rn(pn, (T)weight) : (T)weight;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const T w = rf[i];
+        T dn = w;
+        if (sig_mode) {
+            const double v = (double)w;
+            double f = unit;
+            if (mode) {
+                const T *m = mf ? mf + (map_pitch == W ? i : (i / W) * map_pitch + i % W) : nullptr;
+                const double thr = threshold_at<T>(m, 0, sigma, nz, sigma_e);
+                if (mode == 1) f = unit * erf(fabs(v / thr));
+                else f = unit * (fabs(v) > thr ? 1.0 : 0.0);
+            }
+            dn = (T)(v * f);
+        }
+        if (gf) gf[i] = add_rn(first ? T(0) : gf[i], dn);
+        if (write_mode == 1) pf[i] = mul_rn(pf[i], pn);
+        else if (write_mode == 2) pf[i] = scale_dn ? mul_rn(dn, factor) : dn;
+    }
+}
+
+// Residual plane (as _wow_general treats it): gamma <- T(gamma + c_L) with the raw c_L (T(+0 + c_L) when `first`:
+// no scale), then c_L <- T(c_L * T(factor)), factor = double(weight) [* double(T(std)) with preserve_variance]
+// [/ max(double(T(std)), 1e-15) with whitening] in float64.  With `gamma`, also the exact per-frame min and max of the
+// final gamma plane: minmax[frame] = {max of the inverted keys (the min), max of the keys, the largest NaN bit pattern
+// seen}, zeroed by the caller.  A NaN anywhere makes both bounds that NaN, as torch.min / torch.max return a NaN
+// element.
+template <typename T>
+__global__ void __launch_bounds__(256) blend_residual_kernel(T *c, long long n, long long bstride, T *gamma,
+                                                             int first, const double *moments, double weight,
+                                                             int preserve_variance, int whitening,
+                                                             unsigned long long *minmax) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int frame = blockIdx.y;
+    T *cf = c + (long long)frame * bstride;
+    T *gf = gamma ? gamma + (long long)frame * n : nullptr;
+    double f = weight;
+    if (preserve_variance || whitening) {
+        double sd = (double)(T)moments[frame * 3 + 2];
+        if (preserve_variance) f = __dmul_rn(f, sd);
+        if (whitening) f = __ddiv_rn(f, sd <= 0.0 ? 1e-15 : sd);
+    }
+    const T tf = (T)f;
+    unsigned long long kmin_inv = 0, kmax = 0, nan = 0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const T v = cf[i];
+        if (gf) {
+            const T g = add_rn(first ? T(0) : gf[i], v);
+            gf[i] = g;
+            if (g != g) {
+                nan = max(nan, bits_of(g));
+            } else {
+                const unsigned long long k = order_key(g);
+                kmin_inv = max(kmin_inv, ~k);
+                kmax = max(kmax, k);
+            }
+        }
+        cf[i] = mul_rn(v, tf);
+    }
+    if (!gf) return;
+    for (int o = 16; o > 0; o >>= 1) {
+        kmin_inv = max(kmin_inv, __shfl_down_sync(0xffffffffu, kmin_inv, o));
+        kmax = max(kmax, __shfl_down_sync(0xffffffffu, kmax, o));
+        nan = max(nan, __shfl_down_sync(0xffffffffu, nan, o));
+    }
+    __shared__ unsigned long long r[3][8];
+    if ((threadIdx.x & 31) == 0) {
+        r[0][threadIdx.x >> 5] = kmin_inv;
+        r[1][threadIdx.x >> 5] = kmax;
+        r[2][threadIdx.x >> 5] = nan;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int k = 1; k < (int)(blockDim.x >> 5); ++k) {
+            kmin_inv = max(kmin_inv, r[0][k]);
+            kmax = max(kmax, r[1][k]);
+            nan = max(nan, r[2][k]);
+        }
+        unsigned long long *mm = minmax + frame * 3;
+        atomicMax(mm + 0, kmin_inv);
+        atomicMax(mm + 1, kmax);
+        if (nan) atomicMax(mm + 2, nan);
+    }
+}
+
+// gamma_scaled.pow_(1 / gamma) as torch dispatches it: exponent 0 fills ones, 1 copies, 0.5 / -0.5 / -1 take sqrt /
+// rsqrt / reciprocal; with the exponent rounded to the dtype, 2 / 3 / -2 take products, anything else pow().
+enum { POW_FILL = 0, POW_COPY, POW_SQRT, POW_RSQRT, POW_RECIP, POW_SQUARE, POW_CUBE, POW_INV_SQUARE, POW_GENERAL };
+template <typename T>
+__device__ __forceinline__ T pow_like_torch(T b, int mode, T e) {
+    switch (mode) {
+        case POW_FILL: return T(1);
+        case POW_COPY: return b;
+        case POW_SQRT: return sqrt_rn(b);
+        case POW_RSQRT: return rsqrt_t(b);
+        case POW_RECIP: return div_rn(T(1), b);
+        case POW_SQUARE: return mul_rn(b, b);
+        case POW_CUBE: return mul_rn(mul_rn(b, b), b);
+        case POW_INV_SQUARE: return (T)__ddiv_rn(1.0, (double)mul_rn(b, b));
+        default: return pow_t(b, e);
+    }
+}
+
+// Scalars of the blend, in the plane dtype as torch forms them: lo / hi are the given bounds (rounded to T) or the
+// per-frame min / max; with both given the division is a multiplication by inv = T(1) / T(hi - lo) (a host-scalar
+// divisor), otherwise a true division by T(hi - lo); c1 = T(1 - h), c2 = T(h).
+template <typename T> struct BlendScalars {
+    T lo, hi, inv, c1, c2, e;
+    int lo_given, hi_given, pow_mode;
+};
+
+// recon = T(T(c1 * sum) + T(c2 * g'')) with sum the plane-order sum of synthesis_kernel and
+// g'' = pow(clamp(T(T(gamma - lo) / T(hi - lo)), 0, 1), 1 / gamma); the clamp keeps NaN.
+template <typename T>
+__global__ void __launch_bounds__(256) synthesis_blend_kernel(const T *planes, int nplanes, long long plane_stride,
+                                                              long long n, long long in_bstride, const T *gamma, T *out,
+                                                              const unsigned long long *minmax, BlendScalars<T> p) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int frame = blockIdx.y;
+    const T *pf = planes + (long long)frame * in_bstride;
+    const T *gf = gamma + (long long)frame * n;
+    T *of = out + (long long)frame * n;
+    const unsigned long long *mm = minmax + frame * 3;
+    const bool nan = mm[2] != 0;
+    const T lo = p.lo_given ? p.lo : nan ? from_bits<T>(mm[2]) : from_order_key<T>(~mm[0]);
+    const T hi = p.hi_given ? p.hi : nan ? from_bits<T>(mm[2]) : from_order_key<T>(mm[1]);
+    const bool by_inverse = p.lo_given && p.hi_given;
+    const T range = sub_rn(hi, lo);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        T acc = pf[i];
+        for (int k = 1; k < nplanes; ++k) acc = add_rn(acc, pf[(long long)k * plane_stride + i]);
+        T g = sub_rn(gf[i], lo);
+        g = by_inverse ? mul_rn(g, p.inv) : div_rn(g, range);
+        if (!(g != g)) g = g < T(0) ? T(0) : (g > T(1) ? T(1) : g);
+        g = pow_like_torch<T>(g, p.pow_mode, p.e);
+        of[i] = add_rn(mul_rn(p.c1, acc), mul_rn(p.c2, g));
     }
 }
 
@@ -314,6 +532,72 @@ __global__ void __launch_bounds__(256) filter2d_kernel(const T *in, T *out, int 
         }
         out[(long long)y * out_pitch + x] = (T)acc;
     }
+}
+
+// Launchers of the blend kernels for wb_wow_cascade_blend (csrc/cascade.cu), which has validated the arguments.
+int blend_scale(const void *raw, void *plane, long long plane_bs, void *gamma, long long n, int W, int batch, int dtype,
+                int first, int write_mode, int sig_mode, double sigma, double sigma_e, double noise_host,
+                const double *noise_dev, const void *noise_map, long long map_pitch, long long map_bstride,
+                const double *moments, double weight, cudaStream_t st) {
+    dim3 grid(grid_for(n), (unsigned)batch);
+    const int acc = gamma != nullptr;
+    if (dtype == WB_F32)
+        return launch_pdl_v(blend_scale_kernel<float>, grid, dim3(256), 0, st, reinterpret_cast<const float *>(raw),
+                            reinterpret_cast<float *>(plane), plane_bs, reinterpret_cast<float *>(gamma), n, W, first, acc,
+                            write_mode, sig_mode, sigma, sigma_e, noise_host, noise_dev,
+                            reinterpret_cast<const float *>(noise_map), map_pitch, map_bstride, moments, weight, 1.0);
+    return launch_pdl_v(blend_scale_kernel<double>, grid, dim3(256), 0, st, reinterpret_cast<const double *>(raw),
+                        reinterpret_cast<double *>(plane), plane_bs, reinterpret_cast<double *>(gamma), n, W, first, acc,
+                        write_mode, sig_mode, sigma, sigma_e, noise_host, noise_dev,
+                        reinterpret_cast<const double *>(noise_map), map_pitch, map_bstride, moments, weight, 1.0);
+}
+
+int blend_residual(void *c, long long n, int batch, long long bstride, void *gamma, int first, int dtype,
+                   const double *moments, double weight, int preserve_variance, int whitening, unsigned long long *minmax,
+                   cudaStream_t st) {
+    dim3 grid(grid_for(n), (unsigned)batch);
+    if (dtype == WB_F32)
+        return launch_pdl_v(blend_residual_kernel<float>, grid, dim3(256), 0, st, reinterpret_cast<float *>(c), n, bstride,
+                            reinterpret_cast<float *>(gamma), first, moments, weight, preserve_variance, whitening,
+                            minmax);
+    return launch_pdl_v(blend_residual_kernel<double>, grid, dim3(256), 0, st, reinterpret_cast<double *>(c), n, bstride,
+                        reinterpret_cast<double *>(gamma), first, moments, weight, preserve_variance, whitening,
+                        minmax);
+}
+
+template <typename T>
+static BlendScalars<T> blend_scalars(double h, double gamma, double gamma_min, int min_given, double gamma_max,
+                                     int max_given) {
+    BlendScalars<T> p;
+    p.lo = (T)gamma_min;
+    p.hi = (T)gamma_max;
+    p.lo_given = min_given;
+    p.hi_given = max_given;
+    p.inv = (min_given && max_given) ? T(1) / (T)(gamma_max - gamma_min) : T(0);
+    p.c1 = (T)(1.0 - h);
+    p.c2 = (T)h;
+    const double e = 1.0 / gamma;
+    p.e = (T)e;
+    p.pow_mode = e == 0.0 ? POW_FILL : e == 1.0 ? POW_COPY : e == 0.5 ? POW_SQRT : e == -0.5 ? POW_RSQRT
+               : e == -1.0 ? POW_RECIP : p.e == T(2) ? POW_SQUARE : p.e == T(3) ? POW_CUBE
+               : p.e == T(-2) ? POW_INV_SQUARE : POW_GENERAL;
+    return p;
+}
+
+int synthesis_blend(const void *planes, int nplanes, long long plane_stride, long long n, int batch,
+                    long long in_bstride, const void *gamma, void *out, int dtype, const unsigned long long *minmax,
+                    double h, double gamma_exp_base, double gamma_min, int min_given, double gamma_max, int max_given,
+                    cudaStream_t st) {
+    dim3 grid(grid_for(n), (unsigned)batch);
+    if (dtype == WB_F32)
+        return launch_pdl_v(synthesis_blend_kernel<float>, grid, dim3(256), 0, st, reinterpret_cast<const float *>(planes),
+                            nplanes, plane_stride, n, in_bstride, reinterpret_cast<const float *>(gamma),
+                            reinterpret_cast<float *>(out), minmax,
+                            blend_scalars<float>(h, gamma_exp_base, gamma_min, min_given, gamma_max, max_given));
+    return launch_pdl_v(synthesis_blend_kernel<double>, grid, dim3(256), 0, st, reinterpret_cast<const double *>(planes),
+                        nplanes, plane_stride, n, in_bstride, reinterpret_cast<const double *>(gamma),
+                        reinterpret_cast<double *>(out), minmax,
+                        blend_scalars<double>(h, gamma_exp_base, gamma_min, min_given, gamma_max, max_given));
 }
 
 }  // namespace wb

@@ -165,8 +165,19 @@ def _stack_noise(noise, b, h, w, dtype, device):
     raise ValueError(f"noise of shape {shape} for {b} frames of {h} x {w}: expected {_STACK_NOISE_FORMS}")
 
 
+def _blend_options(preserve_variance, gamma, gamma_min, gamma_max, h):
+    """The gamma blend (h > 0) and preserve_variance options of wow() for _wow_stack, or None when neither is asked for.
+    ``1 / gamma`` is evaluated here when the blend needs it, so that gamma == 0 raises ZeroDivisionError as the
+    reference's ``pow(1 / gamma)`` does."""
+    if h == 0 and not preserve_variance:
+        return None
+    if h > 0:
+        1 / gamma  # noqa: B018
+    return bool(preserve_variance), float(gamma), gamma_min, gamma_max, float(h)
+
+
 def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilateral, bilateral_scaling, whitening,
-               soft_threshold, noise, buffers=None):
+               soft_threshold, noise, buffers=None, blend=None):
     """The fused WOW pipeline on a stack (B, H, W) of frames.  Returns (recon (B,H,W), planes (B,L+1,H,W), noise).
 
     ``buffers``: optional dict of preallocated device tensors (planes, scratch, reconstruction, workspace), filled in
@@ -174,10 +185,12 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
     that its steady state allocates nothing large).
 
     With whitening and at least one scale, the whole pipeline is ONE library call (wb_wow_cascade, or
-    wb_wow_cascade_map for a per-pixel noise map; csrc/cascade.cu holds its per-scale policy).  Without whitening,
-    K1/K2 write every plane and wb_denoise_plane thresholds and weights it in place, with the MAD noise estimated from
-    plane 0 where a threshold first needs it.  Then the residual plane is rescaled (whitening) or weighted and K5 sums
-    the planes.  The noise is estimated on the device: no host synchronisation anywhere."""
+    wb_wow_cascade_map for a per-pixel noise map; csrc/cascade.cu holds its per-scale policy).  ``blend`` (from
+    _blend_options: preserve_variance, gamma, gamma_min, gamma_max, h) takes wb_wow_cascade_blend, one call for every
+    noise form, with or without whitening and for any scale count.  Without whitening and blend, K1/K2 write every
+    plane and wb_denoise_plane thresholds and weights it in place, with the MAD noise estimated from plane 0 where a
+    threshold first needs it.  Then the residual plane is rescaled (whitening) or weighted and K5 sums the planes.
+    The noise is estimated on the device: no host synchronisation anywhere."""
     lib = _lib.load(require_cuda=True)
     sf = scaling_function_class(2)
     b, h, w = stack.shape
@@ -197,14 +210,13 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
     sigma_e = sf.sigma_e(bilateral=bilateral)
     transform = AtrousTransform(scaling_function_class, bilateral=bilateral, bilateral_scaling=bilateral_scaling)
     factors = transform.var_factors(L) if bilateral is not None else [None] * L
-    if L == 0:
-        planes[:, 0].copy_(stack)
-    if whitening and L >= 1:
+    if blend is not None or (whitening and L >= 1):
         import ctypes
-        scratch3 = buffer("scratch3", (3, b, h, w))
+        scratch3 = buffer("scratch3", (3, b, h, w)) if L >= 1 else None
         recon = buffer("recon", (b, h, w))
         code = _lib.dtype_code(dt)
-        ws_bytes = lib.wb_wow_cascade_workspace_bytes(code, b, h * w)
+        ws_bytes = (lib.wb_wow_cascade_workspace_bytes if blend is None else
+                    lib.wb_wow_cascade_blend_workspace_bytes)(code, b, h * w)
         ws = buffers.get("cascade_ws")
         if ws is None or ws.numel() < ws_bytes or ws.device != dev:
             ws = buffers["cascade_ws"] = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
@@ -217,20 +229,35 @@ def _wow_stack(stack, scaling_function_class, n_scales, wts, dns, sigma_bilatera
         use = nz if nz is not None else _Noise()
         arr = ctypes.c_double * (L + 1)
         _, _, _, pitch, bstride = _frame_layout(stack)
-        args = (stack.data_ptr(), pitch, bstride, planes.data_ptr(), scratch3.data_ptr(), recon.data_ptr(), b, h, w, L,
-                sf.taps_code, code, arr(*[float(x) for x in wts[:L + 1]]),
+        head = (stack.data_ptr(), pitch, bstride, planes.data_ptr(), None if scratch3 is None else scratch3.data_ptr(),
+                recon.data_ptr())
+        tail = (b, h, w, L, sf.taps_code, code, arr(*[float(x) for x in wts[:L + 1]]),
                 arr(*([float(x) for x in dns[:L]] + [0.0])), arr(*([float(x) for x in sigma_e[:L]] + [0.0])),
                 None if bilateral is None else arr(*([float(x) for x in factors[:L]] + [0.0])),
                 1 if soft_threshold else 0)
+        m_pitch = m_bstride = 0
+        if nz_map is not None:
+            _, _, _, m_pitch, m_bstride = _frame_layout(nz_map)
         with torch.cuda.device(dev):
-            if nz_map is not None:
-                _, _, _, m_pitch, m_bstride = _frame_layout(nz_map)
-                _lib.check(lib.wb_wow_cascade_map(*args, nz_map.data_ptr(), m_pitch, m_bstride, ws.data_ptr(),
+            if blend is not None:
+                pv, gamma, gamma_min, gamma_max, hh = blend
+                g = buffer("gamma", (b, h, w)) if hh > 0 else None
+                _lib.check(lib.wb_wow_cascade_blend(
+                    *head, None if g is None else g.data_ptr(), *tail, float(use.host), use.dev_ptr,
+                    1 if estimate else 0, 0 if nz_map is None else 1, None if nz_map is None else nz_map.data_ptr(),
+                    m_pitch, m_bstride, 1 if whitening and hh < 1 else 0, 1 if pv else 0, hh, gamma,
+                    0.0 if gamma_min is None else float(gamma_min), 0 if gamma_min is None else 1,
+                    0.0 if gamma_max is None else float(gamma_max), 0 if gamma_max is None else 1, ws.data_ptr(),
+                    ws.numel(), _lib.stream_ptr(dev)))
+            elif nz_map is not None:
+                _lib.check(lib.wb_wow_cascade_map(*head, *tail, nz_map.data_ptr(), m_pitch, m_bstride, ws.data_ptr(),
                                                   ws.numel(), _lib.stream_ptr(dev)))
             else:
-                _lib.check(lib.wb_wow_cascade(*args, float(use.host), use.dev_ptr, 1 if estimate else 0, ws.data_ptr(),
-                                              ws.numel(), _lib.stream_ptr(dev)))
+                _lib.check(lib.wb_wow_cascade(*head, *tail, float(use.host), use.dev_ptr, 1 if estimate else 0,
+                                              ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev)))
         return recon, planes, nz
+    if L == 0:
+        planes[:, 0].copy_(stack)
     scratch = buffer("scratch", (2, b, h, w)) if L > 1 else None
     nz = noise  # _Noise or None
     nz_map = None if noise is None else noise.map
@@ -276,9 +303,10 @@ def wow(data, scaling_function=B3spline, n_scales=None, weights=[], whitening=Tr
     """Wavelets Optimized Whitening (watroo/utils.py:105-219): ``(recon, coefficients)``.
 
     ``data`` is a 2-D image (ndarray or torch tensor) or a ``Coefficients`` object (which is then whitened in
-    place, as in the reference).  The default call and the ``bilateral`` / ``denoise_coefficients`` / ``weights`` /
-    ``whitening`` options run on the fused kernels; ``h > 0`` (gamma blending, utils.py:157-158, :207-217) and
-    ``preserve_variance`` (utils.py:178-184) take a plane-by-plane route over the same kernels."""
+    place, as in the reference).  For an image every option runs as one library call: the ``bilateral`` /
+    ``denoise_coefficients`` / ``weights`` / ``whitening`` / ``noise`` options on the fused kernels, and ``h > 0`` (gamma
+    blending, utils.py:157-158, :207-217) and ``preserve_variance`` (utils.py:178-184) on wb_wow_cascade_blend.
+    ``Coefficients`` input with those two options takes a plane-by-plane route over the same kernels."""
     general = h != 0 or preserve_variance
     if isinstance(data, Coefficients):
         if general:
@@ -299,21 +327,19 @@ def wow(data, scaling_function=B3spline, n_scales=None, weights=[], whitening=Tr
         return _result(recon, was_numpy), co
     n_scales, sigma_bilateral, wts, dns = _wow_plan(img.shape, scaling_function, n_scales, weights,
                                                     denoise_coefficients, bilateral, h=h)
-    if general:
-        transform = AtrousTransform(scaling_function, bilateral=sigma_bilateral, bilateral_scaling=bilateral_scaling)
-        co = transform(img, n_scales)
-        co.noise = noise
-        recon, co = _wow_general(co, weights, whitening, denoise_coefficients, bilateral, soft_threshold,
-                                 preserve_variance, gamma, gamma_min, gamma_max, h, plan=(n_scales, wts, dns))
-        return _result(recon, was_numpy), co
+    blend = _blend_options(preserve_variance, gamma, gamma_min, gamma_max, h)
     nz = _scalar_noise(noise, img.device)
     if isinstance(nz, str):
         # a per-pixel noise map, broadcast to the image: two passes at every scale, the map applied inside K3
         nz = _Noise(map_=broadcast_noise_map(noise, img.shape, img.dtype, img.device))
     recon, planes, nz = _wow_stack(img.unsqueeze(0), scaling_function, n_scales, wts, dns, sigma_bilateral,
-                                   bilateral_scaling, whitening, soft_threshold, nz)
+                                   bilateral_scaling, whitening, soft_threshold, nz, blend=blend)
     co = Coefficients(planes[0], scaling_function(2), sigma_bilateral)
-    if nz is not None and nz.map is not None:
+    if blend is not None and noise is not None:
+        # the noise as Coefficients._noise_arg leaves it: an array map that a threshold used is kept as its device copy
+        used = isinstance(noise, np.ndarray) and noise.ndim > 0 and any(d != 0 for d in dns[:n_scales])
+        co.noise = nz.map if used else noise
+    elif nz is not None and nz.map is not None:
         co.noise = noise
     elif nz is not None:
         co.noise = nz.dev if nz.dev is not None else nz.host
@@ -372,21 +398,26 @@ def _wow_nd(co, wts, dns, whitening, soft_threshold, preserve_variance, gamma, g
 
 
 def wow_batch(frames, scaling_function=B3spline, n_scales=None, weights=[], whitening=True, denoise_coefficients=[],
-              noise=None, bilateral=None, bilateral_scaling=False, soft_threshold=True):
+              noise=None, bilateral=None, bilateral_scaling=False, soft_threshold=True, preserve_variance=False,
+              gamma=3.2, gamma_min=None, gamma_max=None, h=0):
     """NEW entry point (no reference equivalent): WOW of a stack ``(B, H, W)`` of independent frames, every kernel
     launched once for the whole stack.  Returns ``(recon (B,H,W), planes (B,L+1,H,W), noise)`` as device tensors;
     per-frame results are identical to ``wow(frame, noise=<that frame's noise>, ...)``.
 
     ``noise`` (NumPy or torch): None (MAD estimate per frame), a scalar, per-frame scalars ``(B,)``, one per-pixel map
     ``(H, W)`` for every frame or one map per frame ``(B, H, W)``; anything else raises ValueError.  The returned noise
-    is the one used: the (B,) float64 estimates or scalars, the scalar, or the map in the frame dtype."""
+    is the one used: the (B,) float64 estimates or scalars, the scalar, or the map in the frame dtype.
+
+    ``h > 0`` blends every frame with its own gamma-stretched image; ``gamma_min`` / ``gamma_max`` of None take that
+    frame's min / max, as ``wow`` does frame by frame."""
     stack, _ = to_device_image(frames, ndim_ok=(3,))
     n_scales, sigma_bilateral, wts, dns = _wow_plan(stack.shape[1:], scaling_function, n_scales, weights,
-                                                    denoise_coefficients, bilateral)
-    b, h, w = stack.shape
-    nz = _stack_noise(noise, b, h, w, stack.dtype, stack.device)
+                                                    denoise_coefficients, bilateral, h=h)
+    blend = _blend_options(preserve_variance, gamma, gamma_min, gamma_max, h)
+    b, fh, fw = stack.shape
+    nz = _stack_noise(noise, b, fh, fw, stack.dtype, stack.device)
     recon, planes, nz = _wow_stack(stack, scaling_function, n_scales, wts, dns, sigma_bilateral, bilateral_scaling,
-                                   whitening, soft_threshold, nz)
+                                   whitening, soft_threshold, nz, blend=blend)
     if nz is None:
         noise_out = None
     elif nz.map is not None:
@@ -431,17 +462,15 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
     caller = torch.cuda.current_stream(dev)
     for st in (s_in, s_cmp, s_out):
         st.wait_stream(caller)
-    # The options of the fused pipeline are planned ONCE and every frame in flight owns one set of device buffers
-    # (planes, ping-pong scratch, reconstruction): after the first `depth` frames nothing large is allocated -- with
-    # wow() called per frame the caching allocator split and re-grew its blocks while the host ran ahead of the device
-    # (a cudaMalloc of 0.7 GB per frame: 25 ms instead of 1.3).  h > 0 and preserve_variance take wow() itself, frame by
-    # frame.
+    # Every option is planned ONCE and every frame in flight owns one set of device buffers (planes, scratch, gamma
+    # plane, reconstruction): after the first `depth` frames nothing large is allocated -- with wow() called per frame
+    # the caching allocator split and re-grew its blocks while the host ran ahead of the device (a cudaMalloc of 0.7 GB
+    # per frame: 25 ms instead of 1.3).
     opts = dict(kwargs)
     unknown = set(opts) - {"n_scales", "weights", "whitening", "denoise_coefficients", "noise", "bilateral",
                            "bilateral_scaling", "soft_threshold", "preserve_variance", "gamma", "gamma_min", "gamma_max", "h"}
     if unknown:
         raise TypeError(f"wow_stream() got unexpected keyword arguments {sorted(unknown)}")
-    plan = None
     noise = opts.get("noise")
     # per-frame noise: a device vector of scalars (sliced per frame), or the (N, H, W) maps streamed with the frames
     nz_vec = map_host = None
@@ -457,12 +486,13 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
                                 (nz0.map is not None and nz0.map.ndim == 3)):
             nz_vec, nz0 = nz0, None
         s_cmp.wait_stream(caller)  # the noise was uploaded on the caller's stream
-    if opts.get("h", 0) == 0 and not opts.get("preserve_variance", False):
-        n_scales, sigma_bilateral, wts, dns = _wow_plan((h, w), scaling_function, opts.get("n_scales"),
-                                                        opts.get("weights", []), opts.get("denoise_coefficients", []),
-                                                        opts.get("bilateral"), h=0)
-        plan = (n_scales, wts, dns, sigma_bilateral, opts.get("bilateral_scaling", False),
-                opts.get("whitening", True), opts.get("soft_threshold", True))
+    blend_h = opts.get("h", 0)
+    L, sigma_bilateral, wts, dns = _wow_plan((h, w), scaling_function, opts.get("n_scales"), opts.get("weights", []),
+                                             opts.get("denoise_coefficients", []), opts.get("bilateral"), h=blend_h)
+    blend = _blend_options(opts.get("preserve_variance", False), opts.get("gamma", 3.2), opts.get("gamma_min"),
+                           opts.get("gamma_max"), blend_h)
+    bil_scaling, whitening, soft = (opts.get("bilateral_scaling", False), opts.get("whitening", True),
+                                    opts.get("soft_threshold", True))
     d_in = [torch.empty((h, w), dtype=host.dtype, device=dev) for _ in range(depth)]
     d_map = [torch.empty((h, w), dtype=host.dtype, device=dev) for _ in range(depth)] if map_host is not None else None
     d_out = [None] * depth
@@ -489,21 +519,13 @@ def wow_stream(frames, out=None, depth=2, scaling_function=B3spline, **kwargs):
                 nz_i = _Noise(dev=nz_vec.dev[i:i + 1]) if nz_vec.dev is not None else _Noise(map_=nz_vec.map[i])
             else:
                 nz_i = nz0
-            if plan is not None:
-                L, wts, dns, sigma_bilateral, bil_scaling, whitening, soft = plan
-                recon, _, _ = _wow_stack(d_in[b].unsqueeze(0), scaling_function, L, wts, dns, sigma_bilateral,
-                                         bil_scaling, whitening, soft, nz_i, buffers=bufs[b])
-                d_out[b] = recon[0]
-            else:
-                frame_noise = None if nz_i is None else nz_i.map if nz_i.map is not None else \
-                    nz_i.dev if nz_i.dev is not None else nz_i.host
-                d_out[b], _ = wow(d_in[b], scaling_function=scaling_function, **dict(kwargs, noise=frame_noise))
+            recon, _, _ = _wow_stack(d_in[b].unsqueeze(0), scaling_function, L, wts, dns, sigma_bilateral, bil_scaling,
+                                     whitening, soft, nz_i, buffers=bufs[b], blend=blend)
+            d_out[b] = recon[0]
             ev_cmp[b].record(s_cmp)
         with torch.cuda.stream(s_out):
             s_out.wait_event(ev_cmp[b])
             dst[i].copy_(d_out[b], non_blocking=True)
-            if plan is None:
-                d_out[b].record_stream(s_out)
             ev_out[b].record(s_out)
     for st in (s_in, s_cmp, s_out):
         caller.wait_stream(st)
