@@ -399,6 +399,54 @@ int wb_wow_cascade_blend(const void *in, long long in_pitch, long long in_bstrid
                          double gamma_max, int gamma_max_given, void *workspace, size_t workspace_bytes, void *stream);
 
 /*
+ * Volumes: a C-contiguous (D, H, W) array is a volume (watroo/wavelets.py:322), not a stack of frames.  A scale is the 2-D
+ * smooth of every [i] slice (wb_atrous_scale with the D slices as frames) followed by the depth pass with the
+ * half-sample symmetric border (cv2.filter2D with the (K, 1) kernel on every [:, :, i] slice, :55-63, any number of
+ * reflections when D is smaller than the halo).  Bit-identical to wb_atrous_scale + wb_atrous_axis(WB_BORDER_SYMMETRIC).
+ *
+ * wb_atrous_scale_volume: out_c = S_scale[in], out_w = in - out_c (either may be NULL).  tmp: (D, H, W) scratch of the
+ * dtype for the slice smooth.
+ */
+int wb_atrous_scale_volume(const void *in, void *out_c, void *out_w, void *tmp, int D, int H, int W, int scale, int taps,
+                           int dtype, void *stream);
+
+/*
+ * Scratch of wb_atrous_transform_volume / wb_wow_cascade_volume for `levels` scales: one volume for the slice smooth
+ * and, from two scales on, two ping-pong smooth volumes (0 bytes for levels == 0).
+ */
+size_t wb_volume_scratch_bytes(int dtype, int D, int H, int W, int levels);
+
+/*
+ * The plain cascade of a volume over `levels` scales: planes (levels + 1, D, H, W) = [w_0 .. w_{L-1}, c_L]
+ * (AtrousTransform on a 3-D array, watroo/wavelets.py:408-444).  scratch: wb_volume_scratch_bytes bytes.
+ */
+int wb_atrous_transform_volume(const void *in, void *planes, void *scratch, int D, int H, int W, int levels, int taps,
+                               int dtype, void *stream);
+
+/*
+ * wow() of a volume (watroo/utils.py:172-205, h == 0, no preserve_variance) in one call, bit-identical to the element-wise
+ * route (the reference's order and dtypes, every operation rounded once).  Per scale: the transform scale above; then
+ *   whitening != 0: the local power S_s[dtype(w * w)] (slice smooth of the squares + depth pass) and, in the depth pass,
+ *       w <- dtype(double(w) * significance) * dtype(weight / sqrt(P <= 0 ? 1e-15 : P))  (sqrt, divide, multiply);
+ *   whitening == 0: w <- dtype(double(w) * significance) * dtype(weight).
+ * Then the residual plane: c_L * dtype(weight_L / max(std(c_L), 1e-15)) (whitening) or c_L * dtype(weight_L), and
+ * recon (D, H, W) = the sum of the planes.
+ *   planes (n_scales + 1, D, H, W) out; scratch: wb_volume_scratch_bytes(dtype, D, H, W, n_scales) bytes;
+ *   weights[n_scales + 1], sigmas[n_scales], sigma_e[n_scales]: HOST arrays as in wb_wow_cascade; soft: erf or hard mask.
+ *   Noise: estimate_noise != 0 -> the MAD estimate of plane 0 as it stands when a threshold first needs it
+ *   (watroo/wavelets.py:131-132), written to noise_dev[0]; else noise_dev[0] when non-NULL, else noise_host; or a
+ *   per-voxel map of the plane dtype (noise_map != NULL, estimate_noise == 0): element (z, y, x) at
+ *   z * map_zstride + y * W + x, map_zstride 0 (one (H, W) map for every slice) or >= H * W.
+ *   workspace: wb_wow_cascade_volume_workspace_bytes(dtype, D, H, W) bytes of device memory.
+ */
+size_t wb_wow_cascade_volume_workspace_bytes(int dtype, int D, int H, int W);
+int wb_wow_cascade_volume(const void *in, void *planes, void *scratch, void *recon, int D, int H, int W, int n_scales,
+                          int taps, int dtype, const double *weights, const double *sigmas, const double *sigma_e,
+                          int soft, int whitening, double noise_host, double *noise_dev, int estimate_noise,
+                          const void *noise_map, long long map_zstride, void *workspace, size_t workspace_bytes,
+                          void *stream);
+
+/*
  * n standard-normal float32 samples (Philox4x32-10 + Box-Muller), the device stand-in for
  * np.random.normal(...).astype(np.float32) of compute_noise_weights (watroo/wavelets.py:225).
  * `offset` advances the counter so that successive calls with one seed give independent fields.

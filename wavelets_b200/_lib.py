@@ -88,6 +88,14 @@ SIGNATURES = {
                                       _c_int, _c_vp, _c_sz, _c_vp]),
     "wb_filter2d": (_c_int, [_c_vp, _c_vp, _c_int, _c_int, _c_ll, _c_ll, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_vp]),
     "wb_atrous_axis": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_ll, _c_ll, _c_ll, _c_int, _c_int, _c_int, _c_int, _c_vp]),
+    "wb_atrous_scale_volume": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int,
+                                        _c_vp]),
+    "wb_volume_scratch_bytes": (_c_sz, [_c_int, _c_int, _c_int, _c_int, _c_int]),
+    "wb_atrous_transform_volume": (_c_int, [_c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int, _c_vp]),
+    "wb_wow_cascade_volume_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_int, _c_int]),
+    "wb_wow_cascade_volume": (_c_int, [_c_vp, _c_vp, _c_vp, _c_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int,
+                                       ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), ctypes.POINTER(_c_dbl), _c_int,
+                                       _c_int, _c_dbl, _c_vp, _c_int, _c_vp, _c_ll, _c_vp, _c_sz, _c_vp]),
 }
 # development hooks exported by the library but not part of the stable ABI
 _EXTRA = {

@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
         Pack<T, V> cv[NG];
 #pragma unroll
         for (int q = 0; q < NG; ++q) {
-            const Pack<T, V> v = row_pass_b<T, TAPS, DMODE, OP == OP_WHITEN>(row_addr, plan[q]);
+            const Pack<T, V> v = row_pass_b<T, TAPS, DMODE, OP != OP_TRANSFORM>(row_addr, plan[q]);
 #pragma unroll
             for (int e = 0; e < V; ++e) cv[q].v[e] = col_feed<T, TAPS>(S[q][e], v.v[e]);
         }
@@ -171,6 +171,8 @@ __global__ void __launch_bounds__(544) atrous_rows_kernel(const ScaleParams p) {
                         for (int e = 0; e < V; ++e) raw.v[e] -= cv[q].v[e];
                         if (act[q]) st_vec_cs(w_ptr + xg[q], raw);
                     }
+                } else if constexpr (OP == OP_POWER) {
+                    if (act[q]) st_vec(c_ptr + xg[q], cv[q]);
                 } else {
                     const Pack<T, V> raw = lds_vec<T>(crow_addr + xb[q]);
                     Pack<T, V> out;
@@ -483,7 +485,7 @@ __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p
 #pragma unroll
             for (int k = 0; k < TAPS; ++k) {
                 T v = row[xs[k]];
-                if (OP == OP_WHITEN) v = v * v;
+                if (OP != OP_TRANSFORM) v = v * v;
                 ra = (k == 0) ? Taps<T, TAPS>::h(0) * v : fma_t<T>(Taps<T, TAPS>::h(k), v, ra);
             }
             acc = (i == 0) ? Taps<T, TAPS>::h(0) * ra : fma_t<T>(Taps<T, TAPS>::h(i), ra, acc);
@@ -496,6 +498,8 @@ __global__ void __launch_bounds__(256) atrous_generic_kernel(const ScaleParams p
                 push_store(p, dst, out_c + (long long)frame * p.c_bstride + p.row_off_c * p.c_pitch, y, acc);
             }
             if (out_w) out_w[(long long)frame * p.w_bstride + ((long long)y + p.row_off_w) * p.w_pitch + x] = raw - acc;
+        } else if constexpr (OP == OP_POWER) {
+            out_c[(long long)frame * p.c_bstride + (long long)y * p.c_pitch + x] = acc;
         } else {
             T v = epi.apply(raw, acc);
             if constexpr (MAP)
@@ -626,13 +630,14 @@ static int dispatch(ScaleParams &p, int batch, int scale, cudaStream_t st) {
         // fp32 strips 2 - 11 % faster at d >= 4 (kept; d < 4 keeps the generic kernel), float64 K1 equal within 2 % except
         // with paired columns (d >= 16: 1 - 5 us faster, kept), float64 K3 12 - 22 us faster per 4096^2 plane except with
         // the soft threshold (the inlined double-precision erf: 10 us slower, generic kept).
-        if ((sizeof(T) == 8 || p.n_strips > 1) && lean_ok && p.l2_hints &&
+        if (OP != OP_POWER && (sizeof(T) == 8 || p.n_strips > 1) && lean_ok && p.l2_hints &&
             (long long)p.row_stride * (long long)sizeof(T) <= (long long)kLeanStripKiB * 1024 &&
             // (only where the planner laid the segments out for ONE block per SM, which is what 24 KiB slots give)
             2 * ((long long)kLeanSlots * p.row_stride * (long long)sizeof(T) + 16 * kLeanSlots + 1024) > (long long)kMaxSmem) {
             const int cols = p.n_strips == 1 ? p.W : p.wt;
             const bool pair = dmode == 0 && k1_pair_step(p.d, cols, cfg.nt, V);
-            if constexpr (sizeof(T) == 4) {
+            if constexpr (OP == OP_POWER) {
+            } else if constexpr (sizeof(T) == 4) {
                 if (pair) return launch_rows_lean_strip<T, TAPS, 0, OP, 1>(p, batch, cfg.nt, st);
                 if (dmode == 0) return launch_rows_lean_strip<T, TAPS, 0, OP, 0>(p, batch, cfg.nt, st);
             } else if constexpr (OP == OP_TRANSFORM) {
@@ -691,6 +696,22 @@ static int scale_impl(const void *in, void *out_c, void *out_w, int batch, int H
     p.w_pitch = w_pitch; p.w_bstride = w_bstride;
     p.l2_hints = l2_hints_enabled();
     return dispatch_typed<OP_TRANSFORM>(p, batch, scale, taps, dtype, st);
+}
+
+// OP_POWER: out = S_s[T(w * w)] of every frame (the local power of a volume's wow(), smoothed within each slice).
+int atrous_power_slices(const void *w, void *out, int batch, int H, int W, int scale, int taps, int dtype, cudaStream_t st) {
+    int rc = check_common(batch, H, W, taps, dtype);
+    if (rc) return rc;
+    if (scale < 0 || scale > 30) return WB_EINVAL_SCALE;
+    if (!w || !out || w == out) return WB_EINVAL_POINTER;
+    ScaleParams p;
+    memset(&p, 0, sizeof(p));
+    p.in = w; p.out_c = out;
+    p.H = H; p.W = W; p.d = 1 << scale; p.Hg = H;
+    p.in_pitch = W; p.in_bstride = (long long)H * W;
+    p.c_pitch = W; p.c_bstride = (long long)H * W;
+    p.l2_hints = l2_hints_enabled();
+    return dispatch_typed<OP_POWER>(p, batch, scale, taps, dtype, st);
 }
 
 }  // namespace wb

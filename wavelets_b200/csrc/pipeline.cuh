@@ -76,7 +76,8 @@ __device__ __forceinline__ const T *input_row(const ScaleParams &p, long long gy
     return reinterpret_cast<const T *>(p.peer_in[k]) + (gy - p.peer_y0[k]) * p.in_pitch;
 }
 
-enum { OP_TRANSFORM = 0, OP_WHITEN = 1 };
+// OP_POWER: the row pipeline filters the squares of the staged rows (rounded, as T(w * w)) and writes only out_c.
+enum { OP_TRANSFORM = 0, OP_WHITEN = 1, OP_POWER = 2 };
 enum { SIG_MAP = 3 };  // ScaleParams::sig_mode of the noise-map whitening (wb_wow_whiten_scale_map)
 
 // Per-thread, per-column-group tap plan, computed ONCE per thread block: the shared-memory element offset of the

@@ -7,6 +7,8 @@ results; torch tensor in -> torch CUDA tensor out.  ``coefficients.data`` always
 from __future__ import annotations
 
 import copy
+import ctypes
+import numbers
 import warnings
 
 import numpy as np
@@ -320,6 +322,9 @@ def wow(data, scaling_function=B3spline, n_scales=None, weights=[], whitening=Tr
         # 1-D signals and 3-D volumes: the reference's loop is dimension-generic (watroo/utils.py:148-150, :194)
         n_scales, sigma_bilateral, wts, dns = _wow_plan(img.shape, scaling_function, n_scales, weights,
                                                         denoise_coefficients, bilateral, h=h, n_dims=img.ndim)
+        if img.ndim == 3 and sigma_bilateral is None and h == 0 and not preserve_variance and n_scales >= 0:
+            recon, co = _wow_volume(img, scaling_function, n_scales, wts, dns, whitening, soft_threshold, noise)
+            return _result(recon, was_numpy), co
         transform = AtrousTransform(scaling_function, bilateral=sigma_bilateral, bilateral_scaling=bilateral_scaling)
         co = transform(img, n_scales)
         co.noise = noise
@@ -348,11 +353,78 @@ def wow(data, scaling_function=B3spline, n_scales=None, weights=[], whitening=Tr
     return _result(recon[0], was_numpy), co
 
 
-def _wow_nd(co, wts, dns, whitening, soft_threshold, preserve_variance, gamma, gamma_min, gamma_max, h):
+def _volume_noise(noise, shape, dtype, device, thresholded):
+    """The noise of wow() on a volume of ``shape`` (D, H, W), classified as Coefficients._noise_arg classifies it.
+    Returns (_Noise or None for the MAD estimate, map z-stride, the noise the coefficients keep afterwards)."""
+    d, h, w = shape
+    if noise is None:
+        return None, 0, None
+    if isinstance(noise, torch.Tensor) and not (noise.numel() == 1 and noise.ndim <= 1):
+        m, kept = noise, noise
+    elif isinstance(noise, np.ndarray) and noise.ndim > 0:
+        m, kept = noise, None  # a map that a threshold uses is kept as its device copy
+    else:
+        if isinstance(noise, torch.Tensor):
+            nz = _Noise(dev=noise) if noise.is_cuda and noise.dtype == torch.float64 else _Noise(host=float(noise.item()))
+        elif isinstance(noise, np.ndarray) or isinstance(noise, numbers.Number):
+            nz = _Noise(host=float(noise))
+        elif thresholded:
+            raise TypeError(f"unsupported noise type {type(noise)}")
+        else:
+            nz = _Noise()
+        return nz, 0, noise
+    if not thresholded:
+        return _Noise(), 0, noise
+    if tuple(m.shape) in ((h, w), (1, h, w)):
+        # one (H, W) map for every slice: read with a depth stride of 0
+        plane = broadcast_noise_map(m.reshape(h, w), (h, w), dtype, device)
+        return _Noise(map_=plane), 0, kept if kept is not None else plane.expand(d, h, w)
+    full = broadcast_noise_map(m, shape, dtype, device)
+    return _Noise(map_=full), h * w, kept if kept is not None else full
+
+
+def _wow_volume(img, scaling_function, n_scales, wts, dns, whitening, soft_threshold, noise):
+    """wow() of a plain volume (D, H, W) with h == 0 and no preserve_variance: one wb_wow_cascade_volume call,
+    bit-identical to the transform followed by _wow_nd, the noise left on the coefficients as _wow_nd leaves it."""
+    lib = _lib.load(require_cuda=True)
+    sf = scaling_function(3)
+    img = img.contiguous()
+    dev, dt = img.device, img.dtype
+    code = _lib.dtype_code(dt)
+    L = n_scales
+    shape = tuple(img.shape)
+    planes = torch.empty((L + 1,) + shape, dtype=dt, device=dev)
+    recon = torch.empty(shape, dtype=dt, device=dev)
+    scratch = torch.empty(lib.wb_volume_scratch_bytes(code, *shape, L), dtype=torch.uint8, device=dev)
+    ws = torch.empty(lib.wb_wow_cascade_volume_workspace_bytes(code, *shape), dtype=torch.uint8, device=dev)
+    thresholded = any(d != 0 for d in dns[:L])
+    nz, zstride, kept = _volume_noise(noise, shape, dt, dev, thresholded)
+    estimate = nz is None and thresholded
+    if estimate:
+        nz = _Noise(dev=torch.empty(1, dtype=torch.float64, device=dev))
+        kept = nz.dev
+    use = nz if nz is not None else _Noise()
+    sigma_e = sf.sigma_e()
+    arr = ctypes.c_double * (L + 1)
+    with torch.cuda.device(dev):
+        _lib.check(lib.wb_wow_cascade_volume(
+            img.data_ptr(), planes.data_ptr(), scratch.data_ptr(), recon.data_ptr(), *shape, L, sf.taps_code, code,
+            arr(*[float(x) for x in wts[:L + 1]]), arr(*([float(x) for x in dns[:L]] + [0.0])),
+            arr(*([float(x) for x in sigma_e[:L]] + [0.0])), 1 if soft_threshold else 0, 1 if whitening else 0,
+            float(use.host), use.dev_ptr, 1 if estimate else 0, use.map_ptr or None, zstride, ws.data_ptr(), ws.numel(),
+            _lib.stream_ptr(dev)))
+    co = Coefficients(planes, sf, None)
+    co.noise = kept
+    return recon, co
+
+
+def _wow_nd(co, wts, dns, whitening, soft_threshold, preserve_variance, gamma, gamma_min, gamma_max, h, smooth=None):
     """The loop of wow() (watroo/utils.py:172-217) on the coefficients of a 1-D signal or a 3-D volume, every option
     included: the transform and the n-D smooth of the local power run in the library's kernels, the plane-wise factors
-    are element-wise device arithmetic in the reference's order and dtypes.  A parity path, whitened in place."""
+    are element-wise device arithmetic in the reference's order and dtypes.  A parity path, whitened in place.
+    ``smooth``: the n-D smooth of the local power (default _smooth_nd)."""
     from .wavelets import _smooth_nd
+    smooth = smooth or _smooth_nd
     data = co.data
     dt = data.dtype
     L = len(co) - 1
@@ -372,7 +444,7 @@ def _wow_nd(co, wts, dns, whitening, soft_threshold, preserve_variance, gamma, g
         else:
             local_power = None
             if white:
-                local_power = _smooth_nd(power.contiguous(), s, co.scaling_function)  # plain smooth, utils.py:194
+                local_power = smooth(power.contiguous(), s, co.scaling_function)  # plain smooth, utils.py:194
                 local_power = torch.sqrt(torch.where(local_power <= 0, torch.full_like(local_power, 1e-15), local_power))
             sig = co.significance(dns[s], s, soft_threshold=soft_threshold)
             if sig.dtype == torch.bool or sig.dtype == torch.float64:

@@ -132,7 +132,23 @@ def convolution(arr, scaling_function, s=0, output=None):
 
 def _smooth_nd(arr, s, scaling_function):
     """S_s of a contiguous 1-D signal (mirror border, watroo/wavelets.py:64-69) or 3-D volume (2-D smooth of every
-    slice, then the depth pass, :46-63) -- one scale of AtrousTransform._run_nd without the detail plane."""
+    slice, then the depth pass, :46-63, wb_atrous_scale_volume) -- one scale of AtrousTransform._run_nd without the
+    detail plane."""
+    if arr.ndim == 1:
+        return _smooth_nd_reference(arr, s, scaling_function)
+    lib = _lib.load(require_cuda=True)
+    out = torch.empty_like(arr)
+    tmp = torch.empty_like(arr)
+    with torch.cuda.device(arr.device):
+        _lib.check(lib.wb_atrous_scale_volume(arr.data_ptr(), out.data_ptr(), None, tmp.data_ptr(), *arr.shape, int(s),
+                                              scaling_function.taps_code, _lib.dtype_code(arr.dtype),
+                                              _lib.stream_ptr(arr.device)))
+    return out
+
+
+def _smooth_nd_reference(arr, s, scaling_function):
+    """_smooth_nd on wb_atrous_scale + wb_atrous_axis (one thread per sample, taps gathered from global memory): the
+    route the volume kernels are checked against."""
     lib = _lib.load(require_cuda=True)
     code, taps = _lib.dtype_code(arr.dtype), scaling_function.taps_code
     out = torch.empty_like(arr)
@@ -396,9 +412,10 @@ class AtrousTransform:
     def __call__(self, arr, level, recursive=False):
         """Transform an image over ``level`` scales -> ``Coefficients`` with ``level + 1`` planes.
 
-        2-D images take the row-pipeline kernels.  1-D signals (whole-sample 'mirror' border, watroo/wavelets.py:64-69)
-        and 3-D volumes (2-D smooth of every slice, then the depth pass, watroo/wavelets.py:46-63) run the plain
-        cascade through ``wb_atrous_axis`` and the bilateral one through ``wb_atrous_scale_bilateral_nd``.
+        2-D images take the row-pipeline kernels.  3-D volumes (2-D smooth of every slice, then the depth pass,
+        watroo/wavelets.py:46-63) run the plain cascade through ``wb_atrous_transform_volume``, 1-D signals
+        (whole-sample 'mirror' border, watroo/wavelets.py:64-69) through ``wb_atrous_axis``, and both bilateral
+        cascades through ``wb_atrous_scale_bilateral_nd``.
 
         ``recursive=True`` on a plain 2-D transform reproduces the RESULT of the reference's recursive algorithm
         (watroo/wavelets.py:330-406; it differs from the standard one near the borders: symmetric pad by
@@ -445,7 +462,26 @@ class AtrousTransform:
         return full[:, hw:hw + h, hw:hw + w].contiguous()
 
     def _run_nd(self, arr, level, scaling_function):
-        """Plain cascade of a 1-D signal or a 3-D volume: planes ``(level + 1, *arr.shape)``."""
+        """Plain cascade of a 1-D signal or a 3-D volume: planes ``(level + 1, *arr.shape)``.  A plain volume is one
+        wb_atrous_transform_volume call; bilateral volumes and 1-D signals take _run_nd_reference."""
+        if level < 0:
+            raise ValueError("level must be >= 0")
+        if arr.ndim != 3 or self.bilateral is not None:
+            return self._run_nd_reference(arr, level, scaling_function)
+        lib = _lib.load(require_cuda=True)
+        arr = arr.contiguous()
+        planes = torch.empty((level + 1,) + tuple(arr.shape), dtype=arr.dtype, device=arr.device)
+        code = _lib.dtype_code(arr.dtype)
+        scratch = torch.empty(lib.wb_volume_scratch_bytes(code, *arr.shape, level), dtype=torch.uint8, device=arr.device)
+        with torch.cuda.device(arr.device):
+            _lib.check(lib.wb_atrous_transform_volume(arr.data_ptr(), planes.data_ptr(), scratch.data_ptr(), *arr.shape,
+                                                      level, scaling_function.taps_code, code,
+                                                      _lib.stream_ptr(arr.device)))
+        return planes
+
+    def _run_nd_reference(self, arr, level, scaling_function):
+        """The per-scale cascade of a 1-D signal or a 3-D volume on wb_atrous_axis / wb_atrous_scale_bilateral_nd (for
+        volumes the route wb_atrous_transform_volume is checked against)."""
         if level < 0:
             raise ValueError("level must be >= 0")
         lib = _lib.load(require_cuda=True)
